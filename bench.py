@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — k-mers tested/sec through count -> matrix -> chi2 / Welch -> filter (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config {1..5}] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config {1..5}] [--impl ours|reference] [--dump-outputs DIR]
 
 --config c = BASELINE.json configs[c-1] on synthetic data of that shape (phenotypeseeker_b200/synth_gpu.py):
   1  20 x 4.3 Mbp assemblies, k=16, binary, unweighted chi2, --omit_B_correction      (the CPU-runnable case)
@@ -117,6 +117,30 @@ def result_digest(U, res):
         h.update(np.ascontiguousarray(r.kmer, dtype=np.uint64).tobytes())
         h.update(np.ascontiguousarray(r.n_with, dtype=np.uint32).tobytes())
     return h.hexdigest()[:32]
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, U, res, limit=DUMP_BYTES):
+    """Write what a step returned as float64 .npy files, so that two builds can be compared array by array:
+    union_kmers.npy holds U; the other files have one entry per survivor, the phenotype columns of `res` one after
+    the other: its column (pheno), k-mer, union row, statistic, p-value, group means, sample count and bit-packed
+    matrix row (rowbits, uint32 words). Every value is exact in float64 (k-mers of k <= 26). When the survivors
+    would take more than `limit` bytes, a fixed, seeded sample of them is written; survivor.npy holds the indices
+    of the written survivors among all of them."""
+    cols = {"pheno": np.concatenate([np.full(len(r.kmer), j) for j, r in enumerate(res)])}
+    for name in ("kmer", "row", "stat", "p", "mean_x", "mean_y", "n_with", "rowbits"):
+        cols[name] = np.concatenate([getattr(r, name) for r in res])
+    n = len(cols["pheno"])
+    per_survivor = 8 * (len(cols) + cols["rowbits"].shape[1])   # 8 one-value arrays, survivor.npy, the row words
+    keep = min(n, (limit - 4096) // per_survivor)               # 4 KB for U and the .npy headers
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "union_kmers.npy"), np.array([U], dtype=np.float64))
+    np.save(os.path.join(out_dir, "survivor.npy"), idx.astype(np.float64))
+    for name, a in cols.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a[idx].astype(np.float64))
 
 
 # ---------------------------------------------------------------------------------------
@@ -292,6 +316,8 @@ def run_ours(args):
         return
     digest = result_digest(U, res)
     assert digest == result_digest(U2, res2), "device-resident and host-buffer runs disagree"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, U, res)
     n_surv = int(sum(len(r.kmer) for r in res))
     d2h_bytes = n_surv * (8 * 6 + 4 * 2 + ka.ctx.row_words() * 4) + 64
     # the same (config, size) must give the same result on any number of GPUs: compare with the committed digests
@@ -399,7 +425,14 @@ def main():
     ap.add_argument("--write-digest", action="store_true", help="record this (1-GPU) result in tests/golden/bench_digests.json")
     ap.add_argument("--route", default="auto", choices=["auto", "pages", "streams"],
                     help="multi-GPU exchange route (phenotypeseeker_b200/dist.py)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step (device-resident run) as DIR/<name>.npy, float64, "
+                         "at most 64 MB (a seeded sample of the survivors beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":
