@@ -608,7 +608,7 @@ static void add_samples_impl(ps_ctx *c, int first_idx, int count, const void *co
                 (k_decode_write<F><<<nt, DEC_THREADS, 0, c->stream>>>(stg, d_files, d_tile_file, t0, d_tile_state,      \
                                                                       d_tile_off, d_chunk_next, d_chunk_cnt,            \
                                                                       c->pool_seq.as<uint32_t>(), c->pool_bad.as<uint32_t>())))
-        if (fmt_seen == 2u && c->dec_swar)
+        if (fmt_seen == 2u && !c->dec_bytes)
             KLAUNCH(c, "decode_write", (double)gbytes + (double)(pp - gp0) * 3 / 8,
                     (k_decode_write_fasta<<<nt, DEC_THREADS, 0, c->stream>>>(stg, d_files, d_tile_file, t0, d_tile_state, d_tile_off,
                                                                              d_chunk_next, d_chunk_cnt, c->pool_seq.as<uint32_t>(),
@@ -1070,7 +1070,7 @@ int ps_ctx_create(int device, ps_ctx **out) {
     cudaFuncSetAttribute(k_bucket_count_pg<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     if (const char *ev = getenv("PSKMER_BK_TMA")) c->bk_tma = atoi(ev) != 0;
     if (const char *ev = getenv("PSKMER_PAGED")) c->paged = atoi(ev) != 0;
-    if (const char *ev = getenv("PSKMER_DECODE")) c->dec_swar = strcmp(ev, "swar") == 0;
+    if (const char *ev = getenv("PSKMER_DECODE")) c->dec_bytes = strcmp(ev, "bytes") == 0;
     if (const char *ev = getenv("PSKMER_SC1")) c->sc1_lean = strcmp(ev, "regs") != 0;
     if (c->sc1_lean) c->sc1_grid = 3 * PS_SMS;
     if (const char *ev = getenv("PSKMER_CHI2")) { c->chi2_sparse = strcmp(ev, "masked") != 0; c->chi2_sparse_force = strcmp(ev, "walk") == 0; }

@@ -123,7 +123,7 @@ struct ps_ctx {
     bool bucketed = true;
     int bk_row_words = 10240;   // shared-memory words of k_bucket_build's row table for ordinary buckets (PSKMER_BK_ROW_KB)
 
-    bool dec_swar = false;      // PSKMER_DECODE=swar: FASTA write pass from per-thread bit strings (k_decode_write_fasta; measured slower)
+    bool dec_bytes = false;     // PSKMER_DECODE=bytes: all-FASTA launches take the staged-byte write pass k_decode_write<1> instead of k_decode_write_fasta (A/B runs; =swar names the default)
     bool sc1_lean = true;       // k_scatter1 recomputes its k-mers in the grouping phase (40 registers, 3 blocks per SM); PSKMER_SC1=regs: keeps them in registers (2 blocks per SM)
     bool chi2_sparse_force = false;   // PSKMER_CHI2=walk: the bit-walk kernel for every unweighted shape it can take (tests)
     bool chi2_sparse = true;    // unweighted chi2 walks the row's bits (k_test_chi2_sp); PSKMER_CHI2=masked: one masked popcount per column

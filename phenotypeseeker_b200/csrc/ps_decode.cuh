@@ -11,8 +11,9 @@
 // from every possible incoming state, giving a (next_state[4], emitted[4]) summary; summaries
 // compose associatively, so a warp-shuffle scan + a short walk over tile summaries gives every
 // chunk its true incoming state and output offset. Pass 1 (k_decode_count) produces tile
-// summaries, k_decode_walk walks them per file, pass 2 (k_decode_write) re-simulates with the
-// known state, stages codes in shared memory and packs them 16 bases / 32 mask bits per word.
+// summaries, k_decode_walk walks them per file, pass 2 re-simulates with the known state and packs
+// 16 bases / 32 mask bits per word: k_decode_write_fasta from per-thread bit strings when a launch is
+// all FASTA (ps_decode_bits.h), k_decode_write from staged code bytes otherwise.
 #pragma once
 #include "ps_common.cuh"
 #include "ps_decode_bits.h"
@@ -83,6 +84,17 @@ __device__ __forceinline__ DecSum dec_compose(const DecSum &a, const DecSum &b) 
     return r;
 }
 
+// dec_compose for FASTA summaries: every FASTA summary maps states 0 and 1 into {0, 1} and keeps states 2 and 3 as
+// fixed points with no codes, so only states 0 and 1 (the low 32 bits of cnt) are composed; the result has the same
+// bits as dec_compose.
+__device__ __forceinline__ DecSum dec_compose_fasta(const DecSum &a, const DecSum &b) {
+    const uint32_t n0 = a.next & 3u, n1 = (a.next >> 2) & 3u;
+    const uint32_t ac = (uint32_t)a.cnt, bc = (uint32_t)b.cnt;
+    const uint32_t c0 = (ac & 0xFFFFu) + ((bc >> (16 * n0)) & 0xFFFFu);
+    const uint32_t c1 = (ac >> 16) + ((bc >> (16 * n1)) & 0xFFFFu);
+    return DecSum{((b.next >> (2 * n0)) & 3u) | (((b.next >> (2 * n1)) & 3u) << 2) | 0xE0u, (uint64_t)(c0 | (c1 << 16))};
+}
+
 __device__ __forceinline__ void dec_load_chunk(const uint8_t *file, uint64_t base, uint64_t len,
                                                uint32_t w[DEC_WORDS]) {
 #pragma unroll
@@ -93,69 +105,39 @@ __device__ __forceinline__ void dec_load_chunk(const uint8_t *file, uint64_t bas
     }
 }
 
-// Summary of one chunk for all incoming states; only bytes in [lo, hi) count.
+// Summary of one chunk (its 16 words in w) for all incoming states; only bytes in [lo, hi) count.
 // One walk over the bytes is enough for every incoming state:
-//  FASTA  - walk as if in sequence state. An incoming header state emits nothing up to the
-//           first '\n' of the chunk and is identical to the sequence-state walk after it (both
-//           are in sequence state right after that byte), so cnt[hdr] = total - count at that '\n'.
+//  FASTA  - a full chunk without '>' (all but ~1 chunk in 1000 of an assembly): psd_fasta_count_words, word masks
+//           on the words in registers; any other chunk: psd_fasta_count_bytes (ps_decode_bits.h).
 //  FASTQ  - the phase of a byte is (incoming phase + newlines before it) & 3; count emissions per
 //           newline-segment index q, then cnt[p] = seg[(1 - p) & 3].
-__device__ __forceinline__ DecSum dec_chunk_summary(const uint32_t w[DEC_WORDS], uint64_t base, uint64_t lo,
-                                                    uint64_t hi, uint32_t fmt) {
+// The byte-wise walks read the chunk from the thread's shared-memory row `row`, so that their loops stay rolled.
+__device__ __forceinline__ DecSum dec_chunk_summary(const uint32_t w[DEC_WORDS], uint32_t *row, uint64_t base,
+                                                    uint64_t lo, uint64_t hi, uint32_t fmt) {
     DecSum r{0u, 0ull};
-    // [jlo, jhi) = the chunk's bytes inside [lo, hi), as small ints (the loops are unrolled)
     const int jlo = lo > base ? (int)min((uint64_t)DEC_CHUNK, lo - base) : 0;
     const int jhi = hi > base ? (int)min((uint64_t)DEC_CHUNK, hi - base) : 0;
+    if (fmt == 1 && jlo == 0 && jhi == DEC_CHUNK && psd_fasta_count_words(w, r.next, r.cnt)) return r;
+#pragma unroll
+    for (int q = 0; q < DEC_WORDS; q++) row[q] = w[q];
     if (fmt == 1) {
-        // Fast path (a whole chunk without '>', i.e. all but ~1 chunk in 1000 of an assembly): four
-        // bytes per step. 0x80 flags per byte: zb(v) = byte of v is zero (exact, no carries).
-        if (jlo == 0 && jhi == DEC_CHUNK) {
-            auto zb = [](uint32_t v) { return ~(((v & 0x7F7F7F7Fu) + 0x7F7F7F7Fu) | v | 0x7F7F7F7Fu); };
-            uint32_t any_gt = 0, n = 0, n_at_nl = 0;
-            bool seen_nl = false;
-#pragma unroll
-            for (int q = 0; q < DEC_WORDS; q++) {
-                const uint32_t x = w[q];
-                any_gt |= zb(x ^ 0x3E3E3E3Eu);
-                const uint32_t emit = ~(zb(x & 0xE0E0E0E0u) & ~zb(x)) & 0x80808080u;   // not in 1..31
-                const uint32_t nl = zb(x ^ 0x0A0A0A0Au);
-                if (nl && !seen_nl) {
-                    seen_nl = true;
-                    n_at_nl = n + __popc(emit & ((1u << (__ffs(nl) - 1)) - 1u));
-                }
-                n += __popc(emit);
-            }
-            if (!any_gt) {
-                r.next = ((seen_nl ? 0u : 1u) << 2) | 0xE0u;
-                r.cnt = (uint64_t)n | ((uint64_t)(seen_nl ? n - n_at_nl : 0u) << 16);
-                return r;
-            }
-        }
-        uint32_t s = 0, n = 0, n_at_nl = 0;
-        bool seen_nl = false;
-#pragma unroll
-        for (int j = 0; j < DEC_CHUNK; j++) {
-            const uint32_t b = (w[j >> 2] >> (8 * (j & 3))) & 0xFFu;
-            if (j >= jlo && j < jhi) {
-                if (s == 1) { if (b == '\n') s = 0; }
-                else if (b == '>') { s = 1; n++; }
-                else if (dec_classify(b) != CODE_SKIP) n++;
-                if (b == '\n' && !seen_nl) { seen_nl = true; n_at_nl = n; }
-            }
-        }
-        r.next = s | ((seen_nl ? s : 1u) << 2) | 0xE0u;   // states 2,3 unused: fixed points
-        r.cnt = (uint64_t)n | ((uint64_t)(seen_nl ? n - n_at_nl : 0u) << 16);
+        psd_fasta_count_bytes(row, jlo, jhi, r.next, r.cnt);
     } else {
         uint32_t q = 0, seg0 = 0, seg1 = 0, seg2 = 0, seg3 = 0;
+#pragma unroll 1
+        for (int qw = 0; qw < DEC_WORDS; qw++) {
+            const uint32_t x = row[qw];
 #pragma unroll
-        for (int j = 0; j < DEC_CHUNK; j++) {
-            const uint32_t b = (w[j >> 2] >> (8 * (j & 3))) & 0xFFu;
-            if (j >= jlo && j < jhi) {
-                const bool nl = b == '\n';
-                const uint32_t e = (nl || dec_classify(b) != CODE_SKIP) ? 1u : 0u;   // '\n' -> BREAK
-                seg0 += (q == 0) ? e : 0u; seg1 += (q == 1) ? e : 0u;
-                seg2 += (q == 2) ? e : 0u; seg3 += (q == 3) ? e : 0u;
-                if (nl) q = (q + 1) & 3u;
+            for (int jj = 0; jj < 4; jj++) {
+                const int j = 4 * qw + jj;
+                const uint32_t b = (x >> (8 * jj)) & 0xFFu;
+                if (j >= jlo && j < jhi) {
+                    const bool nl = b == '\n';
+                    const uint32_t e = (nl || dec_classify(b) != CODE_SKIP) ? 1u : 0u;   // '\n' -> BREAK
+                    seg0 += (q == 0) ? e : 0u; seg1 += (q == 1) ? e : 0u;
+                    seg2 += (q == 2) ? e : 0u; seg3 += (q == 3) ? e : 0u;
+                    if (nl) q = (q + 1) & 3u;
+                }
             }
         }
         const uint32_t seg[4] = {seg0, seg1, seg2, seg3};
@@ -168,9 +150,40 @@ __device__ __forceinline__ DecSum dec_chunk_summary(const uint32_t w[DEC_WORDS],
     return r;
 }
 
+// Composition of the block's summaries in thread order, valid in thread 0. dec_compose is associative but not
+// commutative: the shuffle trees combine each lane with the lanes after it, first within each warp, then over
+// the warp totals in warp 0.
+__device__ __forceinline__ DecSum dec_block_reduce(DecSum v, DecSum *smem /*[NW]*/) {
+    const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        DecSum p;
+        p.next = __shfl_down_sync(0xffffffffu, v.next, d);
+        p.cnt = __shfl_down_sync(0xffffffffu, v.cnt, d);
+        if (lane + d < 32u) v = dec_compose(v, p);
+    }
+    if (lane == 0) smem[warp] = v;
+    __syncthreads();
+    constexpr int NW = DEC_THREADS / 32;
+    if (warp == 0) {
+        v = lane < (unsigned)NW ? smem[lane] : dec_identity();
+#pragma unroll
+        for (int d = 1; d < NW; d <<= 1) {
+            DecSum p;
+            p.next = __shfl_down_sync(0xffffffffu, v.next, d);
+            p.cnt = __shfl_down_sync(0xffffffffu, v.cnt, d);
+            if (lane + d < (unsigned)NW) v = dec_compose(v, p);
+        }
+    }
+    return v;
+}
+
 // Block-wide exclusive scan of summaries in thread order. Returns the exclusive prefix of
-// this thread; *total = composition of the whole block (valid in all threads).
+// this thread; *total = composition of the whole block (valid in all threads). FASTA: every summary of the block is
+// a FASTA one (dec_compose_fasta).
+template <bool FASTA = false>
 __device__ __forceinline__ DecSum dec_block_scan(DecSum mine, DecSum *total, DecSum *smem /*[NW + 1]*/) {
+    auto compose = [](const DecSum &a, const DecSum &b) { return FASTA ? dec_compose_fasta(a, b) : dec_compose(a, b); };
     const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     DecSum inc = mine;
 #pragma unroll
@@ -178,7 +191,7 @@ __device__ __forceinline__ DecSum dec_block_scan(DecSum mine, DecSum *total, Dec
         DecSum p;
         p.next = __shfl_up_sync(0xffffffffu, inc.next, d);
         p.cnt = __shfl_up_sync(0xffffffffu, inc.cnt, d);
-        if (lane >= (unsigned)d) inc = dec_compose(p, inc);
+        if (lane >= (unsigned)d) inc = compose(p, inc);
     }
     DecSum exc;
     exc.next = __shfl_up_sync(0xffffffffu, inc.next, 1);
@@ -187,21 +200,27 @@ __device__ __forceinline__ DecSum dec_block_scan(DecSum mine, DecSum *total, Dec
     constexpr int NW = DEC_THREADS / 32;
     if (lane == 31) smem[warp] = inc;
     __syncthreads();
-    // one thread turns the warp totals into exclusive warp prefixes (+ the block total)
-    if (threadIdx.x == 0) {
-        DecSum run = dec_identity();
+    // warp 0 turns the warp totals into exclusive warp prefixes (+ the block total) with a shuffle scan over NW lanes
+    if (warp == 0) {
+        DecSum v = lane < (unsigned)NW ? smem[lane] : dec_identity();
 #pragma unroll
-        for (int w2 = 0; w2 < NW; w2++) {
-            const DecSum t = smem[w2];
-            smem[w2] = run;
-            run = dec_compose(run, t);
+        for (int d = 1; d < NW; d <<= 1) {
+            DecSum p;
+            p.next = __shfl_up_sync(0xffffffffu, v.next, d);
+            p.cnt = __shfl_up_sync(0xffffffffu, v.cnt, d);
+            if (lane >= (unsigned)d) v = compose(p, v);
         }
-        smem[NW] = run;
+        DecSum e;
+        e.next = __shfl_up_sync(0xffffffffu, v.next, 1);
+        e.cnt = __shfl_up_sync(0xffffffffu, v.cnt, 1);
+        if (lane == 0) e = dec_identity();
+        if (lane < (unsigned)NW) smem[lane] = e;
+        if (lane == NW - 1) smem[NW] = v;
     }
     __syncthreads();
     const DecSum wp = smem[warp];
     *total = smem[NW];
-    return dec_compose(wp, exc);
+    return compose(wp, exc);
 }
 
 // First '>' or '@' of each file: one block per file.
@@ -237,13 +256,17 @@ __global__ void k_detect(const uint8_t *__restrict__ staging, FileEnt *__restric
     }
 }
 
+// a thread's shared-memory row of 16 words: stride 17, conflict-free
+#define DEC_IN_STRIDE 17
+
 // Pass 1: per-tile summaries.
-__global__ void __launch_bounds__(DEC_THREADS)
+__global__ void __launch_bounds__(DEC_THREADS, 6)
 k_decode_count(const uint8_t *__restrict__ staging, const FileEnt *__restrict__ files,
                const uint32_t *__restrict__ tile_file, uint32_t tile_base, uint32_t *__restrict__ tile_next,
                uint64_t *__restrict__ tile_cnt, uint32_t *__restrict__ chunk_next,
                uint64_t *__restrict__ chunk_cnt) {
-    __shared__ DecSum sm[DEC_THREADS / 32 + 1];
+    __shared__ DecSum sm[DEC_THREADS / 32];
+    __shared__ uint32_t s_in[DEC_THREADS * DEC_IN_STRIDE];
     const uint32_t t = blockIdx.x + tile_base;
     const FileEnt f = files[tile_file[t]];
     const uint64_t base = ((uint64_t)(t - f.tile0) * DEC_THREADS + threadIdx.x) * DEC_CHUNK;
@@ -251,13 +274,12 @@ k_decode_count(const uint8_t *__restrict__ staging, const FileEnt *__restrict__ 
     if (f.fmt != 0 && base < f.len) {
         uint32_t w[DEC_WORDS];
         dec_load_chunk(staging + f.off, base, f.len, w);
-        mine = dec_chunk_summary(w, base, f.start, f.len, f.fmt);
+        mine = dec_chunk_summary(w, s_in + threadIdx.x * DEC_IN_STRIDE, base, f.start, f.len, f.fmt);
     }
     // pass 2 starts from this summary instead of walking the chunk a second time
     chunk_next[(size_t)t * DEC_THREADS + threadIdx.x] = mine.next;
     chunk_cnt[(size_t)t * DEC_THREADS + threadIdx.x] = mine.cnt;
-    DecSum tot;
-    dec_block_scan(mine, &tot, sm);
+    const DecSum tot = dec_block_reduce(mine, sm);
     if (threadIdx.x == 0) { tile_next[t] = tot.next; tile_cnt[t] = tot.cnt; }
 }
 
@@ -361,9 +383,8 @@ k_decode_write(const uint8_t *__restrict__ staging, const FileEnt *__restrict__ 
 
 // Pass 2 for launches whose files are all FASTA (or empty): the same result as k_decode_write<1>, built from
 // per-thread bit strings instead of one staged code byte per position (ps_decode_bits.h). The chunk's 16 words
-// go through shared memory (row stride 17: conflict-free) so that the word loop stays rolled — the byte-loop
-// kernel's fully unrolled body (3,984 SASS instructions) stalled on instruction fetch a third of the time.
-#define DEC_IN_STRIDE 17
+// go through a shared-memory row so that the word loop stays rolled — the byte-loop kernel's fully unrolled body
+// (3,984 SASS instructions) stalled on instruction fetch a third of the time.
 #define DEC_OUT_POS (DEC_TILE + POS_ALIGN + 64)
 __global__ void __launch_bounds__(DEC_THREADS)
 k_decode_write_fasta(const uint8_t *__restrict__ staging, const FileEnt *__restrict__ files,
@@ -379,6 +400,7 @@ k_decode_write_fasta(const uint8_t *__restrict__ staging, const FileEnt *__restr
     const FileEnt f = files[tile_file[t]];
     const uint64_t base = ((uint64_t)(t - f.tile0) * DEC_THREADS + threadIdx.x) * DEC_CHUNK;
     const bool active = f.fmt != 0 && base < f.len;
+    psd_sel_init();
     for (int i = threadIdx.x; i < DEC_OUT_POS / 16 + 8; i += DEC_THREADS) s_seq[i] = 0u;
     for (int i = threadIdx.x; i < DEC_OUT_POS / 32 + 8; i += DEC_THREADS) s_bad[i] = 0u;
     uint32_t *mine_in = s_in + threadIdx.x * DEC_IN_STRIDE;
@@ -392,7 +414,7 @@ k_decode_write_fasta(const uint8_t *__restrict__ staging, const FileEnt *__restr
     mine.next = chunk_next[(size_t)t * DEC_THREADS + threadIdx.x];
     mine.cnt = chunk_cnt[(size_t)t * DEC_THREADS + threadIdx.x];
     DecSum tot;
-    DecSum exc = dec_block_scan(mine, &tot, sm);          // contains the barriers that publish the cleared tables
+    DecSum exc = dec_block_scan<true>(mine, &tot, sm);    // its barriers publish the cleared and filled tables
     const uint32_t s0 = tile_state[t];
     uint32_t n_codes = (uint32_t)((tot.cnt >> (16 * s0)) & 0xFFFFull);
     const uint64_t gp0 = f.pool_off + tile_off[t];
