@@ -11,6 +11,7 @@
 #include "ps_sort.cuh"
 #include "ps_rows.cuh"
 #include "ps_test.cuh"
+#include "ps_chi2_reach.h"
 
 static std::string g_create_err;
 
@@ -981,19 +982,28 @@ static void launch_chi2(ps_ctx *c, int qpl, int grid, const uint4 *m, int wq, in
 #undef PS_CHI2
 }
 
-static void launch_chi2_sp(ps_ctx *c, int qpl, int grid, const uint4 *m, int wq, int lpr_log2, int P, bool no_na,
-                           const ulonglong2 *e1, const ulonglong2 *e0, int npad, const int *totn, const int *tot1,
-                           const int *tot0, int mn, int mx, double thr, SurvOut o) {
+static void launch_chi2_sp(ps_ctx *c, int grid, const uint4 *m, int wq, int lpr_log2, int P, bool no_na,
+                           const ulonglong2 *e1, const ulonglong2 *e0, int npad, const int *tot1, const int *tot0,
+                           const int2 *reach, int np_lo, int np_hi, double thr, SurvOut o) {
     const double bytes = (double)c->U * c->row_words * 4;
     const int N = c->n_samples;
-#define PS_CHI2SP(Q, NN) KLAUNCH(c, "test_chi2", bytes, (k_test_chi2_sp<Q, NN><<<grid, 256, 0, c->stream>>>(m, c->U, wq, lpr_log2, P, N, e1, e0, npad, totn, tot1, tot0, mn, mx, thr, o)))
-#define PS_CHI2SP_Q(Q) do { if (no_na) PS_CHI2SP(Q, true); else PS_CHI2SP(Q, false); } while (0)
-    if (qpl <= 1) PS_CHI2SP_Q(1);
-    else if (qpl <= 2) PS_CHI2SP_Q(2);
-    else if (qpl <= 4) PS_CHI2SP_Q(4);
-    else PS_CHI2SP_Q(16);
-#undef PS_CHI2SP_Q
+    if (lpr_log2 < 5) {
+#define PS_CHI2SP(NN) KLAUNCH(c, "test_chi2", bytes, (k_test_chi2_sp<NN><<<grid, 256, 0, c->stream>>>(m, c->U, wq, lpr_log2, P, N, e1, e0, npad, tot1, tot0, reach, np_lo, np_hi, thr, o)))
+        if (no_na) PS_CHI2SP(true); else PS_CHI2SP(false);
 #undef PS_CHI2SP
+        return;
+    }
+    // rows that fill the warp: one instance per number of 32-bit words a lane owns (3..8 for 2,048 < N <= 8,190)
+    const uint32_t *mw = reinterpret_cast<const uint32_t *>(m);
+    const int kw = ceil_div(ceil_div(N, 32), 32), wp = c->row_words;
+#define PS_CHI2SPW(K, NN) KLAUNCH(c, "test_chi2", bytes, (k_test_chi2_sp_warp<K, NN><<<grid, 256, 0, c->stream>>>(mw, c->U, wp, P, N, e1, e0, npad, tot1, tot0, reach, np_lo, np_hi, thr, o)))
+#define PS_CHI2SPW_K(K) case K: if (no_na) PS_CHI2SPW(K, true); else PS_CHI2SPW(K, false); break
+    switch (kw) {
+        PS_CHI2SPW_K(3); PS_CHI2SPW_K(4); PS_CHI2SPW_K(5); PS_CHI2SPW_K(6); PS_CHI2SPW_K(7); PS_CHI2SPW_K(8);
+    default: PS_THROW(PS_ERR_ARG, "no bit-walk chi2 kernel for this row width");
+    }
+#undef PS_CHI2SPW_K
+#undef PS_CHI2SPW
 }
 
 static void launch_welch(ps_ctx *c, int qpl, int grid, const uint4 *m, int wq, int lpr_log2, int P, int N,
@@ -1413,6 +1423,8 @@ int ps_test_chi2(ps_ctx *c, int P, const int8_t *pheno, const double *weights, i
     bool no_na = true;
     const ulonglong2 *d_e1 = nullptr, *d_e0 = nullptr;
     const int *d_tot1 = nullptr, *d_tot0 = nullptr;
+    const int2 *d_reach = nullptr;
+    int np_lo = 1, np_hi = 0;     // popcounts a row needs to be tested in some column (none: every row is skipped)
     if (sparse_walk) {
         const int npad = wp * 32, chunks = ceil_div(P, CHI2_SP_COLS);
         std::vector<unsigned long long> e((size_t)2 * chunks * npad * 2, 0ull);     // [class][chunk][sample][half]
@@ -1428,14 +1440,27 @@ int ps_test_chi2(ps_ctx *c, int P, const int8_t *pheno, const double *weights, i
             }
             if (totn[p] != N) no_na = false;
         }
-        c->tmp2.reserve(e.size() * 8 + tots.size() * 4 + 64, c->stream);
+        // Per column, the n_with that pass the sample filter and can reach the threshold at all; a row's popcount
+        // is n_with plus at most the column's NA samples. Every other row fails the kernel's screen in every column.
+        std::vector<int2> reach(P);
+        for (int p = 0; p < P; p++) {
+            ps_chi2_reach(tots[p], tots[(size_t)P + p], min_samples, max_samples, thr, &reach[p].x, &reach[p].y);
+            if (reach[p].x > reach[p].y) continue;
+            const int hi = reach[p].y + (N - totn[p]);
+            if (np_lo > np_hi) { np_lo = reach[p].x; np_hi = hi; }
+            else { np_lo = std::min(np_lo, reach[p].x); np_hi = std::max(np_hi, hi); }
+        }
+        c->tmp2.reserve(e.size() * 8 + tots.size() * 4 + reach.size() * 8 + 64, c->stream);
         CK(cudaMemcpyAsync(c->tmp2.p, e.data(), e.size() * 8, cudaMemcpyHostToDevice, c->stream));
         int *dt = reinterpret_cast<int *>(c->tmp2.as<unsigned long long>() + e.size());
         CK(cudaMemcpyAsync(dt, tots.data(), tots.size() * 4, cudaMemcpyHostToDevice, c->stream));
+        int2 *dr = reinterpret_cast<int2 *>(dt + tots.size());
+        CK(cudaMemcpyAsync(dr, reach.data(), reach.size() * 8, cudaMemcpyHostToDevice, c->stream));
         CK(cudaStreamSynchronize(c->stream));
         d_e1 = c->tmp2.as<ulonglong2>();
         d_e0 = d_e1 + (size_t)chunks * npad;
         d_tot1 = dt; d_tot0 = dt + P;
+        d_reach = dr;
     }
     CK(cudaStreamSynchronize(c->stream));  // host vectors above go out of scope
     c->surv_welch = false;
@@ -1451,7 +1476,7 @@ int ps_test_chi2(ps_ctx *c, int P, const int8_t *pheno, const double *weights, i
         CK(cudaMemsetAsync(c->scalars.p, 0, 8, c->stream));
         SurvOut o = surv_out(c, cap);
         if (weights) launch_chi2<true>(c, qpl, grid, c->matrix.as<uint4>(), wq, lpr_log2, P, c->ph_masks.as<uint32_t>(), d_totw, d_totn, d_w, c->ph_vals.as<double>(), min_samples, max_samples, thr, o);
-        else if (sparse_walk) launch_chi2_sp(c, qpl, grid, c->matrix.as<uint4>(), wq, lpr_log2, P, no_na, d_e1, d_e0, wp * 32, d_totn, d_tot1, d_tot0, min_samples, max_samples, thr, o);
+        else if (sparse_walk) launch_chi2_sp(c, grid, c->matrix.as<uint4>(), wq, lpr_log2, P, no_na, d_e1, d_e0, wp * 32, d_tot1, d_tot0, d_reach, np_lo, np_hi, thr, o);
         else launch_chi2<false>(c, qpl, grid, c->matrix.as<uint4>(), wq, lpr_log2, P, c->ph_masks.as<uint32_t>(), d_totw, d_totn, d_w, c->ph_vals.as<double>(), min_samples, max_samples, thr, o);
         const uint64_t ns = ps_read_scalar<unsigned long long>(c, c->scalars.as<unsigned long long>());
         c->n_surv = ns;

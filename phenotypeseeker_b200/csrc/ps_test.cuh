@@ -210,16 +210,62 @@ k_test_chi2(const uint4 *__restrict__ matrix, unsigned long long U, int wq, int 
 // word per bit: e1[s] holds, for ten columns at a time, a 12-bit field per column that is 1 iff sample s
 // has phenotype 1 in that column (e0: phenotype 0; not needed when no column has NA samples, because then
 // c = popcount(row) - a). One 128-bit load and two 64-bit adds per bit serve ten columns; the fields are
-// summed over the lane group with shuffles, and lane j finishes column j exactly like k_test_chi2 does.
+// summed over the lane group, and lane j finishes column j exactly like k_test_chi2 does.
 // The counts are the same integers, so chi2 is bit-identical. Cost ~ min(n_with, N - n_with) per row.
 // Field width 12 bits: min(popcount, N - popcount) <= 4095, i.e. N <= 8190 (the host checks).
+//
+// Rows whose popcount lies outside [np_lo, np_hi] are not walked: no column can reach the threshold with
+// them (the host's ps_chi2_reach, one interval per column, reach[ph]; np_hi allows for the column's NA samples).
 #define CHI2_SP_COLS 10      // columns per walk: two u64 of five 12-bit fields
-template <int QPL, bool NO_NA>
-__global__ void __launch_bounds__(256, QPL <= 2 ? 3 : 1)
+
+template <int K>
+__device__ __forceinline__ uint32_t pick_reg(const uint32_t (&v)[K], int i) {   // v[i] without local memory
+    uint32_t x = v[0];
+#pragma unroll
+    for (int k = 1; k < K; k++) x = i == k ? v[k] : x;
+    return x;
+}
+
+// Lane j of the row group finishes column ph from its summed fields: fa = number of walked samples with phenotype
+// 1 in that column, fb = with phenotype 0 (the walked samples are the cleared ones of a dense row). A count
+// outside reach[ph] fails the sample filter or the screen below; from the counts on, the arithmetic is that of
+// k_test_chi2 (unweighted), operation for operation.
+template <bool NO_NA>
+__device__ __forceinline__ void chi2_sp_finish(int ph, unsigned long long r, uint32_t fa, uint32_t fb, uint32_t np,
+                                               bool dense, const int *__restrict__ tot1, const int *__restrict__ tot0,
+                                               const int2 *__restrict__ reach, double chi2_min, double thr,
+                                               const SurvOut &out) {
+    const uint32_t ai = dense ? (uint32_t)tot1[ph] - fa : fa;
+    const uint32_t ci = NO_NA ? np - ai : dense ? (uint32_t)tot0[ph] - fb : fb;
+    const uint32_t n_with = ai + ci;
+    const int2 rc = reach[ph];
+    if ((int)n_with < rc.x || (int)n_with > rc.y) return;
+    const double a = (double)ai, c = (double)ci;
+    const double b = (double)tot1[ph] - a, d = (double)tot0[ph] - c;
+    const double w_pheno = a + b, wo_pheno = c + d, w_kmer = a + c, wo_kmer = b + d;
+    const double total = w_pheno + wo_pheno;
+    {
+        const double det = a * d - b * c;
+        const double approx = total * det * det / ((w_pheno * wo_pheno) * (w_kmer * wo_kmer));
+        if (approx < 0.99 * chi2_min) return;
+    }
+    const double ea = (w_pheno * w_kmer) / total, eb = (w_pheno * wo_kmer) / total;
+    const double ec = (wo_pheno * w_kmer) / total, ed = (wo_pheno * wo_kmer) / total;
+    const double ta = (a - ea) * (a - ea) / ea, tb = (b - eb) * (b - eb) / eb;
+    const double tc = (c - ec) * (c - ec) / ec, td = (d - ed) * (d - ed) / ed;
+    const double chi2 = ((ta + tb) + tc) + td;
+    const double p = exp(-0.5 * chi2);
+    if (p < thr) surv_push(out, ph, r, chi2, p, 0.0, 0.0, n_with);  // NaN compares false
+}
+
+// Rows of at most 16 uint4 (N <= 2,048): LPR = pow2 >= wq lanes per row, one uint4 per lane, fields summed with
+// xor-shuffles inside the group.
+template <bool NO_NA>
+__global__ void __launch_bounds__(256, 3)
 k_test_chi2_sp(const uint4 *__restrict__ matrix, unsigned long long U, int wq, int lpr_log2, int P, int n_samples,
                const ulonglong2 *__restrict__ e1, const ulonglong2 *__restrict__ e0, int npad,
-               const int *__restrict__ totn, const int *__restrict__ tot1, const int *__restrict__ tot0,
-               int min_s, int max_s, double thr, SurvOut out) {
+               const int *__restrict__ tot1, const int *__restrict__ tot0, const int2 *__restrict__ reach,
+               int np_lo, int np_hi, double thr, SurvOut out) {
     const int lpr = 1 << lpr_log2;
     const unsigned lane = threadIdx.x & 31;
     const unsigned sub = lane & (lpr - 1);
@@ -229,55 +275,39 @@ k_test_chi2_sp(const uint4 *__restrict__ matrix, unsigned long long U, int wq, i
     const double chi2_min = thr > 0.0 ? -2.0 * log(thr) : 1e300;
     // the row of the NEXT step is loaded before this step's row is walked (the walk is short and would
     // otherwise wait out the whole DRAM latency of its own load: 26 % of the stall samples)
-    auto load_row = [&](unsigned long long rr, uint4 (&dst)[QPL]) {
-#pragma unroll
-        for (int q = 0; q < QPL; q++) {
-            const int qi = sub + q * lpr;
-            dst[q] = (rr < U && qi < wq) ? __ldg(matrix + rr * (unsigned long long)wq + qi) : make_uint4(0, 0, 0, 0);
-        }
+    auto load_row = [&](unsigned long long rr) {
+        return (rr < U && (int)sub < wq) ? __ldg(matrix + rr * (unsigned long long)wq + sub) : make_uint4(0, 0, 0, 0);
     };
-    uint4 nxt[QPL];
-    load_row(warp_g * rpw + (lane >> lpr_log2), nxt);
+    uint4 nxt = load_row(warp_g * rpw + (lane >> lpr_log2));
     for (unsigned long long r0 = warp_g * rpw; r0 < U; r0 += nwarps * rpw) {
         const unsigned long long r = r0 + (lane >> lpr_log2);
         const bool rvalid = r < U;
-        uint4 rw[QPL];
-#pragma unroll
-        for (int q = 0; q < QPL; q++) rw[q] = nxt[q];
-        load_row(r + nwarps * rpw, nxt);
-        uint32_t np = 0;
-#pragma unroll
-        for (int q = 0; q < QPL; q++) np += __popc(rw[q].x) + __popc(rw[q].y) + __popc(rw[q].z) + __popc(rw[q].w);
+        const uint4 rw = nxt;
+        nxt = load_row(r + nwarps * rpw);
+        uint32_t np = __popc(rw.x) + __popc(rw.y) + __popc(rw.z) + __popc(rw.w);
         for (int o = lpr >> 1; o > 0; o >>= 1) np += __shfl_xor_sync(0xffffffffu, np, o);
-        // fewer than min_s samples carry the k-mer: no column can test it (n_with <= popcount)
-        const bool live = rvalid && (int)np >= min_s;
+        const bool live = rvalid && (int)np >= np_lo && (int)np <= np_hi;
         if (__all_sync(0xffffffffu, !live)) continue;
         const bool dense = 2u * np > (uint32_t)n_samples;      // walk the cleared bits of the valid samples instead
         for (int c0 = 0; c0 < P; c0 += CHI2_SP_COLS) {
             const ulonglong2 *t1 = e1 + (size_t)(c0 / CHI2_SP_COLS) * npad;
             const ulonglong2 *t0 = NO_NA ? nullptr : e0 + (size_t)(c0 / CHI2_SP_COLS) * npad;
             unsigned long long a0 = 0, a1 = 0, b0 = 0, b1 = 0;
-            if (live) {
+            if (live && (int)sub < wq) {
 #pragma unroll
-                for (int q = 0; q < QPL; q++) {
-                    const int qi = sub + q * lpr;
-                    if (qi < wq) {
-#pragma unroll
-                        for (int jj = 0; jj < 4; jj++) {
-                            const int s0 = (qi * 4 + jj) * 32;
-                            uint32_t bits = u4_get(rw[q], jj);
-                            if (dense) {
-                                const int left = n_samples - s0;      // valid samples of this word
-                                bits = ~bits & (left >= 32 ? 0xFFFFFFFFu : left <= 0 ? 0u : (1u << left) - 1u);
-                            }
-                            while (bits) {
-                                const int s = s0 + __ffs(bits) - 1;
-                                bits &= bits - 1;
-                                const ulonglong2 v = __ldg(t1 + s);
-                                a0 += v.x; a1 += v.y;
-                                if (!NO_NA) { const ulonglong2 z = __ldg(t0 + s); b0 += z.x; b1 += z.y; }
-                            }
-                        }
+                for (int jj = 0; jj < 4; jj++) {
+                    const int s0 = ((int)sub * 4 + jj) * 32;
+                    uint32_t bits = u4_get(rw, jj);
+                    if (dense) {
+                        const int left = n_samples - s0;      // valid samples of this word
+                        bits = ~bits & (left >= 32 ? 0xFFFFFFFFu : left <= 0 ? 0u : (1u << left) - 1u);
+                    }
+                    while (bits) {
+                        const int s = s0 + __ffs(bits) - 1;
+                        bits &= bits - 1;
+                        const ulonglong2 v = __ldg(t1 + s);
+                        a0 += v.x; a1 += v.y;
+                        if (!NO_NA) { const ulonglong2 z = __ldg(t0 + s); b0 += z.x; b1 += z.y; }
                     }
                 }
             }
@@ -289,36 +319,106 @@ k_test_chi2_sp(const uint4 *__restrict__ matrix, unsigned long long U, int wq, i
             if (!live) continue;
             // lane j of the group finishes columns c0 + j, c0 + j + lpr, ...
             for (int j = (int)sub; j < CHI2_SP_COLS && c0 + j < P; j += lpr) {
-                const int ph = c0 + j;
                 const int sh = 12 * (j % 5);
                 const uint32_t fa = (uint32_t)(((j < 5 ? a0 : a1) >> sh) & 4095ull);
-                const uint32_t ai = dense ? (uint32_t)tot1[ph] - fa : fa;
-                uint32_t ci;
-                if (NO_NA) ci = np - ai;
-                else {
-                    const uint32_t fb = (uint32_t)(((j < 5 ? b0 : b1) >> sh) & 4095ull);
-                    ci = dense ? (uint32_t)tot0[ph] - fb : fb;
+                const uint32_t fb = NO_NA ? 0u : (uint32_t)(((j < 5 ? b0 : b1) >> sh) & 4095ull);
+                chi2_sp_finish<NO_NA>(c0 + j, r, fa, fb, np, dense, tot1, tot0, reach, chi2_min, thr, out);
+            }
+        }
+    }
+}
+
+// The ten 12-bit fields of (x0, x1) as five u32 of two 16-bit fields: field j in p[j / 2] at bit 16 (j % 2).
+// A lane's own fields are at most 256 (its words' bits), the warp's sums at most 4,095: no field carries.
+__device__ __forceinline__ void fields16(unsigned long long x0, unsigned long long x1, uint32_t (&p)[5]) {
+    const auto two = [](uint32_t v) { return (v & 0xFFFu) | ((v << 4) & 0xFFF0000u); };
+    p[0] = two((uint32_t)x0);
+    p[1] = two((uint32_t)(x0 >> 24));
+    p[2] = (uint32_t)(x0 >> 48) | (((uint32_t)x1 & 0xFFFu) << 16);
+    p[3] = two((uint32_t)(x1 >> 12));
+    p[4] = two((uint32_t)(x1 >> 36));
+#pragma unroll
+    for (int i = 0; i < 5; i++) p[i] = __reduce_add_sync(0xffffffffu, p[i]);
+}
+
+// Rows that fill the warp (N > 2,048): lane l owns the 32-bit words l, l + 32, ... of the row, KW =
+// ceil(W / 32) of them for the W words that hold samples, so no lane has more than one word more than another
+// and each warp load is one 128-byte line. A lane walks all bits of all its words in ONE loop — when the current
+// word is empty it takes the next non-empty one — so the warp runs max over lanes of the lane's bit count, not
+// the sum over words of the per-word maxima. The fields are summed over the warp by REDUX (five u32 of two 16-bit
+// fields) instead of twenty shuffles and adds; every lane gets every sum and lane j finishes column c0 + j.
+template <int KW, bool NO_NA>
+__global__ void __launch_bounds__(256, 3)
+k_test_chi2_sp_warp(const uint32_t *__restrict__ matrix, unsigned long long U, int wp, int P, int n_samples,
+                    const ulonglong2 *__restrict__ e1, const ulonglong2 *__restrict__ e0, int npad,
+                    const int *__restrict__ tot1, const int *__restrict__ tot0, const int2 *__restrict__ reach,
+                    int np_lo, int np_hi, double thr, SurvOut out) {
+    __shared__ uint32_t s_valid[KW * 32];    // s_valid[wi]: the bits of row word wi that are samples
+    const int lane = (int)(threadIdx.x & 31);
+    const int wv = (n_samples + 31) >> 5;
+    for (int wi = threadIdx.x; wi < KW * 32; wi += blockDim.x) {
+        const int left = n_samples - wi * 32;
+        s_valid[wi] = left >= 32 ? 0xFFFFFFFFu : left <= 0 ? 0u : (1u << left) - 1u;
+    }
+    __syncthreads();
+    const unsigned long long warp_g = ((unsigned long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const unsigned long long nwarps = ((unsigned long long)gridDim.x * blockDim.x) >> 5;
+    const double chi2_min = thr > 0.0 ? -2.0 * log(thr) : 1e300;
+    // the next row is loaded before this one is walked, as in k_test_chi2_sp
+    auto load_row = [&](unsigned long long rr, uint32_t (&dst)[KW]) {
+#pragma unroll
+        for (int k = 0; k < KW; k++) {
+            const int wi = lane + 32 * k;
+            dst[k] = (rr < U && wi < wv) ? __ldg(matrix + rr * (unsigned long long)wp + wi) : 0u;
+        }
+    };
+    uint32_t nxt[KW];
+    load_row(warp_g, nxt);
+    for (unsigned long long r = warp_g; r < U; r += nwarps) {
+        uint32_t w[KW];
+#pragma unroll
+        for (int k = 0; k < KW; k++) w[k] = nxt[k];
+        load_row(r + nwarps, nxt);
+        uint32_t np = 0;
+#pragma unroll
+        for (int k = 0; k < KW; k++) np += __popc(w[k]);
+        np = __reduce_add_sync(0xffffffffu, np);
+        if ((int)np < np_lo || (int)np > np_hi) continue;
+        const bool dense = 2u * np > (uint32_t)n_samples;      // walk the cleared bits of the valid samples instead
+        if (dense) {
+#pragma unroll
+            for (int k = 0; k < KW; k++) w[k] = ~w[k] & s_valid[lane + 32 * k];
+        }
+        uint32_t nz = 0;                                         // bit k: word k has bits to walk
+#pragma unroll
+        for (int k = 0; k < KW; k++) nz |= (w[k] != 0u ? 1u : 0u) << k;
+        for (int c0 = 0; c0 < P; c0 += CHI2_SP_COLS) {
+            const ulonglong2 *t1 = e1 + (size_t)(c0 / CHI2_SP_COLS) * npad;
+            const ulonglong2 *t0 = NO_NA ? nullptr : e0 + (size_t)(c0 / CHI2_SP_COLS) * npad;
+            unsigned long long a0 = 0, a1 = 0, b0 = 0, b1 = 0;
+            uint32_t cur = 0, more = nz;
+            int s0 = 0;
+            while (cur | more) {
+                if (cur == 0u) {
+                    const int k = __ffs(more) - 1;
+                    more &= more - 1u;
+                    cur = pick_reg(w, k);
+                    s0 = (lane + 32 * k) * 32;
                 }
-                const uint32_t n_with = ai + ci;
-                const int n_without = totn[ph] - (int)n_with;
-                if ((int)n_with < min_s || n_without < 2 || (int)n_with > max_s) continue;
-                // from here on: the arithmetic of k_test_chi2 (unweighted), operation for operation
-                const double a = (double)ai, c = (double)ci;
-                const double b = (double)tot1[ph] - a, d = (double)tot0[ph] - c;
-                const double w_pheno = a + b, wo_pheno = c + d, w_kmer = a + c, wo_kmer = b + d;
-                const double total = w_pheno + wo_pheno;
-                {
-                    const double det = a * d - b * c;
-                    const double approx = total * det * det / ((w_pheno * wo_pheno) * (w_kmer * wo_kmer));
-                    if (approx < 0.99 * chi2_min) continue;
-                }
-                const double ea = (w_pheno * w_kmer) / total, eb = (w_pheno * wo_kmer) / total;
-                const double ec = (wo_pheno * w_kmer) / total, ed = (wo_pheno * wo_kmer) / total;
-                const double ta = (a - ea) * (a - ea) / ea, tb = (b - eb) * (b - eb) / eb;
-                const double tc = (c - ec) * (c - ec) / ec, td = (d - ed) * (d - ed) / ed;
-                const double chi2 = ((ta + tb) + tc) + td;
-                const double p = exp(-0.5 * chi2);
-                if (p < thr) surv_push(out, ph, r, chi2, p, 0.0, 0.0, n_with);  // NaN compares false
+                const int s = s0 + __ffs(cur) - 1;
+                cur &= cur - 1u;
+                const ulonglong2 v = __ldg(t1 + s);
+                a0 += v.x; a1 += v.y;
+                if (!NO_NA) { const ulonglong2 z = __ldg(t0 + s); b0 += z.x; b1 += z.y; }
+            }
+            uint32_t fa[5], fb[5];
+            fields16(a0, a1, fa);
+            if (!NO_NA) fields16(b0, b1, fb);
+            if (lane < CHI2_SP_COLS && c0 + lane < P) {
+                const int sh = 16 * (lane & 1);
+                const uint32_t ca = (pick_reg(fa, lane >> 1) >> sh) & 0xFFFFu;
+                const uint32_t cb = NO_NA ? 0u : (pick_reg(fb, lane >> 1) >> sh) & 0xFFFFu;
+                chi2_sp_finish<NO_NA>(c0 + lane, r, ca, cb, np, dense, tot1, tot0, reach, chi2_min, thr, out);
             }
         }
     }
