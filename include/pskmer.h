@@ -251,6 +251,33 @@ int ps_ipc_close_all(ps_ctx *ctx);
  */
 int ps_sample_quantiles(ps_ctx *ctx, int idx, int nq, uint64_t *out);
 
+/*
+ * -w sample weights (Mash distances + neighbour joining + GSC, modeling.py:386-503) on the device.
+ *
+ * Part 1: MinHash sketches of samples first_idx..first_idx+count-1 from their decoded streams (samples must be
+ * present; any job k / cutoff; FASTQ and cutoff > 1 samples keep their streams too): the s smallest distinct h1 of
+ * MurmurHash3_x64_128(seed) over the upper-case text of every canonical k-mer, as `mash sketch -r -k k -s s -S seed`.
+ * hashes[i*s + j] ascending, n_hashes[i] <= s (entries past n_hashes[i] are 0). k 1..32, s 1..4096.
+ * Replaces: Samples.get_mash_sketches -> `mash sketch -r` (modeling.py:386-390).
+ */
+int ps_mash_sketch(ps_ctx *ctx, int first_idx, int count, int k, int s, uint32_t seed,
+                   uint64_t *hashes, uint32_t *n_hashes);
+/*
+ * Part 2: shared_denom[i*n + j] = shared << 16 | denom for all ordered pairs of n sketches laid out as
+ * ps_mash_sketch returns them (host or device input): denom = min(s, |A u B|), shared = elements of A n B among the
+ * denom smallest of A u B. Replaces: `mash paste` + `mash dist` (modeling.py:404-412).
+ */
+int ps_mash_pairs(ps_ctx *ctx, int n, int s, const uint64_t *hashes, const uint32_t *n_hashes,
+                  uint32_t *shared_denom);
+/*
+ * Part 3: neighbour joining (Biopython 1.76 as restated in weights.py) on a symmetric n x n FP64 matrix (host or
+ * device), n 3..65535. join[2t], join[2t+1] = list positions (mi, mj) joined at step t < n-2; branch[2t],
+ * branch[2t+1] = their branch lengths; branch[2(n-2)] = the last remaining distance.
+ * Replaces: DistanceTreeConstructor.nj (modeling.py:446-452).
+ * None of the three touches the job's union, matrix, survivors or k-mer range.
+ */
+int ps_neighbor_joining(ps_ctx *ctx, int n, const double *dm, int32_t *join, double *branch);
+
 /* Instrumentation: the CUDA stream all work runs on; kernel launch counter; per-kernel
  * CUDA-event timing (enable, run, then read name / launches / total ms per kernel). */
 void *ps_stream(ps_ctx *ctx);

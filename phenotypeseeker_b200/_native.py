@@ -57,6 +57,12 @@ SIGNATURES = {
     "ps_ipc_open": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_char_p, c_void_pp]),
     "ps_ipc_close_all": (ctypes.c_int, [ctypes.c_void_p]),
     "ps_sample_quantiles": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, c_u64_p]),
+    "ps_mash_sketch": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                      ctypes.c_uint32, ctypes.c_void_p, ctypes.c_void_p]),
+    "ps_mash_pairs": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
+                                     ctypes.c_void_p]),
+    "ps_neighbor_joining": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
+                                           ctypes.c_void_p]),
     "ps_stream": (ctypes.c_void_p, [ctypes.c_void_p]),
     "ps_launch_count": (ctypes.c_uint64, [ctypes.c_void_p]),
     "ps_profile_enable": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
@@ -339,6 +345,34 @@ class Context:
         out = (ctypes.c_uint64 * max(nq - 1, 1))()
         self._ck(self.L.ps_sample_quantiles(self.h, int(idx), int(nq), out))
         return [int(out[i]) for i in range(nq - 1)]
+
+    # -- -w sample weights --------------------------------------------------------------
+    def mash_sketch(self, first_idx, count, k=21, s=1000, seed=42):
+        """MinHash sketches of samples first_idx..first_idx+count-1 -> (count x s uint64, count uint32 lengths);
+        row i holds its n[i] ascending hashes first, zeros after them."""
+        h = np.empty((int(count), int(s)), dtype=np.uint64)
+        n = np.empty(int(count), dtype=np.uint32)
+        self._ck(self.L.ps_mash_sketch(self.h, int(first_idx), int(count), int(k), int(s), int(seed), _ptr(h), _ptr(n)))
+        return h, n
+
+    def mash_pairs(self, hashes, n_hashes):
+        """hashes: n x s uint64 (as mash_sketch returns them), n_hashes: n -> n x n uint32, shared << 16 | denom."""
+        h = np.ascontiguousarray(hashes, dtype=np.uint64)
+        nh = np.ascontiguousarray(n_hashes, dtype=np.uint32)
+        n, s = h.shape
+        out = np.empty((n, n), dtype=np.uint32)
+        self._ck(self.L.ps_mash_pairs(self.h, n, s, _ptr(h), _ptr(nh), _ptr(out)))
+        return out
+
+    def neighbor_joining(self, dm):
+        """dm: n x n symmetric float64, n >= 3 -> (join: (n-2) x 2 int32 list positions (mi, mj) per step,
+        branch: 2(n-2)+1 float64, the two branch lengths of every step and the last remaining distance)."""
+        d = np.ascontiguousarray(dm, dtype=np.float64)
+        n = d.shape[0]
+        join = np.empty((max(n - 2, 0), 2), dtype=np.int32)
+        branch = np.empty(2 * max(n - 2, 0) + 1, dtype=np.float64)
+        self._ck(self.L.ps_neighbor_joining(self.h, n, _ptr(d), _ptr(join), _ptr(branch)))
+        return join, branch
 
     # -- instrumentation ---------------------------------------------------------------
     def stream(self):

@@ -12,6 +12,7 @@
 #include "ps_rows.cuh"
 #include "ps_test.cuh"
 #include "ps_chi2_reach.h"
+#include "ps_mash.cuh"
 
 static std::string g_create_err;
 
@@ -1077,6 +1078,8 @@ int ps_ctx_create(int device, ps_ctx **out) {
     PS_BKPG_ATTR(BK_THREADS, true) PS_BKPG_ATTR(BK_THREADS, false) PS_BKPG_ATTR(BK_MAX_THREADS, true) PS_BKPG_ATTR(BK_MAX_THREADS, false)
 #undef PS_BKPG_ATTR
     cudaFuncSetAttribute(k_bucket_count_pg<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    cudaFuncSetAttribute(k_mash_sketch, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mash_smem(PSM_S_MAX));
+    cudaFuncSetAttribute(k_mash_merge, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mash_smem(PSM_S_MAX));
     cudaFuncSetAttribute(k_bucket_count_pg<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     if (const char *ev = getenv("PSKMER_BK_TMA")) c->bk_tma = atoi(ev) != 0;
     if (const char *ev = getenv("PSKMER_PAGED")) c->paged = atoi(ev) != 0;
@@ -1988,3 +1991,138 @@ int ps_profile_reset(ps_ctx *c) {
 }
 
 }  // extern "C"
+
+// ---- -w sample weights: MinHash sketches, pair counts, neighbour joining (ps_mash.cuh) ----------------------------
+int ps_mash_sketch(ps_ctx *c, int first_idx, int count, int k, int s, uint32_t seed, uint64_t *hashes,
+                   uint32_t *n_hashes) {
+    API_BEGIN(c)
+    if (k < 1 || k > 32) PS_THROW(PS_ERR_ARG, "sketch k-mer length %d outside 1..32", k);
+    if (s < 1 || s > PSM_S_MAX) PS_THROW(PS_ERR_ARG, "sketch size %d outside 1..%d", s, PSM_S_MAX);
+    if (count < 1 || first_idx < 0 || first_idx + count > c->n_samples)
+        PS_THROW(PS_ERR_ARG, "samples %d..%d outside the job's 0..%d", first_idx, first_idx + count - 1, c->n_samples - 1);
+    if (!hashes || !n_hashes) PS_THROW(PS_ERR_ARG, "null argument");
+    std::vector<uint64_t> tab(2 * (size_t)count);
+    uint64_t total = 0, longest = 0;
+    for (int i = 0; i < count; i++) {
+        const SampleInfo &si = c->samples[first_idx + i];
+        if (!si.present) PS_THROW(PS_ERR_ARG, "sample %d is not present", first_idx + i);
+        tab[i] = si.pos_off;
+        tab[count + i] = si.n_pos;
+        total += si.n_pos;
+        longest = std::max(longest, si.n_pos);
+    }
+    // chunks of the streams: about 16 blocks per SM over all samples, at most 1 GB of chunk lists
+    uint64_t chunk = round_up<uint64_t>(std::max<uint64_t>(total / (16 * PS_SMS), 1), MASH_ROUND);
+    chunk = std::min<uint64_t>(std::max<uint64_t>(chunk, 16 * MASH_ROUND), 1024 * MASH_ROUND);
+    while ((uint64_t)count * ceil_div<uint64_t>(longest, chunk) * s * 8 > (1ull << 30)) chunk *= 2;
+    const int n_chunks = (int)ceil_div<uint64_t>(longest, chunk);
+    const int cap = mash_cap(s);
+    c->mash_tab.reserve(tab.size() * 8, c->stream);
+    c->mash_parts.reserve((size_t)count * n_chunks * s * 8, c->stream);
+    c->mash_parts_n.reserve((size_t)count * n_chunks * 4, c->stream);
+    c->mash_h.reserve((size_t)count * s * 8, c->stream);
+    c->mash_n.reserve((size_t)count * 4, c->stream);
+    CK(cudaMemcpyAsync(c->mash_tab.p, tab.data(), tab.size() * 8, cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemsetAsync(c->mash_h.p, 0, (size_t)count * s * 8, c->stream));
+    const uint64_t *d_off = c->mash_tab.as<uint64_t>(), *d_npos = d_off + count;
+    KLAUNCH(c, "mash_sketch", (double)total * 3 / 8,
+            (k_mash_sketch<<<dim3(n_chunks, count), MASH_THREADS, mash_smem(s), c->stream>>>(
+                c->pool_seq.as<uint32_t>(), c->pool_bad.as<uint32_t>(), d_off, d_npos, n_chunks, chunk, k, s, cap, seed,
+                c->mash_parts.as<uint64_t>(), c->mash_parts_n.as<uint32_t>())));
+    KLAUNCH(c, "mash_merge", (double)count * n_chunks * s * 8,
+            (k_mash_merge<<<count, MASH_THREADS, mash_smem(s), c->stream>>>(
+                c->mash_parts.as<uint64_t>(), c->mash_parts_n.as<uint32_t>(), n_chunks, s, cap, c->mash_h.as<uint64_t>(),
+                c->mash_n.as<uint32_t>())));
+    CK(cudaMemcpyAsync(hashes, c->mash_h.p, (size_t)count * s * 8, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(n_hashes, c->mash_n.p, (size_t)count * 4, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    API_END(c)
+}
+
+int ps_mash_pairs(ps_ctx *c, int n, int s, const uint64_t *hashes, const uint32_t *n_hashes, uint32_t *shared_denom) {
+    API_BEGIN(c)
+    if (n < 1 || n > 65535) PS_THROW(PS_ERR_ARG, "number of sketches %d outside 1..65535", n);
+    if (s < 1 || s > PSM_S_MAX) PS_THROW(PS_ERR_ARG, "sketch size %d outside 1..%d", s, PSM_S_MAX);
+    if (!hashes || !n_hashes || !shared_denom) PS_THROW(PS_ERR_ARG, "null argument");
+    c->mash_h.reserve((size_t)n * s * 8, c->stream);
+    c->mash_n.reserve((size_t)n * 4, c->stream);
+    c->mash_sd.reserve((size_t)n * n * 4, c->stream);
+    std::vector<uint32_t> hn(n);
+    CK(cudaMemcpyAsync(hn.data(), n_hashes, (size_t)n * 4, cudaMemcpyDefault, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    for (int i = 0; i < n; i++)
+        if (hn[i] > (uint32_t)s) PS_THROW(PS_ERR_ARG, "sketch %d holds %u hashes, more than s = %d", i, hn[i], s);
+    CK(cudaMemcpyAsync(c->mash_h.p, hashes, (size_t)n * s * 8, cudaMemcpyDefault, c->stream));
+    CK(cudaMemcpyAsync(c->mash_n.p, hn.data(), (size_t)n * 4, cudaMemcpyHostToDevice, c->stream));
+    KLAUNCH(c, "mash_pairs", (double)n * (n + 1) / 2 * s * 8,
+            (k_mash_pairs<<<dim3(ceil_div(n, 256), n), 256, (size_t)s * 8, c->stream>>>(
+                c->mash_h.as<uint64_t>(), c->mash_n.as<uint32_t>(), n, s, c->mash_sd.as<uint32_t>())));
+    CK(cudaMemcpyAsync(shared_denom, c->mash_sd.p, (size_t)n * n * 4, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    API_END(c)
+}
+
+int ps_neighbor_joining(ps_ctx *c, int n, const double *dm, int32_t *join, double *branch) {
+    API_BEGIN(c)
+    if (n < 3 || n > 65535) PS_THROW(PS_ERR_ARG, "neighbour joining needs 3..65535 taxa, got %d", n);
+    if (!dm || !join || !branch) PS_THROW(PS_ERR_ARG, "null argument");
+    const size_t nn = (size_t)n * n;
+    std::vector<double> hd;
+    const double *h = dm;
+    cudaPointerAttributes pa;
+    if (cudaPointerGetAttributes(&pa, dm) == cudaSuccess && pa.type == cudaMemoryTypeDevice) {
+        hd.resize(nn);
+        CK(cudaMemcpy(hd.data(), dm, nn * 8, cudaMemcpyDeviceToHost));
+        h = hd.data();
+    }
+    cudaGetLastError();
+    for (int i = 0; i < n; i++)
+        for (int j = 0; j < i; j++)
+            if (!(h[(size_t)i * n + j] == h[(size_t)j * n + i]))
+                PS_THROW(PS_ERR_ARG, "distance matrix is not symmetric at (%d, %d)", i, j);
+    c->nj_d.reserve(nn * 8, c->stream);
+    c->nj_act.reserve((size_t)2 * n * 4, c->stream);
+    c->nj_nd.reserve((size_t)n * 8, c->stream);
+    const int part_max = 4 * PS_SMS;
+    c->nj_part.reserve((size_t)part_max * sizeof(NjBest), c->stream);
+    c->nj_out.reserve((size_t)2 * n * 8 + (size_t)2 * n * 4, c->stream);
+    std::vector<int> iota(n);
+    std::iota(iota.begin(), iota.end(), 0);
+    CK(cudaMemcpyAsync(c->nj_d.p, dm, nn * 8, cudaMemcpyDefault, c->stream));
+    CK(cudaMemcpyAsync(c->nj_act.p, iota.data(), (size_t)n * 4, cudaMemcpyHostToDevice, c->stream));
+    int *act = c->nj_act.as<int>(), *act_next = act + n;
+    double *d_branch = c->nj_out.as<double>();
+    int32_t *d_join = reinterpret_cast<int32_t *>(d_branch + 2 * (size_t)n);
+    size_t ld = n;
+    for (int m = n, step = 0; m > 2; m--, step++) {
+        if (m >= 512 && (size_t)m * 2 <= ld) {        // most slots are dead: copy the live rows and columns together
+            c->nj_d2.reserve((size_t)m * m * 8, c->stream);
+            KLAUNCH(c, "nj_compact", (double)m * m * 16,
+                    (k_nj_compact<<<dim3(ceil_div(m, 256), m), 256, 0, c->stream>>>(c->nj_d.as<double>(), ld, act, m,
+                                                                                   c->nj_d2.as<double>())));
+            std::swap(c->nj_d, c->nj_d2);
+            ld = m;
+            CK(cudaMemcpyAsync(act, iota.data(), (size_t)m * 4, cudaMemcpyHostToDevice, c->stream));
+        }
+        double *D = c->nj_d.as<double>();
+        KLAUNCH(c, "nj_rowsum", (double)m * m * 8,
+                (k_nj_rowsum<<<ceil_div(m, 32), 32, 0, c->stream>>>(D, ld, act, m, c->nj_nd.as<double>())));
+        const int n_part = std::min(ceil_div(m - 1, 8), part_max);
+        KLAUNCH(c, "nj_argmin", (double)m * (m - 1) / 2 * 8,
+                (k_nj_argmin<<<n_part, 256, 0, c->stream>>>(D, ld, act, m, c->nj_nd.as<double>(), c->nj_part.as<NjBest>())));
+        KLAUNCH(c, "nj_update", (double)m * 32,
+                (k_nj_update<<<ceil_div(m, 256), 256, 0, c->stream>>>(D, ld, act, act_next, m, c->nj_nd.as<double>(),
+                                                                      c->nj_part.as<NjBest>(), n_part, step, d_join,
+                                                                      d_branch)));
+        std::swap(act, act_next);
+    }
+    int last[2];
+    CK(cudaMemcpyAsync(last, act, 8, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    CK(cudaMemcpyAsync(branch + 2 * (size_t)(n - 2), c->nj_d.as<double>() + (size_t)last[1] * ld + last[0], 8,
+                       cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(branch, d_branch, (size_t)2 * (n - 2) * 8, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(join, d_join, (size_t)2 * (n - 2) * 4, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    API_END(c)
+}

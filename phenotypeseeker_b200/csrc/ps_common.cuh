@@ -169,6 +169,8 @@ struct ps_ctx {
     DevBuf sel_ph, sel_row, sel_stat, sel_p, sel_mx, sel_my, sel_n;   // ps_select_top
     DevBuf tmp1, tmp2, tmp3;
     DevBuf pg_meta_a, pg_meta_b, pg_plist, pg_tiles, pg_tabs, pg_state, pg_blist;   // paged partition
+    DevBuf mash_tab, mash_parts, mash_parts_n, mash_h, mash_n, mash_sd;              // ps_mash_sketch / ps_mash_pairs
+    DevBuf nj_d, nj_d2, nj_act, nj_nd, nj_part, nj_out;                              // ps_neighbor_joining
 
     void *pinned = nullptr;  // small pinned scratch for readbacks
     size_t pinned_cap = 0;
@@ -184,7 +186,9 @@ struct ps_ctx {
                 &tags_a, &tags_b, &hist, &lookback, &uni, &matrix, &ph_masks, &ph_vals, &ph_tot,
                 &weights, &sv_ph, &sv_row, &sv_stat, &sv_p, &sv_mx, &sv_my, &sv_n, &sv_perm,
                 &sv_bits, &sv_kmer, &tmp1, &tmp2, &tmp3, &pg_meta_a, &pg_meta_b, &pg_plist, &pg_tiles,
-                &pg_tabs, &pg_state, &pg_blist, &sel_ph, &sel_row, &sel_stat, &sel_p, &sel_mx, &sel_my, &sel_n};
+                &pg_tabs, &pg_state, &pg_blist, &sel_ph, &sel_row, &sel_stat, &sel_p, &sel_mx, &sel_my, &sel_n,
+                &mash_tab, &mash_parts, &mash_parts_n, &mash_h, &mash_n, &mash_sd, &nj_d, &nj_d2, &nj_act, &nj_nd,
+                &nj_part, &nj_out};
     }
 };
 

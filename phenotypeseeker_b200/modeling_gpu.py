@@ -152,13 +152,18 @@ def run_hot_path(files, sample_names, k, cutoff, pheno, pheno_names, binary, wei
 def install(m, device=None, native_weights=None):
     """Re-wire the reference module `m` (PhenotypeSeeker.modeling) onto the GPU path.
 
-    native_weights (default: env PS_NATIVE_WEIGHTS=1): also replace the `-w` weight computation
+    native_weights (default: env PS_NATIVE_WEIGHTS): also replace the `-w` weight computation
     (`Samples.get_mash_sketches` / `get_weights`, modeling.py:386-503: mash binary + Biopython + ete3) with
     phenotypeseeker_b200.weights — for installations without those three; see that module for what is
-    pinned against the reference and what is not."""
+    pinned against the reference and what is not. True / "1": on the host, from the sample files. "gpu": sketches,
+    distances and neighbour joining on the device, from the samples get_feature_vector decoded (same weights on
+    well-formed FASTA / FASTQ; the text is read as the k-mer counter reads it, DESIGN.md "Reader semantics")."""
     Input, Samples, phenotypes = m.Input, m.Samples, m.phenotypes
     if native_weights is None:
-        native_weights = os.environ.get("PS_NATIVE_WEIGHTS", "0") == "1"
+        env = os.environ.get("PS_NATIVE_WEIGHTS", "0")
+        native_weights = "gpu" if env == "gpu" else env == "1"
+    elif native_weights != "gpu":
+        native_weights = bool(native_weights)
 
     def get_kmer_lists(self):          # runs in Pool workers: nothing to do
         return None
@@ -240,8 +245,17 @@ def install(m, device=None, native_weights=None):
     def get_weights(cls):
         from . import weights as psw
         samples = list(Input.samples.values())
-        w = psw.gsc_weights_for_samples([s.name for s in samples], [read_sample_file(s.address) for s in samples],
-                                        keep_glob_quirk=True)
+        names = [s.name for s in samples]
+        if native_weights == "gpu":
+            # the samples get_feature_vector decoded are still on the device; ingesting them again would start a
+            # new job and drop the union and matrix the tests need
+            if _STATE["names"] != names or _STATE["ka"] is None or _STATE["pid"] != os.getpid():
+                raise RuntimeError("native_weights='gpu' computes the weights from the samples get_feature_vector "
+                                   "decoded; call it first, with the same Input.samples")
+            w = psw.gsc_weights_on_device(_STATE["ka"].ctx, names, 0, keep_glob_quirk=True)
+        else:
+            w = psw.gsc_weights_for_samples(names, [read_sample_file(s.address) for s in samples],
+                                            keep_glob_quirk=True)
         for s, wi in zip(samples, w):
             s.weight = float(wi)
 

@@ -32,6 +32,7 @@ name. `gsc_weights_for_samples(..., keep_glob_quirk=True)` reproduces that; the 
 the distances correctly.
 """
 import math
+import sys
 
 import numpy as np
 
@@ -162,20 +163,34 @@ def mash_distance(a, b, k=MASH_K, s=MASH_S):
             denom += nb - j
         if denom > s:
             denom = s
+    return distance_from_counts(common, denom, k), common, denom
+
+
+def distance_from_counts(common, denom, k=MASH_K):
+    """The Mash distance of a sketch pair with `common` of its `denom` smallest union hashes shared."""
     if denom == 0 or common == denom:
-        d = 0.0
-    elif common == 0:
-        d = 1.0
-    else:
-        jac = common / denom
-        d = -math.log(2.0 * jac / (1.0 + jac)) / k
-    return d, common, denom
+        return 0.0
+    if common == 0:
+        return 1.0
+    jac = common / denom
+    return -math.log(2.0 * jac / (1.0 + jac)) / k
 
 
 def printed(x):
     """The value the reference reads back: mash prints distances with 6 significant digits
     (C++ ostream default) and modeling.py:421 parses that text."""
     return float("%g" % x)
+
+
+def printed_distances(shared_denom, k=MASH_K):
+    """N x N array of shared << 16 | denom (ps_mash_pairs) -> the printed distance matrix, through a table of
+    printed(distance) over the (shared, denom) pairs that occur: the same values as distance_matrix()."""
+    sd = np.asarray(shared_denom, dtype=np.uint32)
+    vals, inv = np.unique(sd, return_inverse=True)
+    table = np.array([printed(distance_from_counts(int(v) >> 16, int(v) & 0xFFFF, k)) for v in vals], dtype=np.float64)
+    dm = table[inv].reshape(sd.shape)
+    np.fill_diagonal(dm, 0.0)
+    return dm
 
 
 def distance_matrix(sketches, k=MASH_K, s=MASH_S):
@@ -200,26 +215,40 @@ class Node:
         self.children.append(child)
 
 
-def neighbor_joining(names, dm):
-    """Biopython 1.76 DistanceTreeConstructor.nj restated (see module docstring: unpinned).
-    names: N labels; dm: N x N symmetric. Returns the root Node (branch lengths in .dist)."""
+def _compensated_sum(xs):
+    """Python >= 3.12's sum() of floats (start 0): Neumaier's compensated summation, the compensation added at the
+    end when it is non-zero and finite. Restated for older interpreters, whose sum() adds left to right."""
+    it = iter(xs)
+    f, c = 0 + next(it), 0.0
+    for x in it:
+        t = f + x
+        if abs(f) >= abs(x):
+            c += (f - t) + x
+        else:
+            c += (x - t) + f
+        f = t
+    if c and math.isfinite(c):
+        f += c
+    return f
+
+
+# neighbour joining's row sums: what sum() gives on Python >= 3.12 (ps_neighbor_joining does the same on the device)
+_row_sum = sum if sys.version_info >= (3, 12) else _compensated_sum
+
+
+def nj_joins(dm):
+    """The loop of Biopython 1.76 DistanceTreeConstructor.nj (see module docstring: unpinned) on an N x N symmetric
+    matrix, N >= 3 -> (join, branch): join[t] = the list positions (mi, mj) joined at step t, branch[2t], branch[2t+1]
+    = their branch lengths, branch[-1] = the distance left between the last two nodes. Row sums are Python 3.12's
+    sum() on every interpreter (_row_sum). ps_neighbor_joining restates this bit for bit."""
     dm = [list(map(float, row)) for row in np.asarray(dm, dtype=np.float64)]
-    clades = [Node(nm) for nm in names]
-    n = len(clades)
-    if n == 1:
-        return clades[0]
-    if n == 2:
-        c1, c2 = clades[1], clades[0]
-        c1.dist = dm[1][0] / 2.0
-        c2.dist = dm[1][0] - c1.dist
-        root = Node("Inner")
-        root.add(c1); root.add(c2)
-        return root
-    inner = None
-    count = 0
+    n = len(dm)
+    join = np.empty((n - 2, 2), dtype=np.int32)
+    branch = np.empty(2 * (n - 2) + 1, dtype=np.float64)
+    step = 0
     while len(dm) > 2:
         m = len(dm)
-        nd = [sum(dm[i]) / (m - 2) for i in range(m)]
+        nd = [_row_sum(dm[i]) / (m - 2) for i in range(m)]
         min_dist = dm[1][0] - nd[1] - nd[0]
         mi, mj = 0, 1
         for i in range(1, m):
@@ -227,59 +256,92 @@ def neighbor_joining(names, dm):
                 t = dm[i][j] - nd[i] - nd[j]
                 if min_dist > t:
                     min_dist, mi, mj = t, i, j
-        c1, c2 = clades[mi], clades[mj]
-        count += 1
-        inner = Node("Inner" + str(count))
-        inner.add(c1); inner.add(c2)
-        c1.dist = (dm[mi][mj] + nd[mi] - nd[mj]) / 2.0
-        c2.dist = dm[mi][mj] - c1.dist
-        clades[mj] = inner
-        del clades[mi]
+        c1 = (dm[mi][mj] + nd[mi] - nd[mj]) / 2.0
+        join[step] = mi, mj
+        branch[2 * step], branch[2 * step + 1] = c1, dm[mi][mj] - c1
         for x in range(m):
             if x != mi and x != mj:
                 dm[mj][x] = dm[x][mj] = (dm[mi][x] + dm[mj][x] - dm[mi][mj]) / 2.0
         del dm[mi]
         for row in dm:
             del row[mi]
+        step += 1
+    branch[-1] = dm[1][0]
+    return join, branch
+
+
+def tree_from_joins(names, join, branch):
+    """Replays the list operations of nj_joins on the clades: inner nodes "Inner1", "Inner2", ... and the rooting of
+    the last two nodes (the last inner node stays the root when it is first in the list). Returns the root Node."""
+    clades = [Node(nm) for nm in names]
+    inner = None
+    for t, (mi, mj) in enumerate(np.asarray(join).tolist()):
+        c1, c2 = clades[mi], clades[mj]
+        inner = Node("Inner" + str(t + 1))
+        inner.add(c1); inner.add(c2)
+        c1.dist = float(branch[2 * t])
+        c2.dist = float(branch[2 * t + 1])
+        clades[mj] = inner
+        del clades[mi]
+    last = float(branch[-1])
     if clades[0] is inner:
         clades[0].dist = 0.0
-        clades[1].dist = dm[1][0]
+        clades[1].dist = last
         clades[0].add(clades[1])
-        root = clades[0]
-    else:
-        clades[0].dist = dm[1][0]
-        clades[1].dist = 0.0
-        clades[1].add(clades[0])
-        root = clades[1]
-    return root
+        return clades[0]
+    clades[0].dist = last
+    clades[1].dist = 0.0
+    clades[1].add(clades[0])
+    return clades[1]
+
+
+def neighbor_joining(names, dm):
+    """Biopython 1.76 DistanceTreeConstructor.nj restated (see module docstring: unpinned).
+    names: N labels; dm: N x N symmetric. Returns the root Node (branch lengths in .dist)."""
+    n = len(names)
+    if n == 1:
+        return Node(names[0])
+    if n == 2:
+        d = float(np.asarray(dm, dtype=np.float64)[1][0])
+        c1, c2 = Node(names[1]), Node(names[0])
+        c1.dist = d / 2.0
+        c2.dist = d - c1.dist
+        root = Node("Inner")
+        root.add(c1); root.add(c2)
+        return root
+    return tree_from_joins(names, *nj_joins(dm))
 
 
 def newick(node):
     """Bio.Phylo's Newick writer: names + "%1.5f" branch lengths (the reference converts the
-    phyloxml tree to Newick before handing it to ete3, modeling.py:454-458)."""
-    label = (node.name or "") + ":%1.5f" % node.dist
-    if node.children:
-        return "(" + ",".join(newick(c) for c in node.children) + ")" + label
-    return label
+    phyloxml tree to Newick before handing it to ete3, modeling.py:454-458). Iterative, so that
+    trees thousands of levels deep (a caterpillar from N = 5,000 samples) can be written."""
+    out, stack = [], [node]
+    while stack:
+        it = stack.pop()
+        if isinstance(it, str):
+            out.append(it)
+            continue
+        label = (it.name or "") + ":%1.5f" % it.dist
+        if not it.children:
+            out.append(label)
+            continue
+        out.append("(")
+        stack.append(")" + label)
+        for i in range(len(it.children) - 1, -1, -1):
+            stack.append(it.children[i])
+            if i:
+                stack.append(",")
+    return "".join(out)
 
 
 def parse_newick(text):
-    """Minimal Newick reader (names + branch lengths, ete3 format=1 subset) -> root Node."""
+    """Minimal Newick reader (names + branch lengths, ete3 format=1 subset) -> root Node. Iterative, like newick()."""
     text = text.strip().rstrip(";")
     pos = 0
 
-    def parse():
+    def label(node):
         nonlocal pos
-        node = Node()
-        if text[pos] == "(":
-            pos += 1
-            while True:
-                node.add(parse())
-                if text[pos] == ",":
-                    pos += 1
-                    continue
-                pos += 1          # ')'
-                break
         start = pos
         while pos < len(text) and text[pos] not in ",():":
             pos += 1
@@ -290,9 +352,27 @@ def parse_newick(text):
             while pos < len(text) and text[pos] not in ",()":
                 pos += 1
             node.dist = float(text[start:pos])
-        return node
 
-    return parse()
+    open_nodes, root = [], None
+    while True:
+        node = Node()                      # a node begins at pos
+        if open_nodes:
+            open_nodes[-1].add(node)
+        else:
+            root = node
+        if text[pos] == "(":
+            pos += 1
+            open_nodes.append(node)
+            continue
+        label(node)
+        while True:                        # after a finished node: a sibling follows, or parents close
+            if not open_nodes:
+                return root
+            if text[pos] == ",":
+                pos += 1
+                break
+            pos += 1                       # ')'
+            label(open_nodes.pop())
 
 
 def gsc_weights(root, normalize="mean1", min_val=1e-9, max_val=1e9):
@@ -336,5 +416,24 @@ def gsc_weights_for_samples(names, texts, keep_glob_quirk=False, k=MASH_K, s=MAS
     order = sorted(names, key=lambda nm: nm + ".msh") if keep_glob_quirk else list(names)
     dm = distance_matrix([sk[nm] for nm in order], k, s)
     root = neighbor_joining(list(names), dm)          # rows are labelled in data.pheno order either way
+    w = gsc_weights(parse_newick(newick(root) + ";"))
+    return np.array([w[nm] for nm in names], dtype=np.float64)
+
+
+def gsc_weights_on_device(ctx, names, first_idx=0, keep_glob_quirk=False, k=MASH_K, s=MASH_S, seed=MASH_SEED):
+    """gsc_weights_for_samples for samples first_idx.. of a libpskmer context that already holds them (decoded by
+    ps_add_samples): sketches, pair counts and neighbour joining on the device, the distance table, the tree replay,
+    Newick and GSC here. Bit-identical to the host path on well-formed FASTA / FASTQ; the device reads the text as
+    the k-mer counter does (DESIGN.md "Reader semantics"), which differs on bytes 1-31 inside a sequence and on U."""
+    n = len(names)
+    h, nh = ctx.mash_sketch(first_idx, n, k, s, seed)
+    if keep_glob_quirk:                               # see gsc_weights_for_samples
+        order = sorted(range(n), key=lambda i: names[i] + ".msh")
+        h, nh = h[order], nh[order]
+    dm = printed_distances(ctx.mash_pairs(h, nh), k)
+    if n >= 3:
+        root = tree_from_joins(list(names), *ctx.neighbor_joining(dm))
+    else:
+        root = neighbor_joining(list(names), dm)
     w = gsc_weights(parse_newick(newick(root) + ";"))
     return np.array([w[nm] for nm in names], dtype=np.float64)
