@@ -237,6 +237,12 @@ uint64_t ps_instances_upper(ps_ctx *ctx);
 int ps_route_setup(ps_ctx *ctx, int nparts, int my_rank, const uint64_t *splitters, uint64_t pages_per_sender,
                    void **pool_ptr, void **meta_ptr);
 int ps_route_peers(ps_ctx *ctx, int nparts, void *const *pool_ptrs, void *const *meta_ptrs);
+/* One process, several contexts (one per rank, any devices): register the receive pools of ranks[0..nparts-1]
+ * (ranks[d] has done ps_route_setup(nparts, d, ...); ranks[my_rank] == ctx) and enable peer access from ctx's
+ * device to every other device among them. Call after every rank's ps_route_setup, before ps_route_begin.
+ * PS_ERR_STATE: a rank set up with another nparts or rank index, or without a pool; PS_ERR_ARG: more than
+ * PART_MAX ranks, or two devices without peer access. */
+int ps_route_connect(ps_ctx *ctx, int nparts, ps_ctx *const *ranks);
 int ps_route_begin(ps_ctx *ctx);
 int ps_route_scatter(ps_ctx *ctx);
 int ps_route_build(ps_ctx *ctx, uint64_t *n_union, int *overflow);

@@ -50,6 +50,7 @@ SIGNATURES = {
     "ps_route_setup": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, c_u64_p, ctypes.c_uint64, c_void_pp,
                                       c_void_pp]),
     "ps_route_peers": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, c_void_pp, c_void_pp]),
+    "ps_route_connect": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, c_void_pp]),
     "ps_route_begin": (ctypes.c_int, [ctypes.c_void_p]),
     "ps_route_scatter": (ctypes.c_int, [ctypes.c_void_p]),
     "ps_route_build": (ctypes.c_int, [ctypes.c_void_p, c_u64_p, ctypes.POINTER(ctypes.c_int)]),
@@ -314,6 +315,13 @@ class Context:
         pp = (ctypes.c_void_p * n)(*[int(x) for x in pool_ptrs])
         mp = (ctypes.c_void_p * n)(*[int(x) for x in meta_ptrs])
         self._ck(self.L.ps_route_peers(self.h, n, pp, mp))
+
+    def route_connect(self, contexts):
+        """Pools of every rank of one process (contexts[r] is rank r, this context among them), with peer access
+        from this context's device to the others' (ps_route_connect)."""
+        n = len(contexts)
+        hs = (ctypes.c_void_p * n)(*[c.h.value if c.h else None for c in contexts])
+        self._ck(self.L.ps_route_connect(self.h, n, hs))
 
     def route_begin(self):
         self._ck(self.L.ps_route_begin(self.h))

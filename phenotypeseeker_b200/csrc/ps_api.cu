@@ -1791,6 +1791,36 @@ int ps_route_peers(ps_ctx *c, int nparts, void *const *pool_ptrs, void *const *m
     API_END(c)
 }
 
+int ps_route_connect(ps_ctx *c, int nparts, ps_ctx *const *ranks) {
+    API_BEGIN(c)
+    if (nparts < 1 || nparts > PART_MAX) PS_THROW(PS_ERR_ARG, "nparts must be 1..%d", PART_MAX);
+    if (!ranks) PS_THROW(PS_ERR_ARG, "null rank table");
+    if (nparts != c->route_n) PS_THROW(PS_ERR_STATE, "ps_route_setup with the same nparts first");
+    if (ranks[c->route_rank] != c) PS_THROW(PS_ERR_ARG, "ranks[%d] must be this context", c->route_rank);
+    for (int d = 0; d < nparts; d++) {
+        const ps_ctx *r = ranks[d];
+        if (!r) PS_THROW(PS_ERR_ARG, "null context of rank %d", d);
+        if (r->route_n != nparts || r->route_rank != d)
+            PS_THROW(PS_ERR_STATE, "context given as rank %d is set up as rank %d of %d", d, r->route_rank, r->route_n);
+        if (!r->route_pool[d] || r->route_pool[d] != r->keys_a.p || r->route_meta[d] != r->pg_meta_a.p)
+            PS_THROW(PS_ERR_STATE, "rank %d has no receive pool: ps_route_setup first", d);
+    }
+    // k_scatter1 stores straight into the other ranks' pools: every device among them must be reachable from
+    // this one before the first ps_route_scatter (plain cudaMalloc buffers: device-level peer access covers them)
+    for (int d = 0; d < nparts; d++) {
+        const int dev = ranks[d]->device;
+        if (dev == c->device) continue;
+        int ok = 0;
+        CK(cudaDeviceCanAccessPeer(&ok, c->device, dev));
+        if (!ok) PS_THROW(PS_ERR_ARG, "device %d cannot access device %d (no peer access between them)", c->device, dev);
+        const cudaError_t e = cudaDeviceEnablePeerAccess(dev, 0);
+        if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
+        else CK(e);
+    }
+    for (int d = 0; d < nparts; d++) { c->route_pool[d] = ranks[d]->route_pool[d]; c->route_meta[d] = ranks[d]->route_meta[d]; }
+    API_END(c)
+}
+
 static void route_check(ps_ctx *c) {
     if (c->route_n < 1) PS_THROW(PS_ERR_STATE, "ps_route_setup first");
     if (c->keys_a.p != c->route_pool[c->route_rank] || (uint64_t)c->route_n * c->route_pages != c->pgA_cap)

@@ -22,7 +22,15 @@ Exchange routes:
 Collectives per step: all_gather (pool sizes; sticky, so IPC handles move only when a pool grows),
 2 x all_reduce (barriers), all_reduce (U, the Bonferroni denominator, modeling.py:641-644, plus
 the pool-overflow flag), one all_gather of the packed survivors.
+
+The collectives go through a group object with torch.distributed's calls (all_reduce,
+all_gather_into_tensor, broadcast) plus the exchange of the receive pools:
+  * TorchGroup: one process per GPU (torchrun, NCCL); pools are mapped with CUDA IPC.
+  * ThreadGroup: one thread per rank inside one process (group.GpuGroup); pools are plain device
+    pointers of the other contexts, connected by ps_route_connect, which also enables peer access.
 """
+import threading
+
 import numpy as np
 
 from .pipeline import KmerAssociation, PhenoResult
@@ -101,7 +109,139 @@ def unpack_results(names, counts, buf, n_samples):
     return out
 
 
-_GATHER_CAP = {"bytes": 1 << 16}     # sticky capacity of the survivor all-gather (grows when a rank needs more)
+class PoolOverflow(RuntimeError):
+    """A receive page pool overflowed while routing k-mers. Every rank raises it at the same point and has doubled
+    its pools for the next step, which can simply be run again."""
+
+
+class TorchGroup:
+    """Collectives of one process per GPU: torch.distributed (NCCL), receive pools mapped with CUDA IPC. Lives for
+    the process (TORCH_GROUP), so the survivor all-gather keeps its sticky capacity from step to step."""
+
+    def __init__(self):
+        self.gather_cap = 1 << 16       # bytes per rank of the survivor all-gather (grows when a rank needs more)
+
+    def all_reduce(self, t):
+        import torch.distributed as dist
+        dist.all_reduce(t)
+
+    def all_gather_into_tensor(self, out, t):
+        import torch.distributed as dist
+        dist.all_gather_into_tensor(out, t)
+
+    def broadcast(self, t, src):
+        import torch.distributed as dist
+        dist.broadcast(t, src=src)
+
+    def connect_pools(self, ctx, rank, world, device, pool, meta):
+        """Every rank's receive pool into ctx's route (ps_route_peers), through CUDA IPC handles."""
+        import torch
+        h = np.frombuffer(ctx.ipc_export(pool) + ctx.ipc_export(meta), dtype=np.uint8).copy()
+        allh = torch.empty(world * 128, dtype=torch.uint8, device=device)
+        self.all_gather_into_tensor(allh, torch.from_numpy(h).to(device))
+        allh = allh.cpu().numpy().reshape(world, 128)
+        pools = [pool if d == rank else ctx.ipc_open(allh[d, :64].tobytes()) for d in range(world)]
+        metas = [meta if d == rank else ctx.ipc_open(allh[d, 64:].tobytes()) for d in range(world)]
+        ctx.route_peers(pools, metas)
+
+
+TORCH_GROUP = TorchGroup()
+
+
+class ThreadGroup:
+    """The collectives of TorchGroup for `world` threads of one process; rank r is the thread that run() started
+    for it. Data moves device to device (Tensor.copy_), never through the host.
+
+    Like NCCL's, a collective is ordered after the work queued on the caller's current stream: it synchronises that
+    stream (the library stream inside build_and_test) BEFORE it meets the other ranks, so that, used as a barrier,
+    no rank scatters into a pool whose ps_route_begin memset is still queued. It synchronises again after reading the
+    other ranks' tensors and meets them once more, so no rank reuses a tensor another one is still reading.
+
+    When a rank raises, run() aborts the barrier: the other ranks get BrokenBarrierError instead of waiting forever,
+    and run() re-raises the first error in the caller."""
+
+    def __init__(self, world):
+        self.world = int(world)
+        self.gather_cap = 1 << 16
+        self._slots = [None] * self.world
+        self._local = threading.local()
+        self._bar = threading.Barrier(self.world)
+
+    def run(self, fn):
+        """fn(rank) on one thread per rank; every thread is joined before this returns. -> [result per rank]."""
+        self._bar = threading.Barrier(self.world)
+        out, errs, lock = [None] * self.world, [], threading.Lock()
+
+        def body(r):
+            self._local.rank = r
+            try:
+                out[r] = fn(r)
+            except BaseException as e:       # noqa: B902 - handed to the caller below
+                with lock:
+                    errs.append(e)
+                self._bar.abort()
+
+        threads = [threading.Thread(target=body, args=(r,), name=f"ps-rank{r}") for r in range(self.world)]
+        for t in threads:
+            t.start()
+        for t in threads:
+            t.join()
+        if errs:
+            first = next((e for e in errs if not isinstance(e, threading.BrokenBarrierError)), errs[0])
+            raise first
+        return out
+
+    def _sync(self, t):
+        import torch
+        if t.is_cuda:
+            torch.cuda.current_stream(t.device).synchronize()
+
+    def _collective(self, t, combine):
+        """Meet the other ranks with t, return combine(every rank's t) once every rank has read what it needs."""
+        self._sync(t)
+        self._slots[self._local.rank] = t
+        self._bar.wait()
+        res = combine(list(self._slots))
+        self._sync(res)
+        self._bar.wait()
+        return res
+
+    def all_reduce(self, t):
+        def total(ts):
+            acc = ts[0].to(t.device, copy=True)
+            for x in ts[1:]:
+                acc += x.to(t.device)
+            return acc
+        t.copy_(self._collective(t, total))
+
+    def all_gather_into_tensor(self, out, t):
+        n = t.numel()
+        assert out.numel() == self.world * n, "every rank gathers equal parts"
+
+        def gather(ts):
+            for r, x in enumerate(ts):
+                assert x.numel() == n, "every rank gathers equal parts"
+                out[r * n:(r + 1) * n].copy_(x.reshape(-1))
+            return out
+        self._collective(t, gather)
+
+    def broadcast(self, t, src):
+        t.copy_(self._collective(t, lambda ts: ts[src].to(t.device, copy=True)))
+
+    def connect_pools(self, ctx, rank, world, device, pool, meta):
+        """Every rank's receive pool into ctx's route: the contexts meet here after their ps_route_setup, and
+        ps_route_connect reads the pools from them (and enables peer access). Nobody changes a route before every
+        rank has read all of them."""
+        self._slots[rank] = ctx
+        self._bar.wait()
+        ctx.route_connect(list(self._slots))
+        self._bar.wait()
+
+
+def _cap_owner(group):
+    """The object that carries the survivor all-gather's capacity: the group, or the process-wide TorchGroup when
+    the caller hands torch.distributed itself."""
+    return group if hasattr(group, "gather_cap") else TORCH_GROUP
 
 
 def gather_results(parts, rank, world, device, dist, top_k=None, p_exact=None):
@@ -124,8 +264,9 @@ def gather_results(parts, rank, world, device, dist, top_k=None, p_exact=None):
         bufs.append(buf)
     buf = np.concatenate(bufs) if bufs else np.empty(0, np.uint8)
     hdr = np.array(hdr_rows, dtype=np.int64).reshape(-1).view(np.uint8)
+    owner = _cap_owner(dist)
     while True:
-        cap = _GATHER_CAP["bytes"]
+        cap = owner.gather_cap
         mine = np.zeros(len(hdr) + cap, dtype=np.uint8)
         mine[:len(hdr)] = hdr
         if len(buf) <= cap:
@@ -138,7 +279,7 @@ def gather_results(parts, rank, world, device, dist, top_k=None, p_exact=None):
         need = int(metas[:, :, 1].sum(axis=1).max())
         if need <= cap:
             break
-        _GATHER_CAP["bytes"] = 2 * need
+        owner.gather_cap = 2 * need
     if rank != 0:
         return None
     names = [r.name for r in res0]
@@ -168,11 +309,10 @@ class _DevView:
                                          "version": 2, "strides": None}
 
 
-def exchange_streams(ka: KmerAssociation, n_samples, rank, world, device):
+def exchange_streams(ka: KmerAssociation, n_samples, rank, world, device, dist=TORCH_GROUP):
     """All-gather every rank's packed stream block; import the blocks this rank does not own.
     Returns the bytes received over NVLink by this rank."""
     import torch
-    import torch.distributed as dist
 
     ctx = ka.ctx
     mine = list(sample_block(rank, world, n_samples))
@@ -233,7 +373,8 @@ class PageRoute:
         hi = 0 if j == self.passes - 1 else S[(j + 1) * W - 1]
         return lo, hi, S[j * W:j * W + W - 1]
 
-    def prepare(self, k, n_samples, dist, torch):
+    def prepare(self, k, n_samples, dist, torch, passes=None):
+        """passes: number of super-ranges; None = as many as the pool budget needs."""
         ctx = self.ka.ctx
         if self.bar is None:
             self.bar = torch.zeros(1, dtype=torch.int32, device=self.device)
@@ -241,11 +382,11 @@ class PageRoute:
         allc = torch.empty(self.world, dtype=torch.int64, device=self.device)
         dist.all_gather_into_tensor(allc, mine)
         counts = tuple(int(x) for x in allc.cpu().tolist())
-        key = (k, n_samples, counts)
+        key = (k, n_samples, counts, passes)
         if key != self.key:
             # a new job: passes so that a pool fits the budget, then quantile splitters of sample 0 (held by rank 0)
             total = sum(counts)
-            self.passes = max(1, int(np.ceil(total * 1.5 * 4 / (self.world * POOL_BUDGET_BYTES))))
+            self.passes = int(passes) if passes else max(1, int(np.ceil(total * 1.5 * 4 / (self.world * POOL_BUDGET_BYTES))))
             nq = self.world * self.passes
             spl_t = torch.zeros(max(nq - 1, 1), dtype=torch.int64, device=self.device)
             if self.rank == 0:
@@ -260,55 +401,77 @@ class PageRoute:
             self.pages = max(self.pages, int(allneed.max().item()))
             self.key = key
         if self.pages != self.live_pages:
-            # pools (re)allocated on every rank: unmap the old ones first, then exchange the new handles
+            # pools (re)allocated on every rank: unmap the old ones first (CUDA IPC; threads map nothing), then
+            # exchange the new ones
             ctx.ipc_close_all()
             self.barrier(dist)
             torch.cuda.synchronize(self.device)
             pool, meta = ctx.route_setup(self.world, self.rank, self.pass_range(0)[2], self.pages)
-            h = np.frombuffer(ctx.ipc_export(pool) + ctx.ipc_export(meta), dtype=np.uint8).copy()
-            allh = torch.empty(self.world * 128, dtype=torch.uint8, device=self.device)
-            dist.all_gather_into_tensor(allh, torch.from_numpy(h).to(self.device))
-            allh = allh.cpu().numpy().reshape(self.world, 128)
-            pools = [pool if d == self.rank else ctx.ipc_open(allh[d, :64].tobytes()) for d in range(self.world)]
-            metas = [meta if d == self.rank else ctx.ipc_open(allh[d, 64:].tobytes()) for d in range(self.world)]
-            ctx.route_peers(pools, metas)
+            dist.connect_pools(ctx, self.rank, self.world, self.device, pool, meta)
             self.live_pages = self.pages
 
 
-def run_sharded(ka: KmerAssociation, buffers_by_sample, n_samples, k, pheno, binary, weights,
-                rank, world, device, cutoff=1, route="auto", **test_kw):
-    """Whole hot path on `world` GPUs. buffers_by_sample: {sample_idx: bytes or (dev_ptr, n)} for the
-    samples this rank owns (sample_block(rank, world, n_samples)).
-    Returns (U_total, results on rank 0 / None elsewhere, info)."""
-    import os
-    import time
-    timing = os.environ.get("PS_DIST_TIMING") and rank == 0
-    marks = []
+class _Marks:
+    """PS_DIST_TIMING=1: device-synchronised wall-clock marks of rank 0, written to stderr."""
 
-    def mark(name):
-        if timing:
+    def __init__(self, rank, device):
+        import os
+        self.on = bool(os.environ.get("PS_DIST_TIMING")) and rank == 0
+        self.device, self.marks = device, []
+
+    def __call__(self, name):
+        if self.on:
+            import time
             import torch
-            torch.cuda.synchronize(device)
-            marks.append((name, time.time()))
+            torch.cuda.synchronize(self.device)
+            self.marks.append((name, time.time()))
 
-    ctx = ka.ctx
+    def report(self):
+        if self.on:
+            import sys
+            sys.stderr.write("[dist timing ms] " + " ".join(
+                f"{b[0]}={1e3 * (b[1] - a[1]):.1f}" for a, b in zip(self.marks, self.marks[1:])) + "\n")
+
+
+def begin_block(ka: KmerAssociation, n_samples, k, rank, world, cutoff=1):
+    """Start the job on this rank's context (all n_samples, global indices) -> the samples this rank ingests."""
     ka.k, ka.n_samples = int(k), int(n_samples)
-    mark("start")
-    ctx.begin(int(k), int(n_samples), int(cutoff))
-    mine = list(sample_block(rank, world, n_samples))
-    assert sorted(buffers_by_sample) == mine, "this rank must hold exactly its own block of samples"
+    ka.ctx.begin(int(k), int(n_samples), int(cutoff))
+    ka._streams_imported = False
     if world == 1:
-        ctx.route_clear()
+        ka.ctx.route_clear()
+    return list(sample_block(rank, world, n_samples))
+
+
+def ingest(ka: KmerAssociation, buffers_by_sample, n_samples, k, rank, world, cutoff=1):
+    """Ingest step of run_sharded: begin + add_samples of this rank's block. buffers_by_sample: {sample_idx: bytes
+    or (dev_ptr, n)} for exactly sample_block(rank, world, n_samples)."""
+    mine = begin_block(ka, n_samples, k, rank, world, cutoff)
+    assert sorted(buffers_by_sample) == mine, "this rank must hold exactly its own block of samples"
     if mine:
-        ctx.add_samples(mine[0], [buffers_by_sample[s] for s in mine])
+        ka.ctx.add_samples(mine[0], [buffers_by_sample[s] for s in mine])
+
+
+def build_and_test(ka: KmerAssociation, n_samples, k, pheno, binary, weights, rank, world, device, route="auto",
+                   group=None, restrict=None, passes=None, marks=None, **test_kw):
+    """Build-and-test step of run_sharded, after ingest() on every rank: the exchange, each rank's union and matrix
+    of its k-mer ranges, the tests, the exact filter and the gather of the survivors on rank 0.
+    group: TorchGroup (default, torch.distributed) or ThreadGroup. restrict: ascending distinct database k-mers
+    (--kmerDB): each range keeps only those (ps_restrict_union) and U counts what is left. passes: number of
+    super-ranges of the "pages" route (None: as many as the pool budget needs). A page-pool overflow raises
+    PoolOverflow after every rank has doubled its pools: running this step again (without a new ingest) retries.
+    Returns (U_total, results on rank 0 / None elsewhere, info)."""
+    ctx = ka.ctx
+    dist = TORCH_GROUP if group is None else group
+    mark = marks or _Marks(rank, device)
     if world == 1:
         U = ka.build()
+        if restrict is not None:
+            U = ka.restrict_to(restrict)
         res = ka.test(pheno, binary, weights, **test_kw)
         return U, res, {"U_local": U, "nvlink_bytes": 0, "splitters": []}
     import torch
-    import torch.distributed as dist
 
-    mark("ingest")
     if route == "auto":
         route = "pages" if 9 <= int(k) <= 16 else "streams"
     if route == "pages" and not 9 <= int(k) <= 16:
@@ -320,7 +483,7 @@ def run_sharded(ka: KmerAssociation, buffers_by_sample, n_samples, k, pheno, bin
             pr = getattr(ka, "_page_route", None)
             if pr is None or (pr.rank, pr.world) != (rank, world):
                 pr = ka._page_route = PageRoute(ka, rank, world, device)
-            pr.prepare(int(k), int(n_samples), dist, torch)
+            pr.prepare(int(k), int(n_samples), dist, torch, passes)
             spl = pr.splitters
             mark("prepare")
             U_seen = 0
@@ -335,6 +498,8 @@ def run_sharded(ka: KmerAssociation, buffers_by_sample, n_samples, k, pheno, bin
                 ctx.route_scatter()
                 pr.barrier(dist)            # every sender's stores have landed
                 U_local, ovf = ctx.route_build()
+                if restrict is not None and not ovf:
+                    U_local = ctx.restrict_union(restrict)
                 ka.U = U_local
                 u = torch.tensor([U_local, 1 if ovf else 0], dtype=torch.int64, device=device)
                 dist.all_reduce(u)
@@ -343,7 +508,7 @@ def run_sharded(ka: KmerAssociation, buffers_by_sample, n_samples, k, pheno, bin
                     pr.pages *= 2          # same decision on every rank: larger pools from the next step on
                     if pr.passes > 1:
                         ctx.set_range(0, 0)
-                    raise RuntimeError("a page pool overflowed while routing k-mers (skewed k-mer ranges); "
+                    raise PoolOverflow("a page pool overflowed while routing k-mers (skewed k-mer ranges); "
                                        "the next step will use pools twice as large")
                 # Bonferroni needs the total U: a pass tests against the union seen so far (a laxer threshold),
                 # the exact filter follows when every pass is done
@@ -355,10 +520,15 @@ def run_sharded(ka: KmerAssociation, buffers_by_sample, n_samples, k, pheno, bin
             nvl_bytes = None
         else:
             ctx.route_clear()
-            nvl_bytes = exchange_streams(ka, n_samples, rank, world, device)
+            nvl_bytes = 0
+            if not getattr(ka, "_streams_imported", False):      # imported streams stay until the next ingest
+                nvl_bytes = exchange_streams(ka, n_samples, rank, world, device, dist)
+                ka._streams_imported = True
             mark("exchange")
             spl = ctx.sample_quantiles(0, world)          # identical on every rank: all hold sample 0
             U_local = ka.build(range_of(rank, spl))
+            if restrict is not None:
+                U_local = ka.restrict_to(restrict)
             mark("build")
             u = torch.tensor([U_local], dtype=torch.int64, device=device)
             dist.all_reduce(u)
@@ -369,9 +539,20 @@ def run_sharded(ka: KmerAssociation, buffers_by_sample, n_samples, k, pheno, bin
                                 p_exact=(float(test_kw.get("pvalue_cutoff", 0.05)) / U_total if U_total else 0.0)
                                 if not (binary and test_kw.get("omit_b")) else None)
         mark("gather")
-    if timing:
-        import sys
-        sys.stderr.write("[dist timing ms] " + " ".join(
-            f"{b[0]}={1e3 * (b[1] - a[1]):.1f}" for a, b in zip(marks, marks[1:])) + "\n")
+    mark.report()
     return U_total, merged, {"U_local": sum(p[0] for p in parts), "nvlink_bytes": nvl_bytes, "splitters": spl, "route": route,
                              "passes": len(parts)}
+
+
+def run_sharded(ka: KmerAssociation, buffers_by_sample, n_samples, k, pheno, binary, weights,
+                rank, world, device, cutoff=1, route="auto", group=None, **test_kw):
+    """Whole hot path on `world` GPUs: ingest() then build_and_test(). buffers_by_sample: {sample_idx: bytes or
+    (dev_ptr, n)} for the samples this rank owns (sample_block(rank, world, n_samples)). group: see build_and_test.
+    Returns (U_total, results on rank 0 / None elsewhere, info)."""
+    marks = _Marks(rank, device)
+    marks("start")
+    ingest(ka, buffers_by_sample, n_samples, k, rank, world, cutoff)
+    if world > 1:
+        marks("ingest")
+    return build_and_test(ka, n_samples, k, pheno, binary, weights, rank, world, device, route=route, group=group,
+                          marks=marks, **test_kw)

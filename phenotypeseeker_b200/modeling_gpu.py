@@ -31,14 +31,37 @@ import pandas as pd
 
 from .pipeline import KmerAssociation, kmers_to_str, read_sample_file
 
-_STATE = {"ka": None, "pid": None, "names": None, "ranges": 1, "results": None}
+_STATE = {"ka": None, "pid": None, "devices": None, "names": None, "ranges": 1, "results": None, "db": None}
+
+
+def parse_devices(spec):
+    """PS_DEVICE / device= -> one device index (int: the single-GPU KmerAssociation) or a list of them (several
+    entries: a GpuGroup, one rank per entry, repeats allowed). Accepts an int, "0", "0,1,2,3", "0, 0" or a sequence."""
+    if isinstance(spec, str):
+        parts = [p.strip() for p in spec.split(",") if p.strip()]
+    elif isinstance(spec, (list, tuple, range)):
+        parts = list(spec)
+    else:
+        return int(spec)
+    if not parts:
+        raise ValueError(f"no device in {spec!r}")
+    devs = [int(p) for p in parts]
+    return devs[0] if len(devs) == 1 else devs
 
 
 def _ka(device=None):
-    if _STATE["ka"] is None or _STATE["pid"] != os.getpid():
-        dev = int(os.environ.get("PS_DEVICE", "0")) if device is None else device
-        _STATE["ka"] = KmerAssociation(device=dev)
-        _STATE["pid"] = os.getpid()
+    """The engine of this process: a KmerAssociation for one device, a GpuGroup for several. Made again when the
+    process changes (fork) or an explicit `device` asks for other devices."""
+    spec = None if device is None else parse_devices(device)
+    if _STATE["ka"] is None or _STATE["pid"] != os.getpid() or (spec is not None and spec != _STATE["devices"]):
+        devs = parse_devices(os.environ.get("PS_DEVICE", "0")) if spec is None else spec
+        _STATE["ka"] = None                   # free the old engine's device memory before the new one allocates
+        if isinstance(devs, int):
+            _STATE["ka"] = KmerAssociation(device=devs)
+        else:
+            from .group import GpuGroup
+            _STATE["ka"] = GpuGroup(devs)
+        _STATE["pid"], _STATE["devices"] = os.getpid(), devs
     return _STATE["ka"]
 
 
@@ -131,18 +154,23 @@ def pheno_matrix(samples, pheno_names):
 
 def run_hot_path(files, sample_names, k, cutoff, pheno, pheno_names, binary, weights, min_samples, max_samples,
                  pvalue_cutoff, omit_b, n_stripes, real_counts=False, device=None):
-    """Stages 1-3 on the GPU -> (U, {pheno_name: ML_df}). Plain-data entry used by tests/standalone."""
+    """Stages 1-3 on the GPU -> (U, {pheno_name: ML_df}). Plain-data entry used by tests/standalone.
+    device: as PS_DEVICE (parse_devices); several entries run on a GpuGroup."""
     ka = _ka(device)
     ka.count(files, k, cutoff)
-    U = ka.build()
-    res = ka.test(pheno, binary, weights, min_samples=min_samples, max_samples=max_samples,
-                  pvalue_cutoff=pvalue_cutoff, omit_b=omit_b, pheno_names=list(pheno_names))
+    kw = dict(min_samples=min_samples, max_samples=max_samples, pvalue_cutoff=pvalue_cutoff, omit_b=omit_b,
+              pheno_names=list(pheno_names))
+    if ka.fits_in_one_build():
+        U = ka.build()
+        res = ka.test(pheno, binary, weights, **kw)
+    else:
+        U, res = ka.test_in_ranges(pheno, binary, ka.ranges_needed(), weights, n_instances=ka.instances_upper(), **kw)
     out = {}
     for j, r in enumerate(res):
         r.na_mask = np.isnan(np.asarray(pheno, dtype=np.float64).reshape(len(sample_names), -1)[:, j])
         counts = None
         if real_counts and len(r.kmer):
-            counts = np.stack([ka.ctx.lookup(s, r.kmer) for s in range(len(sample_names))], axis=1)
+            counts = np.stack([ka.lookup(s, r.kmer) for s in range(len(sample_names))], axis=1)
             counts = counts * (r.presence != 0)       # a count below the cutoff is 0 in the reference's list (glistmaker -c)
         out[r.name] = build_ml_df(r, k, sample_names, n_stripes, binary, counts)
     return U, out
@@ -151,6 +179,10 @@ def run_hot_path(files, sample_names, k, cutoff, pheno, pheno_names, binary, wei
 # ---------------------------------------------------------------------------------------
 def install(m, device=None, native_weights=None):
     """Re-wire the reference module `m` (PhenotypeSeeker.modeling) onto the GPU path.
+
+    device (default: env PS_DEVICE, else 0): one device index, or several ("0,1,2,3" or a sequence) to run on a
+    GpuGroup in this one process. A group builds and tests every column at once in kmer_testing_setup, as a
+    single GPU does for inputs that need k-mer ranges; -rc, native_weights="gpu" and --kmerDB work on both.
 
     native_weights (default: env PS_NATIVE_WEIGHTS): also replace the `-w` weight computation
     (`Samples.get_mash_sketches` / `get_weights`, modeling.py:386-503: mash binary + Biopython + ete3) with
@@ -179,14 +211,12 @@ def install(m, device=None, native_weights=None):
             db = ka.kmers_of(read_sample_file(Samples.kmerDB), int(Samples.kmer_length))
         ka.count_files([s.address for s in samples], int(Samples.kmer_length), int(Samples.cutoff))   # streamed in batches
         _STATE["results"] = None
+        _STATE["db"] = db
         _STATE["ranges"] = 1 if ka.fits_in_one_build() else ka.ranges_needed()
         if _STATE["ranges"] == 1:
             ka.build()
             if db is not None:
                 ka.restrict_to(db)                           # glistcompare -i
-        elif db is not None:
-            raise RuntimeError("--kmerDB needs union and matrix in GPU memory at once; this input needs "
-                               f"{_STATE['ranges']} k-mer ranges")
         os.makedirs("K-mer_lists", exist_ok=True)   # get_mash_sketches (-w) writes its sketches there
         _STATE["names"] = [s.name for s in samples]
 
@@ -205,7 +235,8 @@ def install(m, device=None, native_weights=None):
         kw = dict(min_samples=Samples.min_samples, max_samples=Samples.max_samples, pvalue_cutoff=phenotypes.pvalue_cutoff,
                   omit_b=bool(phenotypes.omit_B), pheno_names=cols)
         if _STATE["ranges"] > 1:
-            _, res = ka.test_in_ranges(ph, binary, _STATE["ranges"], w, n_instances=ka.ctx.instances_upper(), **kw)
+            _, res = ka.test_in_ranges(ph, binary, _STATE["ranges"], w, n_instances=ka.instances_upper(),
+                                       restrict=_STATE["db"], **kw)
         else:
             res = ka.test(ph, binary, w, **kw)
         for j, r in enumerate(res):
@@ -229,7 +260,7 @@ def install(m, device=None, native_weights=None):
         res = test_all_columns()[self.name]
         counts = None
         if phenotypes.real_counts and len(res.kmer):
-            counts = np.stack([ka.ctx.lookup(s, res.kmer) for s in range(len(names))], axis=1)
+            counts = np.stack([ka.lookup(s, res.kmer) for s in range(len(names))], axis=1)
             counts = counts * (res.presence != 0)         # a count below the cutoff is 0 in the reference's list (glistmaker -c)
         self.ML_df = build_ml_df(res, ka.k, names, Input.num_threads, binary, counts)
         if self.ML_df.shape[0] == 0:
@@ -252,7 +283,7 @@ def install(m, device=None, native_weights=None):
             if _STATE["names"] != names or _STATE["ka"] is None or _STATE["pid"] != os.getpid():
                 raise RuntimeError("native_weights='gpu' computes the weights from the samples get_feature_vector "
                                    "decoded; call it first, with the same Input.samples")
-            w = psw.gsc_weights_on_device(_STATE["ka"].ctx, names, 0, keep_glob_quirk=True)
+            w = psw.gsc_weights_on_device(_STATE["ka"], names, 0, keep_glob_quirk=True)
         else:
             w = psw.gsc_weights_for_samples(names, [read_sample_file(s.address) for s in samples],
                                             keep_glob_quirk=True)

@@ -138,6 +138,10 @@ class KmerAssociation:
         self.k = int(k)
         self.n_samples = len(paths)
         self.ctx.begin(self.k, self.n_samples, int(cutoff))
+        self.add_files(0, paths, batch_bytes)
+
+    def add_files(self, first_idx, paths, batch_bytes=2 << 30):
+        """Samples first_idx, first_idx + 1, ... of the job begun from files, read in batches as count_files does."""
         i = 0
         while i < len(paths):
             batch, tot, j = [], 0, i
@@ -148,7 +152,7 @@ class KmerAssociation:
                 batch.append(read_sample_file(paths[j]))
                 tot += len(batch[-1])
                 j += 1
-            self.ctx.add_samples(i, batch)
+            self.ctx.add_samples(first_idx + i, batch)
             del batch
             i = j
 
@@ -171,6 +175,9 @@ class KmerAssociation:
         have = (free + self.ctx.device_bytes()) * headroom - (1 << 30)
         need = n * 8 * 1.3 + (n / 4) * (8 + row_bytes)
         return max(1, int(np.ceil(need / max(have, 1))))
+
+    def instances_upper(self):
+        return self.ctx.instances_upper()
 
     # stage 2 (modeling.py:1656-1663, 641-644)
     def build(self, kmer_range=None):
@@ -217,6 +224,20 @@ class KmerAssociation:
         self.ctx.load_matrix(rows, u[idx])
         self.U = len(idx)
         return self.U
+
+    # per-sample device work of the drop-in (-rc counts, -w weights); GpuGroup has the same methods
+    def lookup(self, sample, kmers):
+        """Counts of `kmers` in one sample (ps_lookup)."""
+        return self.ctx.lookup(sample, kmers)
+
+    def mash_sketch(self, first_idx, count, k=21, s=1000, seed=42):
+        return self.ctx.mash_sketch(first_idx, count, k, s, seed)
+
+    def mash_pairs(self, hashes, n_hashes):
+        return self.ctx.mash_pairs(hashes, n_hashes)
+
+    def neighbor_joining(self, dm):
+        return self.ctx.neighbor_joining(dm)
 
     # stage 3 (modeling.py:1679-1683)
     def test(self, pheno, binary, weights=None, min_samples=2, max_samples=None, pvalue_cutoff=0.05,
@@ -300,7 +321,7 @@ class KmerAssociation:
         return {"splitters": spl, "grouped": grouped, "slack": slack, "first_of": first_of, "ingest": ingest}
 
     def test_in_ranges(self, pheno, binary, n_ranges, weights=None, pvalue_cutoff=0.05, omit_b=False,
-                       splitters=None, n_instances=None, top_k=None, n_super=None, **kw):
+                       splitters=None, n_instances=None, top_k=None, n_super=None, restrict=None, **kw):
         """Stages 2-3 when records or matrix do not fit in HBM at once (SURVEY.md §7 "memory at
         config 5"): the k-mer space is cut into n_ranges contiguous ranges (quantiles of sample 0,
         or `splitters` from an earlier call on the same job), each range is built and tested on its
@@ -317,7 +338,11 @@ class KmerAssociation:
         far), i.e. a laxer threshold, and the exact pvalue/U filter is applied afterwards.
         n_instances: k-mer instances of the whole job (positions); sizes the page pools of a range
         (ps_set_capacity_hint) instead of reserving for every position of the input.
+        restrict (--kmerDB database k-mers): only with n_ranges == 1, which restricts the one build.
         Call after count(). Returns (U, [PhenoResult per phenotype column])."""
+        if restrict is not None and n_ranges > 1:
+            raise RuntimeError("--kmerDB needs union and matrix in GPU memory at once; this input needs "
+                               f"{n_ranges} k-mer ranges")
         ph = np.asarray(pheno, dtype=np.float64)
         if ph.ndim == 1:
             ph = ph[:, None]
@@ -341,6 +366,8 @@ class KmerAssociation:
                 if n_instances:
                     self.ctx.set_capacity_hint(int(n_instances * slack / n_ranges) + (1 << 20))
             u_r = self.build()
+            if restrict is not None:
+                u_r = self.restrict_to(restrict)
             res = self.test(ph, binary, weights, pvalue_cutoff=pvalue_cutoff, omit_b=omit_b, top_k=top_k,
                             n_union_total=(U + u_r) if not (binary and omit_b) else None, **kw) if u_r else None
             parts.append((U, res))
