@@ -185,11 +185,24 @@ int ps_fetch_survivors(ps_ctx *ctx, size_t cap, int32_t *pheno_idx, uint64_t *ro
                        double *mean_y, uint32_t *n_with, uint32_t *rowbits);
 
 /*
- * Occurrence counts of K given canonical k-mers in sample idx (0 if absent).
- * Replaces: `gmer_counter -db <kmers> <sample>` of prediction.py:72-100, and the
- * raw-count columns of --real_counts (modeling.py:693-695) for surviving k-mers.
+ * Occurrence counts of K given canonical k-mers in sample idx (0 if absent): the
+ * count == 1 case of ps_count_matrix, same rules.
  */
 int ps_lookup(ps_ctx *ctx, int idx, const uint64_t *kmers, size_t K, uint32_t *counts);
+
+/*
+ * counts[i*K + j] = occurrences of kmers[j] in sample first_idx + i, for i < count:
+ * one device pass over the decoded streams of all those samples.
+ * kmers: K <= 2^30 canonical codes (host or device memory), duplicates allowed (every
+ * copy gets the count). A count covers every valid window of the sample's decoded
+ * stream: it is not cut by the job's cutoff or k-mer range. counts: host memory.
+ * The job's union, matrix, survivors and k-mer range are left untouched.
+ * PS_ERR_ARG for a sample that is not present, null pointers, or count x K overflow.
+ * Replaces: `gmer_counter -db <kmers> <sample>` of prediction.py:72-100 for every
+ * sample, and the raw-count columns of --real_counts (modeling.py:693-695).
+ */
+int ps_count_matrix(ps_ctx *ctx, int first_idx, int count, const uint64_t *kmers, size_t K,
+                    uint32_t *counts);
 
 /*
  * Packed streams for the multi-GPU exchange (device pointers, valid until ps_begin):

@@ -40,6 +40,8 @@ SIGNATURES = {
     "ps_fetch_survivors": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_size_t] + [ctypes.c_void_p] * 9),
     "ps_lookup": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_size_t,
                                  ctypes.c_void_p]),
+    "ps_count_matrix": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_void_p, ctypes.c_size_t,
+                                       ctypes.c_void_p]),
     "ps_export_stream": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, c_void_pp, c_void_pp, c_u64_p]),
     "ps_import_stream": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
                                         ctypes.c_uint64]),
@@ -272,6 +274,13 @@ class Context:
         q = np.ascontiguousarray(kmers, dtype=np.uint64)
         out = np.zeros(len(q), dtype=np.uint32)
         self._ck(self.L.ps_lookup(self.h, int(idx), _ptr(q), len(q), _ptr(out)))
+        return out
+
+    def count_matrix(self, first_idx, count, kmers):
+        """(count, K) uint32: occurrences of every k-mer in samples first_idx .. first_idx + count - 1."""
+        q = np.ascontiguousarray(kmers, dtype=np.uint64)
+        out = np.zeros((int(count), len(q)), dtype=np.uint32)
+        self._ck(self.L.ps_count_matrix(self.h, int(first_idx), int(count), _ptr(q), len(q), _ptr(out)))
         return out
 
     # -- exchange ----------------------------------------------------------------------

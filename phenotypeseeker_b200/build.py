@@ -8,7 +8,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libpskmer.so")
 SOURCES = ["ps_api.cu"]
 HEADERS = ["ps_common.cuh", "ps_decode.cuh", "ps_decode_bits.h", "ps_extract.cuh", "ps_sort.cuh", "ps_paged.cuh", "ps_rows.cuh",
-           "ps_test.cuh", "ps_chi2_reach.h", "ps_mash.cuh", "ps_mash_bits.h", os.path.join("..", "..", "include", "pskmer.h")]
+           "ps_test.cuh", "ps_chi2_reach.h", "ps_mash.cuh", "ps_mash_bits.h", "ps_count.cuh", os.path.join("..", "..", "include", "pskmer.h")]
 
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "-shared", "--use_fast_math=false"]

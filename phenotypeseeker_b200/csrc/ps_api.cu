@@ -13,6 +13,7 @@
 #include "ps_test.cuh"
 #include "ps_chi2_reach.h"
 #include "ps_mash.cuh"
+#include "ps_count.cuh"
 
 static std::string g_create_err;
 
@@ -1080,6 +1081,8 @@ int ps_ctx_create(int device, ps_ctx **out) {
     cudaFuncSetAttribute(k_bucket_count_pg<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     cudaFuncSetAttribute(k_mash_sketch, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mash_smem(PSM_S_MAX));
     cudaFuncSetAttribute(k_mash_merge, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mash_smem(PSM_S_MAX));
+    cudaFuncSetAttribute(k_count_matrix<uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(CNT_FILTER_WORDS * 4));
+    cudaFuncSetAttribute(k_count_matrix<uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(CNT_FILTER_WORDS * 4));
     cudaFuncSetAttribute(k_bucket_count_pg<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     if (const char *ev = getenv("PSKMER_BK_TMA")) c->bk_tma = atoi(ev) != 0;
     if (const char *ev = getenv("PSKMER_PAGED")) c->paged = atoi(ev) != 0;
@@ -1677,39 +1680,112 @@ int ps_fetch_survivors(ps_ctx *c, size_t cap, int32_t *pheno_idx, uint64_t *row,
     API_END(c)
 }
 
-int ps_lookup(ps_ctx *c, int idx, const uint64_t *kmers, size_t K, uint32_t *counts) {
+// Device scratch of ps_count_matrix: the counts of one chunk of samples stay under this (one row at the least)
+#define CNT_CHUNK_BYTES (256ull << 20)
+
+int ps_count_matrix(ps_ctx *c, int first_idx, int count, const uint64_t *kmers, size_t K, uint32_t *counts) {
     API_BEGIN(c)
-    if (idx < 0 || idx >= c->n_samples || !c->samples[idx].present) PS_THROW(PS_ERR_ARG, "no such sample %d", idx);
+    if (count < 1 || first_idx < 0 || (int64_t)first_idx + count > c->n_samples)
+        PS_THROW(PS_ERR_ARG, "samples %d..%lld outside the job's 0..%d", first_idx, (long long)first_idx + count - 1,
+                 c->n_samples - 1);
+    for (int i = first_idx; i < first_idx + count; i++)
+        if (!c->samples[i].present) PS_THROW(PS_ERR_ARG, "no such sample %d", i);
     if (K == 0) return PS_OK;
     if (!kmers || !counts) PS_THROW(PS_ERR_ARG, "null argument");
     if (K > (1u << 30)) PS_THROW(PS_ERR_ARG, "too many query k-mers");
-    // sort + dedupe the queries on the host; map results back afterwards
-    std::vector<uint64_t> uq(kmers, kmers + K);
-    std::sort(uq.begin(), uq.end());
-    uq.erase(std::unique(uq.begin(), uq.end()), uq.end());
-    const size_t Ku = uq.size();
-    c->tmp1.reserve(Ku * 8, c->stream);
-    c->tmp2.reserve(Ku * 4, c->stream);
-    CK(cudaMemcpyAsync(c->tmp1.p, uq.data(), Ku * 8, cudaMemcpyHostToDevice, c->stream));
-    CK(cudaMemsetAsync(c->tmp2.p, 0, Ku * 4, c->stream));
-    const SampleInfo &s = c->samples[idx];
-    const unsigned nb = (unsigned)(s.n_pos / EXT_BLOCK_POS);
-    if (nb) {
-        if (key64(c))
-            KLAUNCH(c, "lookup", (double)s.n_pos * 3 / 8,
-                    (k_lookup<uint64_t><<<nb, EXT_THREADS, 0, c->stream>>>(c->pool_seq.as<uint32_t>(), c->pool_bad.as<uint32_t>(), s.pos_off, c->k, c->tmp1.as<uint64_t>(), (int)Ku, c->tmp2.as<uint32_t>())));
-        else
-            KLAUNCH(c, "lookup", (double)s.n_pos * 3 / 8,
-                    (k_lookup<uint32_t><<<nb, EXT_THREADS, 0, c->stream>>>(c->pool_seq.as<uint32_t>(), c->pool_bad.as<uint32_t>(), s.pos_off, c->k, c->tmp1.as<uint64_t>(), (int)Ku, c->tmp2.as<uint32_t>())));
+    if ((size_t)count > SIZE_MAX / sizeof(uint32_t) / K) PS_THROW(PS_ERR_ARG, "count x K overflows");
+    // sorted unique queries; inv maps the caller's order onto them unless the queries already ascend strictly
+    std::vector<uint64_t> q;
+    cudaPointerAttributes pa;
+    if (cudaPointerGetAttributes(&pa, kmers) == cudaSuccess && pa.type == cudaMemoryTypeDevice) {
+        q.resize(K);
+        CK(cudaMemcpy(q.data(), kmers, K * 8, cudaMemcpyDeviceToHost));
+    } else q.assign(kmers, kmers + K);
+    cudaGetLastError();
+    bool identity = true;
+    for (size_t j = 1; j < K && identity; j++) identity = q[j - 1] < q[j];
+    std::vector<uint32_t> inv;
+    if (!identity) {
+        std::vector<uint64_t> u(q);
+        std::sort(u.begin(), u.end());
+        u.erase(std::unique(u.begin(), u.end()), u.end());
+        inv.resize(K);
+        for (size_t j = 0; j < K; j++) inv[j] = (uint32_t)(std::lower_bound(u.begin(), u.end(), q[j]) - u.begin());
+        q.swap(u);
     }
-    std::vector<uint32_t> hc(Ku);
-    CK(cudaMemcpyAsync(hc.data(), c->tmp2.p, Ku * 4, cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaStreamSynchronize(c->stream));
-    for (size_t i = 0; i < K; i++) {
-        const size_t j = std::lower_bound(uq.begin(), uq.end(), kmers[i]) - uq.begin();
-        counts[i] = hc[j];
+    const uint64_t Ku = q.size();
+    // radix index: qidx[t] = first query whose top bits are >= t
+    const int ibits = std::min(2 * c->k, CNT_INDEX_BITS), ishift = 2 * c->k - ibits;
+    std::vector<uint32_t> qidx(((size_t)1 << ibits) + 1, 0);
+    for (uint64_t j = 0; j < Ku; j++) qidx[(q[j] >> ishift) + 1]++;
+    for (size_t t = 1; t < qidx.size(); t++) qidx[t] += qidx[t - 1];
+    c->cm_q.reserve(Ku * 8, c->stream);
+    c->cm_idx.reserve(qidx.size() * 4, c->stream);
+    c->cm_filter.reserve(CNT_FILTER_WORDS * 4, c->stream);
+    CK(cudaMemcpyAsync(c->cm_q.p, q.data(), Ku * 8, cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemcpyAsync(c->cm_idx.p, qidx.data(), qidx.size() * 4, cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemsetAsync(c->cm_filter.p, 0, CNT_FILTER_WORDS * 4, c->stream));
+    KLAUNCH(c, "count_filter", (double)Ku * 8,
+            (k_count_filter<<<(unsigned)std::min<uint64_t>(PS_SMS * 4, ceil_div<uint64_t>(Ku, 256)), 256, 0, c->stream>>>(
+                c->cm_q.as<uint64_t>(), Ku, c->cm_filter.as<uint32_t>())));
+    if (!identity) {
+        c->cm_inv.reserve(K * 4, c->stream);
+        CK(cudaMemcpyAsync(c->cm_inv.p, inv.data(), K * 4, cudaMemcpyHostToDevice, c->stream));
+    }
+    // samples in chunks whose device counts (and their expansion to the caller's order) stay under the cap
+    const uint64_t row_bytes = Ku * 4 + (identity ? 0 : (uint64_t)K * 4);
+    const int chunk = (int)std::min<uint64_t>(count, std::max<uint64_t>(1, CNT_CHUNK_BYTES / row_bytes));
+    c->cm_cnt.reserve((size_t)chunk * Ku * 4, c->stream);
+    if (!identity) c->cm_out.reserve((size_t)chunk * K * 4, c->stream);
+    c->cm_tab.reserve((size_t)chunk * 12 + 16, c->stream);
+    std::vector<uint64_t> tab(chunk + (chunk + 2) / 2);   // blk_first[chunk] then blk_prefix[chunk + 1] (u32)
+    for (int i0 = 0; i0 < count; i0 += chunk) {
+        const int n = std::min(chunk, count - i0);
+        uint32_t *prefix = reinterpret_cast<uint32_t *>(tab.data() + n);
+        uint64_t blocks = 0;
+        for (int i = 0; i < n; i++) {
+            const SampleInfo &s = c->samples[first_idx + i0 + i];
+            tab[i] = s.pos_off / EXT_BLOCK_POS;
+            prefix[i] = (uint32_t)blocks;
+            blocks += s.n_pos / EXT_BLOCK_POS;
+        }
+        if (blocks >= (1ull << 32)) PS_THROW(PS_ERR_ARG, "more than 2^32 stream blocks in one chunk");
+        prefix[n] = (uint32_t)blocks;
+        CK(cudaMemcpyAsync(c->cm_tab.p, tab.data(), (size_t)n * 8 + (size_t)(n + 1) * 4, cudaMemcpyHostToDevice, c->stream));
+        CK(cudaMemsetAsync(c->cm_cnt.p, 0, (size_t)n * Ku * 4, c->stream));
+        if (blocks) {
+            CntArgs a;
+            a.seq = c->pool_seq.as<uint32_t>(); a.bad = c->pool_bad.as<uint32_t>();
+            a.blk_first = c->cm_tab.as<uint64_t>();
+            a.blk_prefix = reinterpret_cast<const uint32_t *>(c->cm_tab.as<uint64_t>() + n);
+            a.nrows = n; a.k = c->k;
+            a.filter = c->cm_filter.as<uint32_t>();
+            a.queries = c->cm_q.as<uint64_t>(); a.qidx = c->cm_idx.as<uint32_t>(); a.ishift = ishift; a.Ku = Ku;
+            a.counts = c->cm_cnt.as<uint32_t>();
+            const unsigned grid = (unsigned)std::min<uint64_t>(PS_SMS, ceil_div<uint64_t>(blocks * (EXT_BLOCK_POS / CNT_UNIT), CNT_THREADS / 32));
+            if (key64(c))
+                KLAUNCH(c, "count_matrix", (double)blocks * EXT_BLOCK_POS * 3 / 8,
+                        (k_count_matrix<uint64_t><<<grid, CNT_THREADS, CNT_FILTER_WORDS * 4, c->stream>>>(a)));
+            else
+                KLAUNCH(c, "count_matrix", (double)blocks * EXT_BLOCK_POS * 3 / 8,
+                        (k_count_matrix<uint32_t><<<grid, CNT_THREADS, CNT_FILTER_WORDS * 4, c->stream>>>(a)));
+        }
+        const uint32_t *res = c->cm_cnt.as<uint32_t>();
+        if (!identity) {
+            const uint64_t m = (uint64_t)n * K;
+            KLAUNCH(c, "count_expand", (double)m * 12,
+                    (k_count_expand<<<(unsigned)std::min<uint64_t>(PS_SMS * 8, ceil_div<uint64_t>(m, 256)), 256, 0, c->stream>>>(
+                        res, Ku, c->cm_inv.as<uint32_t>(), K, m, c->cm_out.as<uint32_t>())));
+            res = c->cm_out.as<uint32_t>();
+        }
+        CK(cudaMemcpyAsync(counts + (size_t)i0 * K, res, (size_t)n * K * 4, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
     }
     API_END(c)
+}
+
+int ps_lookup(ps_ctx *c, int idx, const uint64_t *kmers, size_t K, uint32_t *counts) {
+    return ps_count_matrix(c, idx, 1, kmers, K, counts);
 }
 
 int ps_export_stream(ps_ctx *c, int idx, const void **seq, const void **bad, uint64_t *n_pos) {

@@ -171,6 +171,7 @@ struct ps_ctx {
     DevBuf pg_meta_a, pg_meta_b, pg_plist, pg_tiles, pg_tabs, pg_state, pg_blist;   // paged partition
     DevBuf mash_tab, mash_parts, mash_parts_n, mash_h, mash_n, mash_sd;              // ps_mash_sketch / ps_mash_pairs
     DevBuf nj_d, nj_d2, nj_act, nj_nd, nj_part, nj_out;                              // ps_neighbor_joining
+    DevBuf cm_q, cm_idx, cm_filter, cm_tab, cm_inv, cm_cnt, cm_out;                   // ps_count_matrix
 
     void *pinned = nullptr;  // small pinned scratch for readbacks
     size_t pinned_cap = 0;
@@ -188,7 +189,7 @@ struct ps_ctx {
                 &sv_bits, &sv_kmer, &tmp1, &tmp2, &tmp3, &pg_meta_a, &pg_meta_b, &pg_plist, &pg_tiles,
                 &pg_tabs, &pg_state, &pg_blist, &sel_ph, &sel_row, &sel_stat, &sel_p, &sel_mx, &sel_my, &sel_n,
                 &mash_tab, &mash_parts, &mash_parts_n, &mash_h, &mash_n, &mash_sd, &nj_d, &nj_d2, &nj_act, &nj_nd,
-                &nj_part, &nj_out};
+                &nj_part, &nj_out, &cm_q, &cm_idx, &cm_filter, &cm_tab, &cm_inv, &cm_cnt, &cm_out};
     }
 };
 

@@ -114,25 +114,6 @@ k_extract(const uint32_t *__restrict__ seq, const uint32_t *__restrict__ bad, ui
 
 #define PART_MAX 8   // GPUs of one routed job (ps_paged.cuh)
 
-// Occurrence counts of K sorted query k-mers within [pos_begin, pos_begin + nblocks*4096).
-template <typename KeyT>
-__global__ void __launch_bounds__(EXT_THREADS)
-k_lookup(const uint32_t *__restrict__ seq, const uint32_t *__restrict__ bad, uint64_t pos_begin,
-         int k, const uint64_t *__restrict__ queries, int K, uint32_t *__restrict__ counts) {
-    const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const uint64_t base = pos_begin + (uint64_t)blockIdx.x * EXT_BLOCK_POS + warp * (32 * EXT_ITERS);
-    for (int it = 0; it < EXT_ITERS; it++) {
-        KeyT key = 0;
-        if (!kmer_at<KeyT>(seq, bad, base + it * 32 + lane, k, key)) continue;
-        int a = 0, b = K;  // lower bound
-        while (a < b) {
-            int m = (a + b) >> 1;
-            if (__ldg(queries + m) < (uint64_t)key) a = m + 1; else b = m;
-        }
-        if (a < K && __ldg(queries + a) == (uint64_t)key) atomicAdd(counts + a, 1u);
-    }
-}
-
 // Gather per-sample counted lists (list mode) into the instance arrays, range-filtered, in
 // list order. One block handles 4096 list entries of one sample (lists padded likewise).
 template <typename KeyT, bool WRITE, int TAGS>

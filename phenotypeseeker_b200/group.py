@@ -11,7 +11,7 @@ reference's modeling() forks Pools after the tests). ctypes releases the GIL dur
 ranks' host work runs in parallel.
 
 Besides build and test, a group offers the per-sample device work of the drop-in, each on the context that holds
-the sample: lookup (-rc counts) and mash_sketch, with mash_pairs and neighbor_joining on the first context, so
+the sample: lookup and count_matrix (-rc counts) and mash_sketch, with mash_pairs and neighbor_joining on the first context, so
 that weights.gsc_weights_on_device takes a group as it takes a context.
 """
 import numpy as np
@@ -136,6 +136,23 @@ class GpuGroup:
     # per-sample device work (-rc counts, -w weights), on the context that holds the sample
     def lookup(self, sample, kmers):
         return self.engines[self._owner(sample)].lookup(sample, kmers)
+
+    def count_matrix(self, kmers, first_idx=0, count=None):
+        """(count, K) uint32 occurrences of `kmers` in samples first_idx .. first_idx + count - 1 (all from first_idx
+        by default): each rank counts its share on its own context, parts in sample order (Context.count_matrix)."""
+        first_idx = int(first_idx)
+        count = self.n_samples - first_idx if count is None else int(count)
+        q = np.ascontiguousarray(kmers, dtype=np.uint64)
+        wanted = range(first_idx, first_idx + count)
+
+        def one(r):
+            block = psdist.sample_block(r, self.world, self.n_samples)
+            lo, hi = max(block.start, wanted.start), min(block.stop, wanted.stop)
+            return self.engines[r].count_matrix(q, lo, hi - lo) if hi > lo else None
+        parts = [p for p in self._run(one) if p is not None]
+        if not parts:
+            return np.zeros((0, len(q)), dtype=np.uint32)
+        return np.concatenate(parts)
 
     def mash_sketch(self, first_idx, count, k=21, s=1000, seed=42):
         """Sketches of samples first_idx .. first_idx + count - 1, each rank's share on its own context, in sample

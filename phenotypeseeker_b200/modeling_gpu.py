@@ -170,7 +170,7 @@ def run_hot_path(files, sample_names, k, cutoff, pheno, pheno_names, binary, wei
         r.na_mask = np.isnan(np.asarray(pheno, dtype=np.float64).reshape(len(sample_names), -1)[:, j])
         counts = None
         if real_counts and len(r.kmer):
-            counts = np.stack([ka.lookup(s, r.kmer) for s in range(len(sample_names))], axis=1)
+            counts = ka.count_matrix(r.kmer).T
             counts = counts * (r.presence != 0)       # a count below the cutoff is 0 in the reference's list (glistmaker -c)
         out[r.name] = build_ml_df(r, k, sample_names, n_stripes, binary, counts)
     return U, out
@@ -260,7 +260,7 @@ def install(m, device=None, native_weights=None):
         res = test_all_columns()[self.name]
         counts = None
         if phenotypes.real_counts and len(res.kmer):
-            counts = np.stack([ka.lookup(s, res.kmer) for s in range(len(names))], axis=1)
+            counts = ka.count_matrix(res.kmer).T
             counts = counts * (res.presence != 0)         # a count below the cutoff is 0 in the reference's list (glistmaker -c)
         self.ML_df = build_ml_df(res, ka.k, names, Input.num_threads, binary, counts)
         if self.ML_df.shape[0] == 0:

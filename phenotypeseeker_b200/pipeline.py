@@ -230,6 +230,12 @@ class KmerAssociation:
         """Counts of `kmers` in one sample (ps_lookup)."""
         return self.ctx.lookup(sample, kmers)
 
+    def count_matrix(self, kmers, first_idx=0, count=None):
+        """(count, K) uint32 occurrences of `kmers` in samples first_idx .. first_idx + count - 1 (all samples from
+        first_idx by default): one device pass (ps_count_matrix)."""
+        count = self.n_samples - int(first_idx) if count is None else int(count)
+        return self.ctx.count_matrix(first_idx, count, kmers)
+
     def mash_sketch(self, first_idx, count, k=21, s=1000, seed=42):
         return self.ctx.mash_sketch(first_idx, count, k, s, seed)
 
