@@ -221,7 +221,7 @@ static BucketTables bucket_tables(ps_ctx *c) {
 // ---------------------------------------------------------------------------------------
 // Paged build (ps_paged.cuh) for k = 9..16: k_scatter1 (extraction fused with the level-1 partition)
 // -> page lists -> k_scatter2 -> bucket page lists -> k_bucket_count_pg / k_bucket_build_pg.
-static inline bool paged_ok(const ps_ctx *c) { return c->paged && c->bucketed && c->k >= 9 && c->k <= 16; }
+static inline bool paged_ok(const ps_ctx *c) { return c->bucketed && c->k >= 9 && c->k <= 16; }
 static inline int paged_groups(const ps_ctx *c) { return (c->n_samples + 255) / 256; }
 
 // u32 tables of the paged build inside c->pg_tabs
@@ -334,6 +334,10 @@ static void launch_scatter1(ps_ctx *c, const Sc1Src &src, const Sc1Dst &dst) {
                 (k_scatter1<SRC, false><<<std::min(grid, 2 * PS_SMS), SC_THREADS, smem, c->stream>>>(src, dst, c->pg_state.as<ScState>(), t.ticket)));
 }
 
+// Thrown by paged_finish when records did not fit the page pools (PS_ERR_NOMEM): callers that can take larger pools
+// catch this type and build again.
+struct PagePoolExhausted : PsError {};
+
 // level-1 pages (this GPU's pool, pgA_cap pages, metas final) -> union + matrix
 // bin_lo / bin_hi: only the level-1 bins [bin_lo, bin_hi) take part (a sub-range of what the pool was scattered
 // for); rezero: the tables of an earlier paged_finish on the same pool are cleared first (everything but the
@@ -389,22 +393,15 @@ static void paged_finish(ps_ctx *c, const Sc1Dst &dst_for_close, bool close_loca
     const int nwords = lbits >= 5 ? (1 << (lbits - 5)) : 1;
     c->tmp1.reserve((size_t)BK_N * nwords * 4, c->stream);
     uint32_t *gbm = c->tmp1.as<uint32_t>();
-    if (c->bk_tma)
-        KLAUNCH(c, "bucket_count", (double)n_upper * 4,
-                (k_bucket_count_pg<true><<<BK_N, BK_THREADS, BKP_RING_WORDS * 4, c->stream>>>(
-                    a.recs_b, c->pg_blist.as<unsigned long long>(), bt.bstart, G, bt.order, lbits, bt.counts, gbm)));
-    else
-        KLAUNCH(c, "bucket_count", (double)n_upper * 4,
-                (k_bucket_count_pg<false><<<BK_N, BK_THREADS, 0, c->stream>>>(
-                    a.recs_b, c->pg_blist.as<unsigned long long>(), bt.bstart, G, bt.order, lbits, bt.counts, gbm)));
+    KLAUNCH(c, "bucket_count", (double)n_upper * 4,
+            (k_bucket_count_pg<<<BK_N, BK_THREADS, 0, c->stream>>>(
+                a.recs_b, c->pg_blist.as<unsigned long long>(), bt.bstart, G, bt.order, lbits, bt.counts, gbm)));
     KLAUNCH(c, "scan_counts", (double)BK_N * 12, (k_scan_counts<<<1, 1024, 0, c->stream>>>(bt.counts, BK_N, bt.first_row)));
     const uint32_t stride = (uint32_t)std::min(c->row_words, 8) + 1;      // rows are assembled in 8-word column slices
     const uint32_t cap_small = (uint32_t)std::max(c->bk_row_words, round_up<int>((int)stride, 4));
-    const bool tma = c->bk_tma;
-    const int ring_words = tma ? BKP_RING_WORDS : 0;
-    const uint32_t cap_big = (uint32_t)std::max<int>((BK_MAX_DYN_SMEM - nwords * 8 - ring_words * 4) / 4 & ~3, (int)cap_small);
+    const uint32_t cap_big = (uint32_t)std::max<int>((BK_MAX_DYN_SMEM - nwords * 8) / 4 & ~3, (int)cap_small);
     KLAUNCH(c, "pg_lists", 0.0,
-            (k_bucket_order_rows<<<BK_N / 256, 256, 0, c->stream>>>(bt.counts, cap_small / stride, bt.fill + 2, bt.order2)));
+            (k_bucket_order_pg<<<BK_N / 256, 256, 0, c->stream>>>(bt.counts, cap_small / stride, bt.fill + 2, bt.order2)));
     unsigned long long *h = (unsigned long long *)ps_pinned(c, 64);
     uint32_t *h32 = reinterpret_cast<uint32_t *>(h + 1);
     CK(cudaMemcpyAsync(h, bt.first_row + BK_N, 8, cudaMemcpyDeviceToHost, c->stream));
@@ -413,7 +410,11 @@ static void paged_finish(ps_ctx *c, const Sc1Dst &dst_for_close, bool close_loca
     CK(cudaMemcpyAsync(h32 + 2, t.cursor_a, 4, cudaMemcpyDeviceToHost, c->stream));
     CK(cudaMemcpyAsync(h32 + 3, t.cursor_b, 4, cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
-    if (h32[1]) PS_THROW(PS_ERR_NOMEM, "page pool exhausted (level-1 %u of %u pages, level-2 %u of %u)", h32[2], c->pgA_cap, h32[3], c->pgB_cap);
+    if (h32[1]) {
+        char m[160];
+        snprintf(m, sizeof(m), "page pool exhausted (level-1 %u of %u pages, level-2 %u of %u)", h32[2], c->pgA_cap, h32[3], c->pgB_cap);
+        throw PagePoolExhausted{{PS_ERR_NOMEM, m}};
+    }
     const uint64_t U = h[0];
     const uint32_t nbig = h32[0];
     c->U = U;
@@ -421,22 +422,19 @@ static void paged_finish(ps_ctx *c, const Sc1Dst &dst_for_close, bool close_loca
     c->uni.reserve(std::max<uint64_t>(U, 1) * 8, c->stream);
     c->matrix.reserve(U * row_bytes + 64, c->stream);
     const double alg = (double)n_upper * 4 + (double)U * (8 + row_bytes);
-    const size_t sm_small = (size_t)(ring_words + cap_small) * 4 + (size_t)nwords * 8;
-    const size_t sm_big = (size_t)(ring_words + cap_big) * 4 + (size_t)nwords * 8;
-#define PS_BUILD_PG(NT, TMA_, GRID, SMEM, ORD, CAP, SHARE)                                                             \
-    KLAUNCH(c, "bucket_build", alg * (SHARE) / BK_N,                                                                   \
-            (k_bucket_build_pg<NT, TMA_><<<(GRID), NT, (SMEM), c->stream>>>(                                           \
-                a.recs_b, c->pg_blist.as<unsigned long long>(), bt.bstart, G, (ORD), bt.first_row, gbm, lbits, c->row_words, (CAP), \
-                c->uni.as<uint64_t>(), c->matrix.as<uint32_t>())))
-    if (nbig) {
-        if (tma) PS_BUILD_PG(BK_MAX_THREADS, true, nbig, sm_big, bt.order2, cap_big, nbig);
-        else PS_BUILD_PG(BK_MAX_THREADS, false, nbig, sm_big, bt.order2, cap_big, nbig);
-    }
-    if (nbig < BK_N) {
-        if (tma) PS_BUILD_PG(BK_THREADS, true, BK_N - nbig, sm_small, bt.order2 + nbig, cap_small, BK_N - nbig);
-        else PS_BUILD_PG(BK_THREADS, false, BK_N - nbig, sm_small, bt.order2 + nbig, cap_small, BK_N - nbig);
-    }
-#undef PS_BUILD_PG
+    const size_t sm_small = (size_t)cap_small * 4 + (size_t)nwords * 8;
+    const size_t sm_big = (size_t)cap_big * 4 + (size_t)nwords * 8;
+    const unsigned long long *blist = c->pg_blist.as<unsigned long long>();
+    if (nbig)
+        KLAUNCH(c, "bucket_build", alg * nbig / BK_N,
+                (k_bucket_build_pg<BK_MAX_THREADS><<<nbig, BK_MAX_THREADS, sm_big, c->stream>>>(
+                    a.recs_b, blist, bt.bstart, G, bt.order2, bt.first_row, gbm, lbits, c->row_words, cap_big,
+                    c->uni.as<uint64_t>(), c->matrix.as<uint32_t>())));
+    if (nbig < BK_N)
+        KLAUNCH(c, "bucket_build", alg * (BK_N - nbig) / BK_N,
+                (k_bucket_build_pg<BK_THREADS><<<BK_N - nbig, BK_THREADS, sm_small, c->stream>>>(
+                    a.recs_b, blist, bt.bstart, G, bt.order2 + nbig, bt.first_row, gbm, lbits, c->row_words, cap_small,
+                    c->uni.as<uint64_t>(), c->matrix.as<uint32_t>())));
 }
 
 // single-GPU bin -> d2 table (bin = d2, one destination)
@@ -606,20 +604,11 @@ static void add_samples_impl(ps_ctx *c, int first_idx, int count, const void *co
         uint32_t fmt_seen = 0;                       // bit f set: some file of the group has format f
         for (int i = f0; i < f0 + nf; i++) fmt_seen |= 1u << files[i].fmt;
         fmt_seen &= ~1u;
-#define PS_DECODE_WRITE(F)                                                                                            \
-        KLAUNCH(c, "decode_write", (double)gbytes + (double)(pp - gp0) * 3 / 8,                                       \
-                (k_decode_write<F><<<nt, DEC_THREADS, 0, c->stream>>>(stg, d_files, d_tile_file, t0, d_tile_state,      \
-                                                                      d_tile_off, d_chunk_next, d_chunk_cnt,            \
-                                                                      c->pool_seq.as<uint32_t>(), c->pool_bad.as<uint32_t>())))
-        if (fmt_seen == 2u && !c->dec_bytes)
-            KLAUNCH(c, "decode_write", (double)gbytes + (double)(pp - gp0) * 3 / 8,
-                    (k_decode_write_fasta<<<nt, DEC_THREADS, 0, c->stream>>>(stg, d_files, d_tile_file, t0, d_tile_state, d_tile_off,
-                                                                             d_chunk_next, d_chunk_cnt, c->pool_seq.as<uint32_t>(),
-                                                                             c->pool_bad.as<uint32_t>())));
-        else if (fmt_seen == 2u) PS_DECODE_WRITE(1);
-        else if (fmt_seen == 4u) PS_DECODE_WRITE(2);
-        else PS_DECODE_WRITE(0);
-#undef PS_DECODE_WRITE
+        // all FASTA: the word-wide write pass; otherwise the byte transducer, FASTQ-only or per file
+        auto *write = fmt_seen == 2u ? k_decode_write_fasta : fmt_seen == 4u ? k_decode_write<2> : k_decode_write<0>;
+        KLAUNCH(c, "decode_write", (double)gbytes + (double)(pp - gp0) * 3 / 8,
+                (write<<<nt, DEC_THREADS, 0, c->stream>>>(stg, d_files, d_tile_file, t0, d_tile_state, d_tile_off, d_chunk_next,
+                                                          d_chunk_cnt, c->pool_seq.as<uint32_t>(), c->pool_bad.as<uint32_t>())));
         for (int i = f0; i < f0 + nf; i++) if (files[i].fmt == 2) pre = false;   // raw reads: counted per sample
         if (!pre) { c->pre_valid = false; c->pgA_live = false; }
         if (pre && pp > gp0) {
@@ -813,8 +802,8 @@ static void build_union_impl(ps_ctx *c) {
                     try {
                         paged_finish(c, paged_local_dst(c), false, bin_d2, n_upper, blo, bhi, true);
                         break;
-                    } catch (const PsError &e) {
-                        if (e.code != PS_ERR_NOMEM || e.msg.find("page pool exhausted") == std::string::npos || attempt >= 3) throw;
+                    } catch (const PagePoolExhausted &) {
+                        if (attempt >= 3) throw;
                         n_upper = std::min<uint64_t>(c->l1_instances, n_upper * 2);      // level 2 ran out: larger pool, same level 1
                     }
                 }
@@ -835,9 +824,9 @@ static void build_union_impl(ps_ctx *c) {
             try {
                 paged_finish(c, d, true, bin_d2, n_upper);
                 break;
-            } catch (const PsError &e) {
+            } catch (const PagePoolExhausted &) {
                 // a range held more instances than the hint said: take the pages it needs and go again
-                if (e.code != PS_ERR_NOMEM || e.msg.find("page pool exhausted") == std::string::npos || attempt >= 3) throw;
+                if (attempt >= 3) throw;
                 n_upper = std::min<uint64_t>(n_all, n_upper * 2);
             }
         }
@@ -1073,23 +1062,18 @@ int ps_ctx_create(int device, ps_ctx **out) {
     cudaFuncSetAttribute(k_scatter1<1, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     cudaFuncSetAttribute(k_scatter2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SC2_SMEM);
     cudaFuncSetAttribute(k_scatter2, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-#define PS_BKPG_ATTR(NT, T)                                                                                      \
-    cudaFuncSetAttribute(k_bucket_build_pg<NT, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, BK_MAX_DYN_SMEM); \
-    cudaFuncSetAttribute(k_bucket_build_pg<NT, T>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-    PS_BKPG_ATTR(BK_THREADS, true) PS_BKPG_ATTR(BK_THREADS, false) PS_BKPG_ATTR(BK_MAX_THREADS, true) PS_BKPG_ATTR(BK_MAX_THREADS, false)
-#undef PS_BKPG_ATTR
-    cudaFuncSetAttribute(k_bucket_count_pg<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    cudaFuncSetAttribute(k_bucket_build_pg<BK_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, BK_MAX_DYN_SMEM);
+    cudaFuncSetAttribute(k_bucket_build_pg<BK_THREADS>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    cudaFuncSetAttribute(k_bucket_build_pg<BK_MAX_THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, BK_MAX_DYN_SMEM);
+    cudaFuncSetAttribute(k_bucket_build_pg<BK_MAX_THREADS>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     cudaFuncSetAttribute(k_mash_sketch, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mash_smem(PSM_S_MAX));
     cudaFuncSetAttribute(k_mash_merge, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)mash_smem(PSM_S_MAX));
     cudaFuncSetAttribute(k_count_matrix<uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(CNT_FILTER_WORDS * 4));
     cudaFuncSetAttribute(k_count_matrix<uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(CNT_FILTER_WORDS * 4));
-    cudaFuncSetAttribute(k_bucket_count_pg<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-    if (const char *ev = getenv("PSKMER_BK_TMA")) c->bk_tma = atoi(ev) != 0;
-    if (const char *ev = getenv("PSKMER_PAGED")) c->paged = atoi(ev) != 0;
-    if (const char *ev = getenv("PSKMER_DECODE")) c->dec_bytes = strcmp(ev, "bytes") == 0;
+    cudaFuncSetAttribute(k_bucket_count_pg, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
     if (const char *ev = getenv("PSKMER_SC1")) c->sc1_lean = strcmp(ev, "regs") != 0;
     if (c->sc1_lean) c->sc1_grid = 3 * PS_SMS;
-    if (const char *ev = getenv("PSKMER_CHI2")) { c->chi2_sparse = strcmp(ev, "masked") != 0; c->chi2_sparse_force = strcmp(ev, "walk") == 0; }
+    if (const char *ev = getenv("PSKMER_CHI2")) c->chi2_sparse_force = strcmp(ev, "walk") == 0;
     if (const char *ev = getenv("PSKMER_ROWS")) c->bucketed = strcmp(ev, "sorted") != 0;
     if (const char *ev = getenv("PSKMER_BK_ROW_KB")) {
         const int kb = atoi(ev);
@@ -1423,9 +1407,9 @@ int ps_test_chi2(ps_ctx *c, int P, const int8_t *pheno, const double *weights, i
         d_w = c->weights.as<double>();
     }
     // Unweighted tables: per-sample packed column membership for the bit-walk kernel (k_test_chi2_sp),
-    // ten columns per pair of u64 (five 12-bit fields each); PSKMER_CHI2=masked keeps the masked-popcount kernel.
-    // (it pays once a row times the column count is large: below ~512 mask words per row the masked popcounts are cheaper)
-    const bool sparse_walk = !weights && N <= 8190 && c->chi2_sparse && (c->chi2_sparse_force || (size_t)wp * P >= 512);
+    // ten columns per pair of u64 (five 12-bit fields each). It pays once a row times the column count is large:
+    // below ~512 mask words per row the masked popcounts are cheaper.
+    const bool sparse_walk = !weights && N <= 8190 && (c->chi2_sparse_force || (size_t)wp * P >= 512);
     bool no_na = true;
     const ulonglong2 *d_e1 = nullptr, *d_e0 = nullptr;
     const int *d_tot1 = nullptr, *d_tot0 = nullptr;
@@ -1950,9 +1934,8 @@ int ps_route_build(ps_ctx *c, uint64_t *n_union, int *overflow) {
     int ovf = 0;
     try {
         paged_finish(c, Sc1Dst(), false, bin_d2, (uint64_t)c->pgA_cap * PG_A);
-    } catch (const PsError &e) {
+    } catch (const PagePoolExhausted &) {
         // a sender ran out of pages on some GPU: report it, every rank must learn about it together
-        if (e.code != PS_ERR_NOMEM || e.msg.find("page pool exhausted") == std::string::npos) throw;
         ovf = 1;
     }
     if (overflow) *overflow = ovf; else if (ovf) PS_THROW(PS_ERR_NOMEM, "page pool exhausted while routing");

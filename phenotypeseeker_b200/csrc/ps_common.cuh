@@ -123,14 +123,10 @@ struct ps_ctx {
     bool bucketed = true;
     int bk_row_words = 10240;   // shared-memory words of k_bucket_build's row table for ordinary buckets (PSKMER_BK_ROW_KB)
 
-    bool dec_bytes = false;     // PSKMER_DECODE=bytes: all-FASTA launches take the staged-byte write pass k_decode_write<1> instead of k_decode_write_fasta (A/B runs; =swar names the default)
     bool sc1_lean = true;       // k_scatter1 recomputes its k-mers in the grouping phase (40 registers, 3 blocks per SM); PSKMER_SC1=regs: keeps them in registers (2 blocks per SM)
     bool chi2_sparse_force = false;   // PSKMER_CHI2=walk: the bit-walk kernel for every unweighted shape it can take (tests)
-    bool chi2_sparse = true;    // unweighted chi2 walks the row's bits (k_test_chi2_sp); PSKMER_CHI2=masked: one masked popcount per column
 
     // paged partition (ps_paged.cuh): level-1 pool = keys_a, level-2 pool = keys_b
-    bool bk_tma = false;        // PSKMER_BK_TMA=1: bucket kernels read their pages through a TMA ring instead of 128-bit loads
-    bool paged = true;          // PSKMER_PAGED=0: never (k_part_pass / full-sort paths instead)
     int sc1_grid = 2 * PS_SMS, sc2_grid = 2 * PS_SMS;
     uint32_t pgA_cap = 0, pgB_cap = 0;   // pages
     double sc1_out_frac = 1.0;  // share of the positions whose record k_scatter1 writes (range-restricted runs): profile accounting only

@@ -13,7 +13,7 @@
 // chunk its true incoming state and output offset. Pass 1 (k_decode_count) produces tile
 // summaries, k_decode_walk walks them per file, pass 2 re-simulates with the known state and packs
 // 16 bases / 32 mask bits per word: k_decode_write_fasta from per-thread bit strings when a launch is
-// all FASTA (ps_decode_bits.h), k_decode_write from staged code bytes otherwise.
+// all FASTA (ps_decode_bits.h), k_decode_write from staged code bytes when it holds FASTQ.
 #pragma once
 #include "ps_common.cuh"
 #include "ps_decode_bits.h"
@@ -302,9 +302,10 @@ __global__ void k_decode_walk(FileEnt *__restrict__ files, int nfiles,
     f.m = off;
 }
 
-// Pass 2: emit codes with the known state, pack and store. FMT = 1 / 2: every file of the launch is FASTA /
-// FASTQ (or empty), so only that transducer is compiled into the 64-byte emit loop — half the kernel body
-// (the generic body stalled on instruction fetch half the time); FMT = 0: mixed launch, format per file.
+// Pass 2 for launches that hold FASTQ: emit codes with the known state, pack and store. FMT = 2: every file of the
+// launch is FASTQ (or empty), so only that transducer is compiled into the 64-byte emit loop — half the kernel body
+// (the generic body stalled on instruction fetch half the time); FMT = 0: mixed launch, format per file. All-FASTA
+// launches take k_decode_write_fasta.
 template <int FMT>
 __global__ void __launch_bounds__(DEC_THREADS)
 k_decode_write(const uint8_t *__restrict__ staging, const FileEnt *__restrict__ files,
@@ -312,6 +313,7 @@ k_decode_write(const uint8_t *__restrict__ staging, const FileEnt *__restrict__ 
                const uint32_t *__restrict__ tile_state, const uint32_t *__restrict__ tile_off,
                const uint32_t *__restrict__ chunk_next, const uint64_t *__restrict__ chunk_cnt,
                uint32_t *__restrict__ pool_seq, uint32_t *__restrict__ pool_bad) {
+    static_assert(FMT == 0 || FMT == 2, "k_decode_write: mixed (0) or FASTQ-only (2) launches");
     __shared__ DecSum sm[DEC_THREADS / 32 + 1];
     // codes are staged at (position - first 32-position group of the tile), so that every
     // group is one aligned 32-byte span of shared memory
@@ -381,10 +383,11 @@ k_decode_write(const uint8_t *__restrict__ staging, const FileEnt *__restrict__ 
     }
 }
 
-// Pass 2 for launches whose files are all FASTA (or empty): the same result as k_decode_write<1>, built from
-// per-thread bit strings instead of one staged code byte per position (ps_decode_bits.h). The chunk's 16 words
-// go through a shared-memory row so that the word loop stays rolled — the byte-loop kernel's fully unrolled body
-// (3,984 SASS instructions) stalled on instruction fetch a third of the time.
+// Pass 2 for launches whose files are all FASTA (or empty): the same result as the byte transducer of
+// k_decode_write, built from per-thread bit strings instead of one staged code byte per position
+// (ps_decode_bits.h). The chunk's 16 words go through a shared-memory row so that the word loop stays rolled — the
+// byte loop's fully unrolled body for FASTA (3,984 SASS instructions) stalled on instruction fetch a third of the
+// time.
 #define DEC_OUT_POS (DEC_TILE + POS_ALIGN + 64)
 __global__ void __launch_bounds__(DEC_THREADS)
 k_decode_write_fasta(const uint8_t *__restrict__ staging, const FileEnt *__restrict__ files,

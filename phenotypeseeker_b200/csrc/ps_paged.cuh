@@ -39,7 +39,6 @@
 #define PG_A 1024            // records per level-1 page (4 KB)
 #define PG_A_LOG 10
 #define PG_B 512             // records per level-2 page (2 KB)
-#define PG_B_LOG 9
 #define SC_THREADS 512
 #define SC_ITEMS 16
 #define SC_TILE (SC_THREADS * SC_ITEMS)      // 8192 positions / records per tile

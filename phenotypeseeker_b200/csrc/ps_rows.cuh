@@ -27,7 +27,7 @@ k_row_build(const KeyT *__restrict__ keys, const uint16_t *__restrict__ tags, ui
     unsigned long long run = chunk_offs[chunk];  // heads before this chunk
     for (int it = 0; it < RUN_CHUNK / 32; it++) {
         const uint64_t i = base + it * 32 + lane;
-        bool valid = i < n;
+        const bool valid = i < n;
         KeyT kk = 0;
         uint16_t tag = 0;
         bool head = false, dup = false;
@@ -36,8 +36,7 @@ k_row_build(const KeyT *__restrict__ keys, const uint16_t *__restrict__ tags, ui
                 const KeyT rec = keys[i];
                 kk = rec >> 16;
                 tag = (uint16_t)(rec & 0xFFFFu);
-                if (kk == (KeyT(~KeyT(0)) >> 16)) valid = false;   // sentinel of k_extract_direct
-                else if (i == 0) head = true;
+                if (i == 0) head = true;
                 else {
                     const KeyT prev = keys[i - 1];
                     head = kk != (prev >> 16);
@@ -88,15 +87,6 @@ k_row_build(const KeyT *__restrict__ keys, const uint16_t *__restrict__ tags, ui
 #define BK_MAX_DYN_SMEM (220 * 1024)
 #define BK_WPT 4            // bitmap words per thread at lbits = 16 (2048 words / 512 threads)
 
-// same split on the number of distinct k-mers (rows) once k_bucket_count has run
-__global__ void k_bucket_order_rows(const uint32_t *__restrict__ counts, uint32_t big, uint32_t *__restrict__ fill,
-                                    uint32_t *__restrict__ order) {
-    const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= BK_N) return;
-    const uint32_t pos = counts[b] > big ? atomicAdd(fill, 1u) : (uint32_t)(BK_N - 1) - atomicAdd(fill + 1, 1u);
-    order[pos] = b;
-}
-
 // bm[w].y = number of set presence bits below word w; returns the number of distinct k-mers.
 // Ends with a barrier: bm is complete for every thread on return.
 template <int NT>
@@ -143,68 +133,11 @@ __device__ __forceinline__ uint32_t bk_ranks(int nwords, uint2 *bm, uint32_t *s_
 
 // ---------------------------------------------------------------------------------------
 // Paged variants (ps_paged.cuh): a bucket is a LIST of level-2 pages (<= 512 records each, 4-byte
-// records low << 8 | sample & 255, the page carries the sample group). The pages of a bucket come in
-// through the TMA unit: one thread issues cp.async.bulk copies of BKP_SP pages per stage into a ring
-// of BKP_NS shared-memory stages, every stage completes on its own mbarrier, and the block consumes
-// stage i while the copies of stages i+1 .. i+BKP_NS-1 are in flight.
-#define BKP_SP 4                 // pages per stage (8 KB)
-#define BKP_NS 3                 // stages in flight
-#define BKP_RING_WORDS (BKP_NS * BKP_SP * PG_B)
-struct BkRing {
-    unsigned long long bar[BKP_NS];
-    uint32_t cnt[BKP_NS][BKP_SP];
-    uint32_t grp[BKP_NS][BKP_SP];
-};
-
-// calls f(record, group) for every record of pages [0, npages) of one bucket; `iter` is the running
-// stage counter of this block (mbarrier parity), carried across calls. Ends with a barrier.
-template <int NT, typename F>
-__device__ __forceinline__ void bk_for_each(const unsigned long long *__restrict__ pages, uint32_t npages,
-                                            const uint32_t *__restrict__ recs_b, uint32_t *ring, BkRing &R,
-                                            uint32_t &iter, F f) {
-    const unsigned tid = threadIdx.x;
-    const uint32_t nst = (npages + BKP_SP - 1) / BKP_SP;
-    auto issue = [&](uint32_t s, uint32_t slot) {
-        uint32_t bytes = 0, pc[BKP_SP], pg[BKP_SP];
-#pragma unroll
-        for (int j = 0; j < BKP_SP; j++) {
-            pc[j] = 0;
-            const uint32_t pi = s * BKP_SP + j;
-            if (pi < npages) {
-                const unsigned long long e = pages[pi];
-                pc[j] = BKP_CNT(e); pg[j] = BKP_PAGE(e);
-                R.grp[slot][j] = BKP_GRP(e);
-            }
-            R.cnt[slot][j] = pc[j];
-            bytes += (pc[j] * 4 + 15) & ~15u;
-        }
-        mbar_expect_tx(reinterpret_cast<uint64_t *>(&R.bar[slot]), bytes);
-#pragma unroll
-        for (int j = 0; j < BKP_SP; j++)
-            if (pc[j]) bulk_g2s(ring + (slot * BKP_SP + j) * PG_B, recs_b + (size_t)pg[j] * PG_B, (pc[j] * 4 + 15) & ~15u,
-                                reinterpret_cast<uint64_t *>(&R.bar[slot]));
-    };
-    if (tid == 0)
-        for (uint32_t s = 0; s < nst && s < BKP_NS - 1; s++) issue(s, (iter + s) % BKP_NS);
-    for (uint32_t s = 0; s < nst; s++) {
-        const uint32_t it = iter + s, slot = it % BKP_NS;
-        if (tid == 0 && s + BKP_NS - 1 < nst) issue(s + BKP_NS - 1, (it + BKP_NS - 1) % BKP_NS);
-        mbar_wait(reinterpret_cast<uint64_t *>(&R.bar[slot]), (it / BKP_NS) & 1u);
-        const uint32_t *src = ring + slot * BKP_SP * PG_B;
-#pragma unroll
-        for (int q0 = 0; q0 < BKP_SP * PG_B; q0 += NT) {
-            const uint32_t q = q0 + tid;
-            const uint32_t j = q >> PG_B_LOG;
-            if ((q & (PG_B - 1)) < R.cnt[slot][j]) f(src[q], R.grp[slot][j]);
-        }
-        __syncthreads();             // the stage may be overwritten by the copy issued next iteration
-    }
-    iter += nst;
-}
-
-// The same traversal without staging: warp w takes pages w, w + NT/32, ...; a page (2 KB) is four
-// coalesced 128-bit loads per lane, all independent, nothing shared between warps — no barriers and no
-// shared-memory round trip (the bucket kernels are shared-memory bound: bitmap tests and row atomics).
+// records low << 8 | sample & 255, the page carries the sample group). Warp w of a block takes pages w, w + NT/32,
+// ...; a page (2 KB) is four coalesced 128-bit loads per lane, all independent, nothing shared between warps: no
+// barriers and no shared-memory round trip. The pages are not staged in shared memory because the bucket kernels are
+// shared-memory bound (bitmap tests and row atomics); a cp.async.bulk ring that staged them was measured slower.
+// calls f(record, group) for every record of pages [0, npages) of one bucket; no barrier at the end.
 template <int NT, typename F>
 __device__ __forceinline__ void bk_for_each_direct(const unsigned long long *__restrict__ pages, uint32_t npages,
                                                    const uint32_t *__restrict__ recs_b, F f) {
@@ -228,23 +161,23 @@ __device__ __forceinline__ void bk_for_each_direct(const unsigned long long *__r
     }
 }
 
-__global__ void k_bucket_order_pg(const uint32_t *__restrict__ brecs, uint32_t big, uint32_t *__restrict__ fill,
+// order = the buckets with size[b] > big (from the front), then the others (from the back); size is the records of
+// a bucket for k_bucket_count_pg and its distinct k-mers for k_bucket_build_pg. fill: two zeroed counters, and
+// fill[0] ends as the number of big buckets.
+__global__ void k_bucket_order_pg(const uint32_t *__restrict__ size, uint32_t big, uint32_t *__restrict__ fill,
                                   uint32_t *__restrict__ order) {
     const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= BK_N) return;
-    const uint32_t pos = brecs[b] > big ? atomicAdd(fill, 1u) : (uint32_t)(BK_N - 1) - atomicAdd(fill + 1, 1u);
+    const uint32_t pos = size[b] > big ? atomicAdd(fill, 1u) : (uint32_t)(BK_N - 1) - atomicAdd(fill + 1, 1u);
     order[pos] = b;
 }
 
-template <bool TMA>
 __global__ void __launch_bounds__(BK_THREADS)
 k_bucket_count_pg(const uint32_t *__restrict__ recs_b, const unsigned long long *__restrict__ blist,
                   const unsigned long long *__restrict__ bpstart, uint32_t G, const uint32_t *__restrict__ order, int lbits,
                   uint32_t *__restrict__ counts, uint32_t *__restrict__ gbm) {
     constexpr int NT = BK_THREADS;
     __shared__ uint32_t bits[BK_N / 32];
-    extern __shared__ __align__(128) uint32_t bkc_ring[];            // TMA only: BKP_RING_WORDS
-    __shared__ __align__(8) BkRing R;
     __shared__ uint32_t s_part[NT / 32];
     const unsigned tid = threadIdx.x;
     const uint32_t b = order[blockIdx.x];
@@ -253,10 +186,6 @@ k_bucket_count_pg(const uint32_t *__restrict__ recs_b, const unsigned long long 
     if (npages == 0) { if (tid == 0) counts[b] = 0; return; }
     const int nwords = lbits >= 5 ? (1 << (lbits - 5)) : 1;
     for (int i = tid; i < nwords; i += NT) bits[i] = 0u;
-    if (TMA && tid == 0) {
-        for (int s = 0; s < BKP_NS; s++) mbar_init(reinterpret_cast<uint64_t *>(&R.bar[s]), 1);
-        mbar_fence_init();
-    }
     __syncthreads();
     const uint32_t lmask = (1u << lbits) - 1u;
     volatile uint32_t *vb = bits;
@@ -266,13 +195,8 @@ k_bucket_count_pg(const uint32_t *__restrict__ recs_b, const unsigned long long 
         const uint32_t bit = 1u << (low & 31);
         if (!(vb[low >> 5] & bit)) atomicOr(&bits[low >> 5], bit);
     };
-    if (TMA) {
-        uint32_t iter = 0;
-        bk_for_each<NT>(blist + ps, npages, recs_b, bkc_ring, R, iter, mark);
-    } else {
-        bk_for_each_direct<NT>(blist + ps, npages, recs_b, mark);
-        __syncthreads();
-    }
+    bk_for_each_direct<NT>(blist + ps, npages, recs_b, mark);
+    __syncthreads();
     uint32_t *g = gbm + (size_t)b * nwords;
     uint32_t cnt = 0;
     for (int i = tid; i < nwords; i += NT) {
@@ -296,20 +220,17 @@ k_bucket_count_pg(const uint32_t *__restrict__ recs_b, const unsigned long long 
 // a bucket are listed by sample group, and a page's group is exactly that slice): a row of 5,000 samples is
 // 640 bytes, far too wide to keep hundreds of them in shared memory, while a slice is 32 bytes — the table
 // holds ~1,100 rows whatever N is. Every slice of every row is written exactly once (absent groups as zeros).
-// dynamic shared memory: [ring (BKP_RING_WORDS), TMA only] | rows (row_cap_words) | bm (nwords uint2)
-template <int NT, bool TMA>
+// dynamic shared memory: rows (row_cap_words) | bm (nwords uint2)
+template <int NT>
 __global__ void __launch_bounds__(NT)
 k_bucket_build_pg(const uint32_t *__restrict__ recs_b, const unsigned long long *__restrict__ blist,
                   const unsigned long long *__restrict__ bpstart, uint32_t G, const uint32_t *__restrict__ order,
                   const unsigned long long *__restrict__ first_row, const uint32_t *__restrict__ gbm, int lbits, int wp,
                   uint32_t row_cap_words, uint64_t *__restrict__ union_out, uint32_t *__restrict__ matrix) {
-    extern __shared__ __align__(128) uint32_t bkp_dyn[];
+    extern __shared__ __align__(8) uint32_t rows[];
     const int nwords = lbits >= 5 ? (1 << (lbits - 5)) : 1;
-    uint32_t *ring = bkp_dyn;                                               // 128-byte aligned landing zones first
-    uint32_t *rows = bkp_dyn + (TMA ? BKP_RING_WORDS : 0);
     uint2 *bm = reinterpret_cast<uint2 *>(rows + row_cap_words);
     __shared__ uint32_t s_wsum[33];
-    __shared__ __align__(8) BkRing R;
     const unsigned tid = threadIdx.x;
     const uint32_t b = order[blockIdx.x];
     const unsigned long long *bp = bpstart + (size_t)b * G;
@@ -319,10 +240,6 @@ k_bucket_build_pg(const uint32_t *__restrict__ recs_b, const unsigned long long 
     if (D == 0) return;
     const uint32_t *g0 = gbm + (size_t)b * nwords;
     for (int i = tid; i < nwords; i += NT) bm[i] = make_uint2(g0[i], 0u);
-    if (TMA && tid == 0) {
-        for (int s = 0; s < BKP_NS; s++) mbar_init(reinterpret_cast<uint64_t *>(&R.bar[s]), 1);
-        mbar_fence_init();
-    }
     __syncthreads();
     bk_ranks<NT>(nwords, bm, s_wsum);
     const int wpt = (nwords + NT - 1) / NT;
@@ -344,7 +261,6 @@ k_bucket_build_pg(const uint32_t *__restrict__ recs_b, const unsigned long long 
     const uint32_t stride = gw_full + 1u;                          // odd: a warp's 32 rows spread over all banks
     const uint32_t win = row_cap_words / stride;
     uint32_t *grow = matrix + base * (uint64_t)wp;
-    uint32_t iter = 0;
     // the table is cleared once; every pass clears the words it stores on its way out (one barrier and one
     // sweep of the table less per column slice)
     for (uint32_t i = tid; i < min(win, D) * stride; i += NT) rows[i] = 0u;
@@ -362,12 +278,8 @@ k_bucket_build_pg(const uint32_t *__restrict__ recs_b, const unsigned long long 
                     const uint32_t row = wv.y + __popc(wv.x & ((1u << (low & 31)) - 1u)) - r0;
                     if (row < nr) atomicOr(rows + row * stride + (s8 >> 5), 1u << (s8 & 31));
                 };
-                if (TMA) {
-                    bk_for_each<NT>(blist + bp[g], npages, recs_b, ring, R, iter, place);
-                } else {
-                    bk_for_each_direct<NT>(blist + bp[g], npages, recs_b, place);
-                    __syncthreads();
-                }
+                bk_for_each_direct<NT>(blist + bp[g], npages, recs_b, place);
+                __syncthreads();
             }
             uint32_t *gdst = grow + (uint64_t)r0 * wp + 8u * g;
             for (uint32_t i = tid; i < nr * gw; i += NT) {

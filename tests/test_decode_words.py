@@ -1,8 +1,9 @@
 """The word-wide FASTA reader (phenotypeseeker_b200/csrc/ps_decode_bits.h): the write pass's word step and the count
 pass's chunk summary against a byte-at-a-time reader on the host (every line width 1..200, CRLF, TAB, lower case,
 IUPAC, NUL, bytes >= 128, '>' at every byte of a word, headers over two and three chunks, chunks that start in a
-header, every [jlo, jhi) edge and output alignment); on the GPU, the default FASTA write pass and the staged-byte
-one (PSKMER_DECODE=bytes) against the oracle on text of mixed line widths."""
+header, every [jlo, jhi) edge and output alignment); on the GPU, both FASTA write passes against the oracle on text of
+mixed line widths: the word-wide one (an all-FASTA launch) and the byte transducer's FASTA branch (the same files in
+one launch with a FASTQ sample)."""
 import os
 import subprocess
 
@@ -49,19 +50,23 @@ def _mixed_width_fasta(rng, n_bases):
     return b"".join(parts)
 
 
+def _small_fastq(rng):
+    """Two reads: a launch that holds it decodes with k_decode_write<0>, format per file."""
+    reads = ["".join(rng.choice(list("ACGT"), size=n)) for n in (150, 97)]
+    return "".join("@r%d\n%s\n+\n%s\n" % (i, r, "I" * len(r)) for i, r in enumerate(reads)).encode()
+
+
 @pytest.mark.gpu
-@pytest.mark.parametrize("decode", ["default", "bytes"])
-def test_fasta_write_passes_on_mixed_line_widths(decode, monkeypatch):
+@pytest.mark.parametrize("decode", ["default", "mixed"])
+def test_fasta_write_passes_on_mixed_line_widths(decode):
     from oracle import kmers as ok
     from phenotypeseeker_b200._native import Context
     from phenotypeseeker_b200.pipeline import unpack_rows
-    if decode == "bytes":
-        monkeypatch.setenv("PSKMER_DECODE", "bytes")
-    else:
-        monkeypatch.delenv("PSKMER_DECODE", raising=False)
     rng = np.random.default_rng(31)
     files = [_mixed_width_fasta(rng, int(n)) for n in (50, 16_000, 40_000, 120_000, 300_000)]
     files.append(b"junk before the first record\n" + files[1])
+    if decode == "mixed":
+        files.append(_small_fastq(rng))
     lists = [ok.count_kmers(f, 16) for f in files]
     u = ok.union([l[0] for l in lists])
     c = Context(0)

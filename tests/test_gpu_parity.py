@@ -130,14 +130,13 @@ def test_many_samples_wide_rows(ctx):
     assert np.array_equal(unpack_rows(ctx.get_rows(), 300), ok.presence_matrix(u, lists))
 
 
-@pytest.mark.parametrize("env", [{"PSKMER_ROWS": "sorted"}, {"PSKMER_BK_ROW_KB": "1"}, {"PSKMER_BK_TMA": "1"},
-                                 {"PSKMER_BK_TMA": "1", "PSKMER_BK_ROW_KB": "1"}, {"PSKMER_SC1": "regs", "PSKMER_DECODE": "swar"}])
+@pytest.mark.parametrize("env", [{"PSKMER_ROWS": "sorted"}, {"PSKMER_BK_ROW_KB": "1"}, {"PSKMER_SC1": "regs"}])
 @pytest.mark.parametrize("k", [9, 13, 16])
 def test_row_builders_agree(ctx, env, k, monkeypatch):
     """Every way rows are built gives the same union and matrix as the oracle: the default (paged
-    partition, bucket kernels reading their pages with 128-bit loads), the bucket kernels fed through the
-    TMA ring (PSKMER_BK_TMA=1), a 1 KB row table (every non-trivial bucket goes through the big-bucket
-    launch and several row windows), and the full sort + run detection (PSKMER_ROWS=sorted)."""
+    partition, bucket kernels reading their pages with 128-bit loads), a 1 KB row table (every non-trivial
+    bucket goes through the big-bucket launch and several row windows), the register variant of k_scatter1
+    (PSKMER_SC1=regs), and the full sort + run detection (PSKMER_ROWS=sorted)."""
     from phenotypeseeker_b200._native import Context
     rng = np.random.default_rng(5 + k)
     # low-complexity, AT-rich genomes: a few (top 16 bit) buckets hold most of the k-mers
@@ -165,12 +164,11 @@ def test_row_builders_agree(ctx, env, k, monkeypatch):
         other.close()
 
 
-def test_decoder_variant_on_goldens_and_tile_edges(golden_kmer_lists, monkeypatch):
-    """PSKMER_DECODE=swar (FASTA write pass from per-thread bit strings) and PSKMER_SC1=regs (k-mers kept in registers
-    between ranking and grouping; the default recomputes them) against the glistmaker goldens and headers / newlines /
-    invalid bytes at chunk and tile edges."""
+def test_scatter1_register_variant_on_goldens_and_tile_edges(golden_kmer_lists, monkeypatch):
+    """The register variant of k_scatter1 (PSKMER_SC1=regs: k-mers kept in registers between ranking and grouping;
+    the default recomputes them) against the glistmaker goldens and headers / newlines / invalid bytes at chunk and
+    tile edges."""
     from phenotypeseeker_b200._native import Context
-    monkeypatch.setenv("PSKMER_DECODE", "swar")
     monkeypatch.setenv("PSKMER_SC1", "regs")
     c = Context(0)
     try:
