@@ -116,11 +116,19 @@ static bool radix_sort(ps_ctx *c, KeyT *ka, KeyT *kb, uint16_t *ta, uint16_t *tb
     return in_b;
 }
 
+// exclusive scan of u32 counts -> u64 offsets (offs[n] = total), on the device
+static void scan_counts_dev(ps_ctx *c, const char *name, const uint32_t *counts, uint64_t n, unsigned long long *offs) {
+    const uint64_t chunks = std::max<uint64_t>(1, ceil_div<uint64_t>(n, SCAN_CHUNK));
+    c->scan_sums.reserve(chunks * 8, c->stream);
+    unsigned long long *sums = c->scan_sums.as<unsigned long long>();
+    KLAUNCH(c, name, (double)n * 4, (k_scan_sums<<<(unsigned)chunks, SCAN_THREADS, 0, c->stream>>>(counts, n, sums)));
+    KLAUNCH(c, name, (double)n * 12, (k_scan_chunks<<<(unsigned)chunks, SCAN_THREADS, 0, c->stream>>>(counts, n, sums, offs)));
+}
+
 // exclusive scan of u32 counts -> u64 offsets; returns total (syncs the stream)
 static uint64_t scan_counts(ps_ctx *c, const uint32_t *counts, uint64_t n, DevBuf &offs) {
     offs.reserve((n + 1) * 8, c->stream);
-    KLAUNCH(c, "scan_counts", (double)n * 12,
-            (k_scan_counts<<<1, 1024, 0, c->stream>>>(counts, n, offs.as<unsigned long long>())));
+    scan_counts_dev(c, "scan_counts", counts, n, offs.as<unsigned long long>());
     return ps_read_scalar<unsigned long long>(c, offs.as<unsigned long long>() + n);
 }
 
@@ -228,7 +236,7 @@ static inline int paged_groups(const ps_ctx *c) { return (c->n_samples + 255) / 
 struct PagedTabs {
     uint32_t *cursor_a;      // [PART_MAX]
     uint32_t *cursor_b, *overflow, *ticket, *ntiles_dummy;
-    uint32_t *scnt, *sstart, *tstart, *sfill;      // [ns], [ns + 1], [ns + 1], [ns]
+    uint32_t *scnt, *tstart, *sfill;               // [ns], [ns + 1], [ns]
     uint32_t *bpcnt, *brecs, *bpfill;              // [BK_N * G], [BK_N], [BK_N * G]
     uint8_t *bin_d2;                               // [512]
     uint32_t *trash;                               // SC_TILE
@@ -250,7 +258,6 @@ static PagedTabs paged_tabs(ps_ctx *c) {
     t.brecs = p; p += BK_N;
     t.bpfill = p; p += BK_N * G;
     t.zero_bytes = (size_t)(p - c->pg_tabs.as<uint32_t>()) * 4;
-    t.sstart = p; p += t.ns + 1;
     t.tstart = p; p += t.ns + 1;
     t.bin_d2 = reinterpret_cast<uint8_t *>(p); p += 128;
     t.trash = p;
@@ -352,43 +359,39 @@ static void paged_finish(ps_ctx *c, const Sc1Dst &dst_for_close, bool close_loca
         KLAUNCH(c, "pg_close", 0.0, (k_pg_close1<<<c->sc1_grid, 288, 0, c->stream>>>(st1, dst_for_close, lbits)));
     CK(cudaMemcpyAsync(t.bin_d2, h_bin_d2, 512, cudaMemcpyHostToDevice, c->stream));
     const uint32_t npa = c->pgA_cap;
-    c->pg_plist.reserve((size_t)npa * 4, c->stream);
-    c->pg_tiles.reserve(((size_t)npa + t.ns) * sizeof(Sc2Tile), c->stream);
-    KLAUNCH(c, "pg_lists", (double)npa * 4,
-            (k_pga_hist<<<ceil_div<uint32_t>(npa, 256), 256, 0, c->stream>>>(c->pg_meta_a.as<uint32_t>(), npa, bin_lo, bin_hi, t.scnt)));
-    KLAUNCH(c, "pg_lists", 0.0, (k_pga_scan<<<1, 1024, 0, c->stream>>>(t.scnt, t.ns, t.sstart, t.tstart, t.sfill)));
-    KLAUNCH(c, "pg_lists", (double)npa * 8,
-            (k_pga_fill<<<ceil_div<uint32_t>(npa, 256), 256, 0, c->stream>>>(c->pg_meta_a.as<uint32_t>(), npa, bin_lo, bin_hi,
-                                                                             t.sstart, t.sfill, c->pg_plist.as<uint32_t>())));
-    KLAUNCH(c, "pg_lists", (double)npa * 8,
-            (k_pga_tiles<<<ceil_div<uint32_t>(npa, 256), 256, 0, c->stream>>>(c->pg_meta_a.as<uint32_t>(), c->pg_plist.as<uint32_t>(),
-                                                                              t.sstart, t.tstart, t.ns, c->pg_tiles.as<Sc2Tile>())));
+    c->pg_tiles.reserve(((size_t)npa / SC_TILE_PAGES + t.ns + 1) * sizeof(Sc2Tile), c->stream);
+    KLAUNCH(c, "pga_hist", (double)npa * 4,
+            (k_pga_pages<false><<<ceil_div<uint32_t>(npa, PGL_THREADS * PGL_PER), PGL_THREADS, 0, c->stream>>>(
+                c->pg_meta_a.as<uint32_t>(), npa, bin_lo, bin_hi, t.scnt, t.tstart, t.sfill, c->pg_tiles.as<Sc2Tile>())));
+    KLAUNCH(c, "pga_scan", (double)t.ns * 12, (k_pga_scan<<<1, 1024, 0, c->stream>>>(t.scnt, t.ns, t.tstart, t.sfill)));
+    KLAUNCH(c, "pga_fill", (double)npa * 4,
+            (k_pga_pages<true><<<ceil_div<uint32_t>(npa, PGL_THREADS * PGL_PER), PGL_THREADS, 0, c->stream>>>(
+                c->pg_meta_a.as<uint32_t>(), npa, bin_lo, bin_hi, t.scnt, t.tstart, t.sfill, c->pg_tiles.as<Sc2Tile>())));
     // level-2 pool: every record once + the pages a block leaves half full when it moves to another stream
     const uint64_t capb = ceil_div<uint64_t>(n_upper, PG_B) + ((uint64_t)paged_groups(c) * SC_BINS1 + 2 * c->sc2_grid) * 256;   // open + spare pages
     if (capb >= (1ull << 31)) PS_THROW(PS_ERR_NOMEM, "level-2 page pool of %llu pages: cut the job into k-mer ranges", (unsigned long long)capb);
     c->keys_b.reserve(capb * PG_B * 4, c->stream);
     c->pg_meta_b.reserve(capb * 8, c->stream);
     c->pgB_cap = (uint32_t)capb;
+    const uint32_t G = (uint32_t)paged_groups(c);
     Sc2Args a;
-    a.recs_a = c->keys_a.as<uint32_t>(); a.meta_a = c->pg_meta_a.as<uint32_t>();
-    a.plist = c->pg_plist.as<uint32_t>(); a.tiles = c->pg_tiles.as<Sc2Tile>();
+    a.recs_a = c->keys_a.as<uint32_t>();
+    a.tiles = c->pg_tiles.as<Sc2Tile>();
     a.ntiles = t.tstart + t.ns; a.bin_d2 = t.bin_d2;
     a.recs_b = c->keys_b.as<uint32_t>(); a.meta_b = c->pg_meta_b.as<unsigned long long>();
     a.cap_b = c->pgB_cap; a.cursor_b = t.cursor_b; a.overflow = t.overflow; a.trash = t.trash;
-    KLAUNCH(c, "scatter2", (double)n_upper * 8,
-            (k_scatter2<<<c->sc2_grid, SC_THREADS, SC2_SMEM, c->stream>>>(a, st2)));
-    KLAUNCH(c, "pg_close", 0.0, (k_pg_close2<<<c->sc2_grid, 288, 0, c->stream>>>(st2, t.bin_d2, a.meta_b)));
+    a.bpcnt = t.bpcnt; a.brecs = t.brecs; a.G = G;
+    KLAUNCH(c, "scatter2", (double)n_upper * 8, (k_scatter2<<<c->sc2_grid, SC_THREADS, SC2_SMEM, c->stream>>>(a, st2)));
+    KLAUNCH(c, "pg_close", 0.0, (k_pg_close2<<<c->sc2_grid, 288, 0, c->stream>>>(st2, t.bin_d2, a.meta_b, t.bpcnt, t.brecs, G)));
     // bucket page lists
     const BucketTables bt = bucket_tables(c);
     CK(cudaMemsetAsync(bt.fill, 0, 16, c->stream));
     const int lg = PS_SMS * 8;
-    const uint32_t G = (uint32_t)paged_groups(c);
-    KLAUNCH(c, "pgb_lists", 0.0, (k_pgb_hist<<<lg, 256, 0, c->stream>>>(a.meta_b, t.cursor_b, c->pgB_cap, G, t.bpcnt, t.brecs)));
-    KLAUNCH(c, "scan_counts", (double)BK_N * G * 12, (k_scan_counts<<<1, 1024, 0, c->stream>>>(t.bpcnt, (uint64_t)BK_N * G, bt.bstart)));
+    scan_counts_dev(c, "scan_bpages", t.bpcnt, (uint64_t)BK_N * G, bt.bstart);
     c->pg_blist.reserve((size_t)capb * 8, c->stream);
-    KLAUNCH(c, "pgb_lists", 0.0, (k_pgb_fill<<<lg, 256, 0, c->stream>>>(a.meta_b, t.cursor_b, c->pgB_cap, G, bt.bstart, t.bpfill,
-                                                                       c->pg_blist.as<unsigned long long>())));
-    KLAUNCH(c, "pg_lists", 0.0, (k_bucket_order_pg<<<BK_N / 256, 256, 0, c->stream>>>(
+    KLAUNCH(c, "pgb_fill", (double)capb * 8, (k_pgb_fill<<<lg, 256, 0, c->stream>>>(a.meta_b, t.cursor_b, c->pgB_cap, G, bt.bstart, t.bpfill,
+                                                                                c->pg_blist.as<unsigned long long>())));
+    KLAUNCH(c, "bucket_order", (double)BK_N * 8, (k_bucket_order_pg<<<BK_N / 256, 256, 0, c->stream>>>(
                                      t.brecs, (uint32_t)std::min<uint64_t>(4 * (n_upper / BK_N) + 4096, 0xFFFFFFFFu), bt.fill, bt.order)));
     const int nwords = lbits >= 5 ? (1 << (lbits - 5)) : 1;
     c->tmp1.reserve((size_t)BK_N * nwords * 4, c->stream);
@@ -396,11 +399,11 @@ static void paged_finish(ps_ctx *c, const Sc1Dst &dst_for_close, bool close_loca
     KLAUNCH(c, "bucket_count", (double)n_upper * 4,
             (k_bucket_count_pg<<<BK_N, BK_THREADS, 0, c->stream>>>(
                 a.recs_b, c->pg_blist.as<unsigned long long>(), bt.bstart, G, bt.order, lbits, bt.counts, gbm)));
-    KLAUNCH(c, "scan_counts", (double)BK_N * 12, (k_scan_counts<<<1, 1024, 0, c->stream>>>(bt.counts, BK_N, bt.first_row)));
+    scan_counts_dev(c, "scan_rows", bt.counts, BK_N, bt.first_row);
     const uint32_t stride = (uint32_t)std::min(c->row_words, 8) + 1;      // rows are assembled in 8-word column slices
     const uint32_t cap_small = (uint32_t)std::max(c->bk_row_words, round_up<int>((int)stride, 4));
     const uint32_t cap_big = (uint32_t)std::max<int>((BK_MAX_DYN_SMEM - nwords * 8) / 4 & ~3, (int)cap_small);
-    KLAUNCH(c, "pg_lists", 0.0,
+    KLAUNCH(c, "bucket_order", (double)BK_N * 8,
             (k_bucket_order_pg<<<BK_N / 256, 256, 0, c->stream>>>(bt.counts, cap_small / stride, bt.fill + 2, bt.order2)));
     unsigned long long *h = (unsigned long long *)ps_pinned(c, 64);
     uint32_t *h32 = reinterpret_cast<uint32_t *>(h + 1);

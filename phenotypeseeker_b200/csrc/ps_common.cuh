@@ -127,7 +127,7 @@ struct ps_ctx {
     bool chi2_sparse_force = false;   // PSKMER_CHI2=walk: the bit-walk kernel for every unweighted shape it can take (tests)
 
     // paged partition (ps_paged.cuh): level-1 pool = keys_a, level-2 pool = keys_b
-    int sc1_grid = 2 * PS_SMS, sc2_grid = 2 * PS_SMS;
+    int sc1_grid = 2 * PS_SMS, sc2_grid = 3 * PS_SMS;   // sc2_grid: k_scatter2 runs three blocks per SM (SC2_BLOCKS_PER_SM)
     uint32_t pgA_cap = 0, pgB_cap = 0;   // pages
     double sc1_out_frac = 1.0;  // share of the positions whose record k_scatter1 writes (range-restricted runs): profile accounting only
     uint64_t cap_hint = 0;      // ps_set_capacity_hint: expected k-mer instances of the next build (0 = from input size)
@@ -157,14 +157,14 @@ struct ps_ctx {
     DevBuf pool_seq, pool_bad;                              // 2-bit streams
     DevBuf list_keys, list_counts;                          // per-sample counted lists
     DevBuf samp_tab;                                        // per-sample table on device
-    DevBuf blk_counts, blk_offs, scalars;                   // scans
+    DevBuf blk_counts, blk_offs, scalars, scan_sums;        // scans
     DevBuf keys_a, keys_b, tags_a, tags_b, hist, lookback;  // sort
     DevBuf uni, matrix;                                     // union + matrix
     DevBuf ph_masks, ph_vals, ph_tot, weights;              // phenotypes
     DevBuf sv_ph, sv_row, sv_stat, sv_p, sv_mx, sv_my, sv_n, sv_perm, sv_bits, sv_kmer;
     DevBuf sel_ph, sel_row, sel_stat, sel_p, sel_mx, sel_my, sel_n;   // ps_select_top
     DevBuf tmp1, tmp2, tmp3;
-    DevBuf pg_meta_a, pg_meta_b, pg_plist, pg_tiles, pg_tabs, pg_state, pg_blist;   // paged partition
+    DevBuf pg_meta_a, pg_meta_b, pg_tiles, pg_tabs, pg_state, pg_blist;   // paged partition
     DevBuf mash_tab, mash_parts, mash_parts_n, mash_h, mash_n, mash_sd;              // ps_mash_sketch / ps_mash_pairs
     DevBuf nj_d, nj_d2, nj_act, nj_nd, nj_part, nj_out;                              // ps_neighbor_joining
     DevBuf cm_q, cm_idx, cm_filter, cm_tab, cm_inv, cm_cnt, cm_out;                   // ps_count_matrix
@@ -179,10 +179,10 @@ struct ps_ctx {
 
     std::vector<DevBuf *> all_bufs() {
         return {&staging, &tile_tab, &tile_sum, &file_tab, &pool_seq, &pool_bad, &list_keys,
-                &list_counts, &samp_tab, &blk_counts, &blk_offs, &scalars, &keys_a, &keys_b,
+                &list_counts, &samp_tab, &blk_counts, &blk_offs, &scalars, &scan_sums, &keys_a, &keys_b,
                 &tags_a, &tags_b, &hist, &lookback, &uni, &matrix, &ph_masks, &ph_vals, &ph_tot,
                 &weights, &sv_ph, &sv_row, &sv_stat, &sv_p, &sv_mx, &sv_my, &sv_n, &sv_perm,
-                &sv_bits, &sv_kmer, &tmp1, &tmp2, &tmp3, &pg_meta_a, &pg_meta_b, &pg_plist, &pg_tiles,
+                &sv_bits, &sv_kmer, &tmp1, &tmp2, &tmp3, &pg_meta_a, &pg_meta_b, &pg_tiles,
                 &pg_tabs, &pg_state, &pg_blist, &sel_ph, &sel_row, &sel_stat, &sel_p, &sel_mx, &sel_my, &sel_n,
                 &mash_tab, &mash_parts, &mash_parts_n, &mash_h, &mash_n, &mash_sd, &nj_d, &nj_d2, &nj_act, &nj_nd,
                 &nj_part, &nj_out, &cm_q, &cm_idx, &cm_filter, &cm_tab, &cm_inv, &cm_cnt, &cm_out};

@@ -23,12 +23,13 @@
 //               Records are 4 bytes for any number of samples: d1 << 24 | low << 8 | (sample & 255);
 //               the sample GROUP (sample >> 8) is a property of the page (a block closes its open
 //               pages when the group of its tiles changes).
-//   k_pg_*      tiny kernels: pages -> per-stream page lists -> tiles of up to 8 pages.
+//   k_pga_*     tiny kernels: pages -> tiles of up to 8 pages of one stream (page ids and counts
+//               in the tile descriptor).
 //   k_scatter2  level-2 partition of every stream (group, bin) by d1 into pages of 512 records
 //               tagged (bucket = d2 << 8 | d1, group). Input pages come in through the TMA unit
-//               (cp.async.bulk global -> shared, mbarrier completion, double-buffered), so the load
-//               of tile t+1 overlaps ranking / scatter / write-out of tile t.
-//   k_pg_*      pages -> per-bucket page lists (+ record counts for largest-first scheduling).
+//               (cp.async.bulk global -> shared, mbarrier completion); closing a page also counts
+//               it for its bucket's page list.
+//   k_pgb_fill  pages -> per-bucket page lists (+ record counts for largest-first scheduling).
 //
 // The order of records inside a bucket is arbitrary (and varies from run to run); the bucket
 // kernels OR presence bits, so union and matrix are deterministic.
@@ -480,94 +481,119 @@ __global__ void k_pg_reset_state(ScState *__restrict__ state) {
 }
 
 // ---- level-1 pages -> stream page lists -> level-2 tiles ---------------------------------------------
-// scnt[key]++ for every used page
-// Only pages of level-1 bins [bin_lo, bin_hi) are listed: a build may cover a sub-range of the k-mer range
-// the pool was scattered for (bins ascend with the k-mer), see ps_scatter_range.
-__global__ void k_pga_hist(const uint32_t *__restrict__ meta, uint32_t npages, uint32_t bin_lo, uint32_t bin_hi,
-                           uint32_t *__restrict__ scnt) {
-    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= npages) return;
-    const uint32_t m = meta[p];
-    if (!m) return;
-    const uint32_t bin = PGA_KEY(m) & 511u;
-    if (bin >= bin_lo && bin < bin_hi) atomicAdd(&scnt[PGA_KEY(m)], 1u);
-}
-
-// Single block: exclusive scans of the page counts (-> sstart) and of the tile counts ceil(cnt / 8)
-// (-> tstart); both arrays get ns + 1 entries. sfill is zeroed.
+// Single block: exclusive scan of the tile counts ceil(scnt / 8) (-> tstart, ns + 1 entries; tstart[ns] = tiles).
+// sfill is zeroed.
 __global__ void __launch_bounds__(1024)
-k_pga_scan(const uint32_t *__restrict__ scnt, uint32_t ns, uint32_t *__restrict__ sstart,
-           uint32_t *__restrict__ tstart, uint32_t *__restrict__ sfill) {
-    __shared__ uint32_t wsA[32], wsB[32];
-    __shared__ uint32_t carryA, carryB;
+k_pga_scan(const uint32_t *__restrict__ scnt, uint32_t ns, uint32_t *__restrict__ tstart,
+           uint32_t *__restrict__ sfill) {
+    __shared__ uint32_t ws[32];
+    __shared__ uint32_t carry;
     const unsigned tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    if (tid == 0) { carryA = 0; carryB = 0; }
+    if (tid == 0) carry = 0;
     __syncthreads();
     for (uint32_t base = 0; base < ns; base += 1024) {
         const uint32_t i = base + tid;
-        const uint32_t a = i < ns ? scnt[i] : 0u, b = (a + SC_TILE_PAGES - 1) / SC_TILE_PAGES;
-        uint32_t ia = a, ib = b;
+        const uint32_t b = i < ns ? (scnt[i] + SC_TILE_PAGES - 1) / SC_TILE_PAGES : 0u;
+        uint32_t ib = b;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t ta = __shfl_up_sync(0xffffffffu, ia, o), tbv = __shfl_up_sync(0xffffffffu, ib, o);
-            if (lane >= (unsigned)o) { ia += ta; ib += tbv; }
+            const uint32_t t = __shfl_up_sync(0xffffffffu, ib, o);
+            if (lane >= (unsigned)o) ib += t;
         }
-        if (lane == 31) { wsA[warp] = ia; wsB[warp] = ib; }
+        if (lane == 31) ws[warp] = ib;
         __syncthreads();
         if (warp == 0) {
-            const uint32_t wa = wsA[lane], wb = wsB[lane];
-            uint32_t xa = wa, xb = wb;
+            const uint32_t w = ws[lane];
+            uint32_t x = w;
 #pragma unroll
             for (int o = 1; o < 32; o <<= 1) {
-                const uint32_t ta = __shfl_up_sync(0xffffffffu, xa, o), tbv = __shfl_up_sync(0xffffffffu, xb, o);
-                if (lane >= (unsigned)o) { xa += ta; xb += tbv; }
+                const uint32_t t = __shfl_up_sync(0xffffffffu, x, o);
+                if (lane >= (unsigned)o) x += t;
             }
-            wsA[lane] = xa - wa; wsB[lane] = xb - wb;
+            ws[lane] = x - w;
         }
         __syncthreads();
-        const uint32_t ea = carryA + wsA[warp] + ia - a, eb = carryB + wsB[warp] + ib - b;
-        if (i < ns) { sstart[i] = ea; tstart[i] = eb; sfill[i] = 0; }
+        const uint32_t e = carry + ws[warp] + ib - b;
+        if (i < ns) { tstart[i] = e; sfill[i] = 0; }
         __syncthreads();
-        if (tid == 1023) { carryA = ea + a; carryB = eb + b; }
+        if (tid == 1023) carry = e + b;
         __syncthreads();
     }
-    if (tid == 0) { sstart[ns] = carryA; tstart[ns] = carryB; }
+    if (tid == 0) tstart[ns] = carry;
 }
 
-// plist[sstart[key] + j] = page (any order inside a stream)
-__global__ void k_pga_fill(const uint32_t *__restrict__ meta, uint32_t npages, uint32_t bin_lo, uint32_t bin_hi,
-                           const uint32_t *__restrict__ sstart, uint32_t *__restrict__ sfill, uint32_t *__restrict__ plist) {
-    const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= npages) return;
-    const uint32_t m = meta[p];
-    if (!m) return;
-    const uint32_t key = PGA_KEY(m);
-    if ((key & 511u) < bin_lo || (key & 511u) >= bin_hi) return;
-    plist[sstart[key] + atomicAdd(&sfill[key], 1u)] = p;
-}
+// One level-2 tile: up to SC_TILE_PAGES level-1 pages of one stream, with their record counts, so that k_scatter2
+// starts the copies of a tile after a single load.
+struct __align__(16) Sc2Tile {
+    uint32_t key, np;                    // stream key (group << 9 | bin), pages in the tile
+    uint32_t page[SC_TILE_PAGES];
+    uint16_t cnt[SC_TILE_PAGES];
+    uint32_t pad[2];
+};
 
-// One entry per level-2 tile: first slot in plist | pages << 28 (1..8), and the stream key.
-struct Sc2Tile { uint32_t slot_np; uint32_t key; };
-__global__ void k_pga_tiles(const uint32_t *__restrict__ meta, const uint32_t *__restrict__ plist,
-                            const uint32_t *__restrict__ sstart, const uint32_t *__restrict__ tstart, uint32_t ns,
-                            Sc2Tile *__restrict__ tiles) {
-    const uint32_t slot = blockIdx.x * blockDim.x + threadIdx.x;
-    if (slot >= sstart[ns]) return;
-    const uint32_t key = PGA_KEY(meta[plist[slot]]);
-    const uint32_t j = slot - sstart[key];
-    if (j % SC_TILE_PAGES) return;
-    const uint32_t np = min((uint32_t)SC_TILE_PAGES, sstart[key + 1] - slot);
-    Sc2Tile t;
-    t.slot_np = slot | (np << 28);
-    t.key = key;
-    tiles[tstart[key] + j / SC_TILE_PAGES] = t;
+// Page counts per stream (FILL = false: scnt[key] += pages) and tiles (FILL = true: page p, the j-th page of its
+// stream in any order, goes to slot j % 8 of the stream's tile j / 8). A block takes PGL_THREADS x PGL_PER consecutive
+// pages and adds them up per stream key in shared memory first (slot = key mod PGL_SLOTS; a page whose slot another
+// key already holds goes to global memory on its own): one global atomicAdd per key and block instead of one per page.
+// Consecutive pages were taken at about the same time, so they belong to a few dozen keys; the keys of a range
+// share a few cache lines of scnt / sfill, and single atomics on them serialise (1 ms per launch on config 5).
+// Only pages of level-1 bins [bin_lo, bin_hi) are listed: a build may cover a sub-range of the k-mer range
+// the pool was scattered for (bins ascend with the k-mer), see ps_scatter_range.
+#define PGL_THREADS 256
+#define PGL_PER 8
+#define PGL_SLOTS 2048
+template <bool FILL>
+__global__ void __launch_bounds__(PGL_THREADS)
+k_pga_pages(const uint32_t *__restrict__ meta, uint32_t npages, uint32_t bin_lo, uint32_t bin_hi,
+            uint32_t *__restrict__ scnt, const uint32_t *__restrict__ tstart, uint32_t *__restrict__ sfill,
+            Sc2Tile *__restrict__ tiles) {
+    __shared__ uint32_t s_tag[PGL_SLOTS], s_cnt[PGL_SLOTS];
+    const unsigned tid = threadIdx.x;
+    for (uint32_t i = tid; i < PGL_SLOTS; i += PGL_THREADS) { s_tag[i] = PG_NONE; s_cnt[i] = 0; }
+    __syncthreads();
+    const uint32_t p0 = blockIdx.x * (PGL_THREADS * PGL_PER) + tid;
+    uint32_t m[PGL_PER], rank[PGL_PER];                // rank inside the block's pages of the key; PG_NONE: on its own
+#pragma unroll
+    for (int j = 0; j < PGL_PER; j++) {
+        const uint32_t p = p0 + j * PGL_THREADS;
+        m[j] = p < npages ? meta[p] : 0u;
+        const uint32_t key = PGA_KEY(m[j]);
+        if (!m[j] || (key & 511u) < bin_lo || (key & 511u) >= bin_hi) { m[j] = 0; continue; }
+        const uint32_t slot = key & (PGL_SLOTS - 1);
+        uint32_t tag = s_tag[slot];
+        if (tag == PG_NONE) {
+            tag = atomicCAS(&s_tag[slot], PG_NONE, key);
+            if (tag == PG_NONE) tag = key;
+        }
+        rank[j] = tag == key ? atomicAdd(&s_cnt[slot], 1u) : PG_NONE;
+        if (!FILL && rank[j] == PG_NONE) atomicAdd(&scnt[key], 1u);
+    }
+    __syncthreads();
+    // one global atomicAdd per key; FILL: s_cnt[slot] becomes the index of the slot's first page in its stream
+    for (uint32_t i = tid; i < PGL_SLOTS; i += PGL_THREADS) {
+        const uint32_t c = s_cnt[i];
+        if (!c) continue;
+        const uint32_t b = atomicAdd(FILL ? &sfill[s_tag[i]] : &scnt[s_tag[i]], c);
+        if (FILL) s_cnt[i] = b;
+    }
+    if (!FILL) return;
+    __syncthreads();
+#pragma unroll
+    for (int j = 0; j < PGL_PER; j++) {
+        if (!m[j]) continue;
+        const uint32_t key = PGA_KEY(m[j]);
+        const uint32_t idx = rank[j] == PG_NONE ? atomicAdd(&sfill[key], 1u) : s_cnt[key & (PGL_SLOTS - 1)] + rank[j];
+        const uint32_t q = idx % SC_TILE_PAGES;
+        Sc2Tile &t = tiles[tstart[key] + idx / SC_TILE_PAGES];
+        t.page[q] = p0 + j * PGL_THREADS;
+        t.cnt[q] = (uint16_t)PGA_CNT(m[j]);
+        if (q == 0) { t.key = key; t.np = min((uint32_t)SC_TILE_PAGES, scnt[key] - idx); }
+    }
 }
 
 // ---- level 2: pages of one stream -> pages of its 256 buckets ----------------------------------------
 struct Sc2Args {
     const uint32_t *recs_a;              // level-1 pool (this GPU's own)
-    const uint32_t *meta_a;
-    const uint32_t *plist;
     const Sc2Tile *tiles;
     const uint32_t *ntiles;              // device scalar: tstart[ns]
     const uint8_t *bin_d2;               // [SC_BINS1] bin -> d2 for the bins this GPU owns
@@ -577,22 +603,38 @@ struct Sc2Args {
     uint32_t *cursor_b;
     uint32_t *overflow;
     uint32_t *trash;
+    uint32_t *bpcnt, *brecs;             // [BK_N * G] pages per (bucket, group), [BK_N] records per bucket
+    uint32_t G;
 };
 
-#define SC2_SMEM (3 * SC_TILE * 4 + sizeof(ScShared<256>) + 64)
+// Closes level-2 page `page` (n records of bucket, group) and counts it for the bucket page lists.
+__device__ __forceinline__ void pgb_close(unsigned long long *meta_b, uint32_t *bpcnt, uint32_t *brecs, uint32_t G,
+                                          uint32_t page, uint32_t bucket, uint32_t grp, uint32_t n) {
+    meta_b[page] = PGB_META(bucket, grp, n);
+    atomicAdd(&bpcnt[bucket * G + grp], 1u);
+    atomicAdd(&brecs[bucket], n);
+}
 
-__global__ void __launch_bounds__(SC_THREADS, 2)
+// 8192-record tiles through ONE landing zone, three blocks per SM (40 registers). Phase A only counts the bins,
+// phase C reads each record from the landing zone again and takes its slot with an atomicAdd on the bin's base; the
+// copy of tile t + 1 starts once phase C has read the zone, and the other blocks on the SM cover the wait.
+// (Two landing zones of 4096 records at four blocks per SM, ranks kept in registers: 124 vs 81 ms on config 5.)
+#define SC2_BLOCKS_PER_SM 3
+#define SC2_SMEM (2 * SC_TILE * 4 + sizeof(ScShared<256>))
+
+__global__ void __launch_bounds__(SC_THREADS, SC2_BLOCKS_PER_SM)
 k_scatter2(Sc2Args a, ScState *__restrict__ state) {
     constexpr int NB = 256;
     extern __shared__ __align__(128) uint8_t sc2_dyn[];
-    uint32_t *sin0 = reinterpret_cast<uint32_t *>(sc2_dyn);                     // 2 x SC_TILE records (TMA landing zones)
-    uint32_t *sk = sin0 + 2 * SC_TILE;                                          // SC_TILE records
-    ScShared<NB> &S = *reinterpret_cast<ScShared<NB> *>(sc2_dyn + 3 * SC_TILE * 4);
-    __shared__ __align__(8) uint64_t bar[2];
-    __shared__ uint32_t s_pcnt[2][SC_TILE_PAGES];
-    __shared__ uint32_t s_key[2];
+    uint32_t *sin = reinterpret_cast<uint32_t *>(sc2_dyn);                      // SC_TILE records (TMA landing zone)
+    uint32_t *sk = sin + SC_TILE;                                               // SC_TILE records
+    ScShared<NB> &S = *reinterpret_cast<ScShared<NB> *>(sc2_dyn + 2 * SC_TILE * 4);
+    __shared__ __align__(8) uint64_t bar;
+    __shared__ uint32_t s_pcnt[SC_TILE_PAGES];
+    __shared__ uint32_t s_key;
     __shared__ uint32_t s_cur_key;
-    const unsigned tid = threadIdx.x;
+    __shared__ Sc2Tile s_next;                                      // descriptor of the next tile to copy in
+    const unsigned tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     ScState &st = state[blockIdx.x];
     const uint32_t T = *a.ntiles;
     const uint32_t t_lo = (uint32_t)((uint64_t)T * blockIdx.x / gridDim.x), t_hi = (uint32_t)((uint64_t)T * (blockIdx.x + 1) / gridDim.x);
@@ -600,86 +642,91 @@ k_scatter2(Sc2Args a, ScState *__restrict__ state) {
     if (tid < NB) { my_pg = st.page[tid]; my_fill = st.fill[tid]; my_spare = st.spare[tid]; S.cnt[0][tid] = 0; S.cnt[1][tid] = 0; }
     if (tid == 0) {
         s_cur_key = st.key;
-        mbar_init(&bar[0], 1);
-        mbar_init(&bar[1], 1);
+        mbar_init(&bar, 1);
         mbar_fence_init();
     }
     __syncthreads();
-    // one thread feeds the TMA unit: up to 8 page copies per tile, one mbarrier per landing zone
-    auto issue = [&](uint32_t t, int b) {
-        const Sc2Tile tl = a.tiles[t];
-        const uint32_t slot = tl.slot_np & 0x0FFFFFFFu, np = tl.slot_np >> 28;
-        uint32_t bytes = 0;
-        uint32_t pc[SC_TILE_PAGES], pgid[SC_TILE_PAGES];
-#pragma unroll
-        for (int j = 0; j < SC_TILE_PAGES; j++) {
-            pc[j] = 0;
-            if ((uint32_t)j < np) { pgid[j] = a.plist[slot + j]; pc[j] = PGA_CNT(a.meta_a[pgid[j]]); }
-            s_pcnt[b][j] = pc[j];
-            bytes += (pc[j] * 4 + 15) & ~15u;
-        }
-        s_key[b] = tl.key;
-        mbar_expect_tx(&bar[b], bytes);
-#pragma unroll
-        for (int j = 0; j < SC_TILE_PAGES; j++)
-            if (pc[j]) bulk_g2s(sin0 + b * SC_TILE + j * PG_A, a.recs_a + (size_t)pgid[j] * PG_A, (pc[j] * 4 + 15) & ~15u, &bar[b]);
+    // Warp 0 feeds the TMA unit. The descriptor of the next tile comes into shared memory by cp.async a whole tile
+    // ahead, so that no load waits when the copies start; lane j < SC_TILE_PAGES copies page j.
+    auto fetch = [&](uint32_t t) {
+        if (lane < sizeof(Sc2Tile) / 16 && t < t_hi)
+            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(reinterpret_cast<uint4 *>(&s_next) + lane)),
+                         "l"(reinterpret_cast<const uint4 *>(a.tiles + t) + lane) : "memory");
+        asm volatile("cp.async.commit_group;" ::: "memory");
     };
-    if (tid == 0 && t_lo < t_hi) issue(t_lo, 0);
-    uint32_t phase = 0;                                            // bit b = parity to wait for on landing zone b
+    auto issue = [&]() {
+        asm volatile("cp.async.wait_all;" ::: "memory");
+        __syncwarp();
+        const uint32_t c = lane < SC_TILE_PAGES && lane < s_next.np ? (uint32_t)s_next.cnt[lane] : 0u;
+        const uint32_t bytes = (c * 4 + 15) & ~15u;
+        const uint32_t total = __reduce_add_sync(0xffffffffu, bytes);
+        if (lane < SC_TILE_PAGES) s_pcnt[lane] = c;
+        if (lane == 0) { s_key = s_next.key; mbar_expect_tx(&bar, total); }
+        __syncwarp();
+        if (bytes) bulk_g2s(sin + lane * PG_A, a.recs_a + (size_t)s_next.page[lane] * PG_A, bytes, &bar);
+        __syncwarp();                                               // s_next has been read: the next fetch may land
+    };
+    if (warp == 0 && t_lo < t_hi) {
+        fetch(t_lo);
+        issue();
+    }
+    uint32_t phase = 0;                                            // parity to wait for on the landing zone
     int buf = 0;
     for (uint32_t t = t_lo; t < t_hi; t++, buf ^= 1) {
         uint32_t *cnt = S.cnt[buf], *cnt_next = S.cnt[buf ^ 1];
-        if (tid == 0 && t + 1 < t_hi) issue(t + 1, buf ^ 1);      // zone buf^1 was released by the barrier that ended tile t-1
-        mbar_wait(&bar[buf], (phase >> buf) & 1u);
-        phase ^= 1u << buf;
-        const uint32_t *sin = sin0 + buf * SC_TILE;
-        // ---- A: rank every record inside its bin (one shared-memory atomic per record) ----
-        uint32_t rec[SC_ITEMS];
-        uint32_t rk[SC_ITEMS / 2];
-        uint32_t vmask = 0;
+        mbar_wait(&bar, phase);
+        phase ^= 1u;
+        if (warp == 0) fetch(t + 1);
+        // ---- A: count the records of every bin (one shared-memory atomic per record) ----
 #pragma unroll
         for (int it = 0; it < SC_ITEMS; it++) {
             const uint32_t i = it * SC_THREADS + tid;
-            const bool ok = (i & (PG_A - 1)) < s_pcnt[buf][i >> PG_A_LOG];
-            rec[it] = sin[i];
-            vmask |= (ok ? 1u : 0u) << it;
-            const uint32_t rnk = ok ? atomicAdd(&cnt[rec[it] >> 24], 1u) : 0u;
-            if (it & 1) rk[it >> 1] |= rnk << 16; else rk[it >> 1] = rnk;
+            if ((i & (PG_A - 1)) < s_pcnt[i >> PG_A_LOG]) atomicAdd(&cnt[sin[i] >> 24], 1u);
         }
         __syncthreads();
-        // ---- B ----
+        // ---- B: bins -> tile-local bases, page bookkeeping ----
         const uint32_t c = tid < NB ? cnt[tid] : 0u;
         const uint32_t tb = sc_bin_scan<NB>(c, S.wsum);
-        const uint32_t key = s_key[buf];
+        const uint32_t key = s_key;
         if (tid < NB) {
             cnt[tid] = tb;
             if (tid == NB - 1) cnt[NB] = tb + c;
             cnt_next[tid] = 0;
             const uint32_t ckey = s_cur_key;
             if (key != ckey && my_pg != PG_NONE) {                 // the block moved on to another stream
-                if (my_fill) a.meta_b[my_pg] = PGB_META(((uint32_t)a.bin_d2[ckey & 511u] << 8) | tid, ckey >> 9, my_fill);
+                if (my_fill) pgb_close(a.meta_b, a.bpcnt, a.brecs, a.G, my_pg, ((uint32_t)a.bin_d2[ckey & 511u] << 8) | tid, ckey >> 9, my_fill);
                 my_pg = PG_NONE; my_fill = 0;
             }
             if (c) {
                 const uint32_t bucket = ((uint32_t)a.bin_d2[key & 511u] << 8) | tid, grp = key >> 9;
                 unsigned long long *meta = a.meta_b;
+                uint32_t nfull = 0;                                // pages sc_place_run closes are full
                 sc_place_run<PG_B>(c, tb, my_pg, my_fill, my_spare, a.recs_b, 0u, a.cap_b, a.cursor_b, a.overflow, a.trash,
                                    S.split[tid], S.pab[tid][0], S.pab[tid][1],
-                                   [meta, bucket, grp](uint32_t page, uint32_t n) { meta[page] = PGB_META(bucket, grp, n); });
+                                   [meta, bucket, grp, &nfull](uint32_t page, uint32_t n) { meta[page] = PGB_META(bucket, grp, n); nfull++; });
+                if (nfull) {
+                    atomicAdd(&a.bpcnt[bucket * a.G + grp], nfull);
+                    atomicAdd(&a.brecs[bucket], nfull * PG_B);
+                }
             }
         }
         __syncthreads();
         if (tid == 0) s_cur_key = key;
-        // ---- C ----
+        // ---- C: group the records in shared memory ----
+        // cnt[bin] holds the bin's base and moves up with every record placed (the order inside a bin is free). The
+        // volatile reads make this a second read of shared memory, not phase A's values kept in (spilled) registers.
 #pragma unroll
         for (int it = 0; it < SC_ITEMS; it++) {
-            if ((vmask >> it) & 1u) {
-                const uint32_t pos = cnt[rec[it] >> 24] + ((it & 1) ? (rk[it >> 1] >> 16) : (rk[it >> 1] & 0xFFFFu));
-                sk[pos] = rec[it];                                  // the top byte (bin) is dropped on the way out
+            const uint32_t i = it * SC_THREADS + tid;
+            if ((i & (PG_A - 1)) < reinterpret_cast<const volatile uint32_t *>(s_pcnt)[i >> PG_A_LOG]) {
+                const uint32_t r = reinterpret_cast<const volatile uint32_t *>(sin)[i];
+                sk[atomicAdd(&cnt[r >> 24], 1u)] = r;               // the top byte (bin) is dropped on the way out
             }
         }
         __syncthreads();
-        // ---- D ----
+        // the landing zone has been read: the next tile comes in during the write-out
+        if (warp == 0 && t + 1 < t_hi) issue();
+        // ---- D: runs -> pages ----
         sc_write_flat<NB>(sk, cnt[NB], S.split, S.pab, [](uint32_t v, uint32_t) { return v >> 24; },
                           [](uint32_t v) { return v & 0x00FFFFFFu; });
         __syncthreads();
@@ -689,7 +736,8 @@ k_scatter2(Sc2Args a, ScState *__restrict__ state) {
 }
 
 __global__ void k_pg_close2(ScState *__restrict__ state, const uint8_t *__restrict__ bin_d2,
-                            unsigned long long *__restrict__ meta_b) {
+                            unsigned long long *__restrict__ meta_b, uint32_t *__restrict__ bpcnt,
+                            uint32_t *__restrict__ brecs, uint32_t G) {
     const unsigned tid = threadIdx.x;
     ScState &st = state[blockIdx.x];
     const uint32_t key = st.key;
@@ -697,7 +745,7 @@ __global__ void k_pg_close2(ScState *__restrict__ state, const uint8_t *__restri
     if (tid < 256) {
         const uint32_t pg = st.page[tid], fill = st.fill[tid];
         if (pg != PG_NONE && fill)
-            meta_b[pg] = PGB_META(((uint32_t)bin_d2[key & 511u] << 8) | tid, key >> 9, fill);
+            pgb_close(meta_b, bpcnt, brecs, G, pg, ((uint32_t)bin_d2[key & 511u] << 8) | tid, key >> 9, fill);
         const uint32_t sp = st.spare[tid];
         if (sp != PG_NONE) meta_b[sp] = 0ull;                  // taken ahead of need, never used: no stale meta
     }
@@ -707,19 +755,8 @@ __global__ void k_pg_close2(ScState *__restrict__ state, const uint8_t *__restri
 
 // ---- level-2 pages -> bucket page lists ---------------------------------------------------------------
 // Pages are listed per (bucket, sample group): key = bucket * G + group, so a bucket's pages are contiguous
-// and ordered by group. bpcnt[key] = pages, brecs[bucket] = records.
-__global__ void k_pgb_hist(const unsigned long long *__restrict__ meta, const uint32_t *__restrict__ npages_dev, uint32_t cap,
-                           uint32_t G, uint32_t *__restrict__ bpcnt, uint32_t *__restrict__ brecs) {
-    const uint32_t np = min(*npages_dev, cap);
-    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < np; p += gridDim.x * blockDim.x) {
-        const unsigned long long m = meta[p];
-        if (!m) continue;
-        const uint32_t bucket = (uint32_t)(m >> 40), grp = (uint32_t)(m >> 32) & 255u;
-        atomicAdd(&bpcnt[bucket * G + grp], 1u);
-        atomicAdd(&brecs[bucket], (uint32_t)m);
-    }
-}
-
+// and ordered by group. bpcnt[key] (pages) and brecs[bucket] (records) were counted as k_scatter2 closed the pages.
+// ---- level-2 pages -> bucket page lists ---------------------------------------------------------------
 __global__ void k_pgb_fill(const unsigned long long *__restrict__ meta, const uint32_t *__restrict__ npages_dev, uint32_t cap,
                            uint32_t G, const unsigned long long *__restrict__ bpstart, uint32_t *__restrict__ bpfill,
                            unsigned long long *__restrict__ blist) {

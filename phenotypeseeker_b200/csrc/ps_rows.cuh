@@ -167,8 +167,18 @@ __device__ __forceinline__ void bk_for_each_direct(const unsigned long long *__r
 __global__ void k_bucket_order_pg(const uint32_t *__restrict__ size, uint32_t big, uint32_t *__restrict__ fill,
                                   uint32_t *__restrict__ order) {
     const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= BK_N) return;
-    const uint32_t pos = size[b] > big ? atomicAdd(fill, 1u) : (uint32_t)(BK_N - 1) - atomicAdd(fill + 1, 1u);
+    if (b >= BK_N) return;                                 // BK_N is a multiple of 32: whole warps leave
+    // one atomicAdd per warp and side: 65,536 single ones on two counters serialise
+    const bool is_big = size[b] > big;
+    const unsigned mbig = __ballot_sync(0xffffffffu, is_big), msmall = ~mbig, lt = lanemask_lt();
+    uint32_t base_big = 0, base_small = 0;
+    if ((threadIdx.x & 31) == 0) {
+        if (mbig) base_big = atomicAdd(fill, (uint32_t)__popc(mbig));
+        if (msmall) base_small = atomicAdd(fill + 1, (uint32_t)__popc(msmall));
+    }
+    base_big = __shfl_sync(0xffffffffu, base_big, 0);
+    base_small = __shfl_sync(0xffffffffu, base_small, 0);
+    const uint32_t pos = is_big ? base_big + __popc(mbig & lt) : (uint32_t)(BK_N - 1) - (base_small + __popc(msmall & lt));
     order[pos] = b;
 }
 
@@ -296,7 +306,7 @@ k_bucket_build_pg(const uint32_t *__restrict__ recs_b, const unsigned long long 
 // --kmerDB (modeling.py:367-372: `glistcompare -i` of the database list with the feature vector):
 // keep the union k-mers that occur in the sorted database list `db`, and their matrix rows.
 // One warp per 32 union rows: a binary search per row, ballot -> the warp's kept rows. WRITE = false
-// counts them per warp (scanned by k_scan_counts); WRITE = true copies k-mer and row to their new
+// counts them per warp (scanned by k_scan_sums / k_scan_chunks); WRITE = true copies k-mer and row to their new
 // position, the lanes of the warp moving one row's words together.
 template <bool WRITE>
 __global__ void __launch_bounds__(256)

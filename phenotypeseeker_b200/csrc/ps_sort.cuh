@@ -259,48 +259,75 @@ k_rs_pass(const KeyT *__restrict__ kin, KeyT *__restrict__ kout, const uint16_t 
 }
 
 // ---------------------------------------------------------------------------------------
-// Exclusive scan u32 counts -> u64 offsets (offs[n] = total). Single block, 1024 threads.
-__global__ void __launch_bounds__(1024)
-k_scan_counts(const uint32_t *__restrict__ counts, uint64_t n, unsigned long long *__restrict__ offs) {
-    __shared__ unsigned long long wsum[32];
-    __shared__ unsigned long long carry_s;
-    const unsigned tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    if (tid == 0) carry_s = 0;
-    __syncthreads();
-    constexpr int PER = 8;
-    for (uint64_t base = 0; base < n; base += 1024ull * PER) {
-        uint32_t v[PER];
-        unsigned long long tsum = 0;
-        const uint64_t i0 = base + (uint64_t)tid * PER;
+// Exclusive scan u32 counts -> u64 offsets (offs[n] = total) in two launches over chunks of SCAN_CHUNK counts:
+// k_scan_sums adds up every chunk, k_scan_chunks scans each chunk from the sum of the chunks before it.
+#define SCAN_THREADS 1024
+#define SCAN_PER 8
+#define SCAN_CHUNK (SCAN_THREADS * SCAN_PER)
+
+// block-wide sum of one value per thread (SCAN_THREADS threads); every thread gets it
+__device__ __forceinline__ unsigned long long scan_block_sum(unsigned long long v, unsigned long long *ws) {
+    const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
-        for (int j = 0; j < PER; j++) { v[j] = (i0 + j < n) ? counts[i0 + j] : 0u; tsum += v[j]; }
-        unsigned long long inc = tsum;
+    for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if (lane == 0) ws[warp] = v;
+    __syncthreads();
+    unsigned long long t = ws[lane];
+#pragma unroll
+    for (int o = 16; o; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
+    __syncthreads();
+    return t;
+}
+
+__global__ void __launch_bounds__(SCAN_THREADS)
+k_scan_sums(const uint32_t *__restrict__ counts, uint64_t n, unsigned long long *__restrict__ sums) {
+    __shared__ unsigned long long ws[32];
+    const uint64_t base = (uint64_t)blockIdx.x * SCAN_CHUNK + threadIdx.x;
+    unsigned long long v = 0;
+#pragma unroll
+    for (int j = 0; j < SCAN_PER; j++) {
+        const uint64_t i = base + (uint64_t)j * SCAN_THREADS;
+        if (i < n) v += counts[i];
+    }
+    v = scan_block_sum(v, ws);
+    if (threadIdx.x == 0) sums[blockIdx.x] = v;
+}
+
+__global__ void __launch_bounds__(SCAN_THREADS)
+k_scan_chunks(const uint32_t *__restrict__ counts, uint64_t n, const unsigned long long *__restrict__ sums,
+              unsigned long long *__restrict__ offs) {
+    __shared__ unsigned long long ws[32];
+    const unsigned tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    unsigned long long before = 0;
+    for (uint32_t b = tid; b < blockIdx.x; b += SCAN_THREADS) before += sums[b];
+    before = scan_block_sum(before, ws);
+    uint32_t v[SCAN_PER];
+    unsigned long long tsum = 0;
+    const uint64_t i0 = (uint64_t)blockIdx.x * SCAN_CHUNK + (uint64_t)tid * SCAN_PER;
+#pragma unroll
+    for (int j = 0; j < SCAN_PER; j++) { v[j] = (i0 + j < n) ? counts[i0 + j] : 0u; tsum += v[j]; }
+    unsigned long long inc = tsum;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        unsigned long long t = __shfl_up_sync(0xffffffffu, inc, o);
+        if (lane >= (unsigned)o) inc += t;
+    }
+    if (lane == 31) ws[warp] = inc;
+    __syncthreads();
+    if (warp == 0) {
+        unsigned long long w = ws[lane], wi = w;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
-            unsigned long long t = __shfl_up_sync(0xffffffffu, inc, o);
-            if (lane >= (unsigned)o) inc += t;
+            unsigned long long t = __shfl_up_sync(0xffffffffu, wi, o);
+            if (lane >= (unsigned)o) wi += t;
         }
-        if (lane == 31) wsum[warp] = inc;
-        __syncthreads();
-        if (warp == 0) {
-            unsigned long long w = wsum[lane], wi = w;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                unsigned long long t = __shfl_up_sync(0xffffffffu, wi, o);
-                if (lane >= (unsigned)o) wi += t;
-            }
-            wsum[lane] = wi - w;  // exclusive
-        }
-        __syncthreads();
-        const unsigned long long carry = carry_s;
-        unsigned long long run = carry + wsum[warp] + inc - tsum;
-#pragma unroll
-        for (int j = 0; j < PER; j++) { if (i0 + j < n) offs[i0 + j] = run; run += v[j]; }
-        __syncthreads();
-        if (tid == 1023) carry_s = run;
-        __syncthreads();
+        ws[lane] = wi - w;  // exclusive
     }
-    if (tid == 0) offs[n] = carry_s;
+    __syncthreads();
+    unsigned long long run = before + ws[warp] + inc - tsum;
+#pragma unroll
+    for (int j = 0; j < SCAN_PER; j++) { if (i0 + j < n) offs[i0 + j] = run; run += v[j]; }
+    if (blockIdx.x == gridDim.x - 1 && tid == SCAN_THREADS - 1) offs[n] = run;
 }
 
 // ---------------------------------------------------------------------------------------
