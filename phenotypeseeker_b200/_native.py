@@ -401,6 +401,12 @@ class Context:
     def device_bytes(self):
         return self.L.ps_device_bytes(self.h)
 
+    def mem_info(self):
+        """(free bytes of the device, bytes this context holds): what a build could take."""
+        import torch
+        free, _total = torch.cuda.mem_get_info(self.device)
+        return int(free), int(self.device_bytes())
+
     def profile(self, on):
         self._ck(self.L.ps_profile_enable(self.h, 1 if on else 0))
 

@@ -280,20 +280,33 @@ static Sc1Dst paged_local_dst(ps_ctx *c) {
     return d;
 }
 
+// Level-2 reserve (2 KB pages behind the level-1 pages): what k_scatter2's blocks may need beyond the halves of the
+// level-1 pages they have read, (streams + 2 x blocks) x 256 pages (the bound is derived in ps_paged.cuh).
+static uint64_t paged_reserve_pages(const ps_ctx *c) {
+    return ((uint64_t)paged_groups(c) * SC_BINS1 + 2 * c->sc2_grid) * 256 * c->pgR_mult;
+}
+
+// The level-1 buffer: cap pages of 4 KB and the level-2 reserve behind them, reserved exactly (it is most of the
+// device memory a large job takes). Level-2 slot numbers must fit 32 bits.
+static void paged_reserve_pool(ps_ctx *c, uint64_t cap, bool keep) {
+    if (keep) cap = std::max<uint64_t>(cap, c->pgA_cap);
+    const uint64_t res = paged_reserve_pages(c);
+    if (2 * cap + res >= (1ull << 32)) PS_THROW(PS_ERR_NOMEM, "level-1 page pool of %llu pages: cut the job into k-mer ranges", (unsigned long long)cap);
+    const uint32_t old_cap = c->pgA_cap;
+    c->keys_a.reserve(cap * PG_A * 4 + res * PG_B * 4, c->stream, keep, (size_t)old_cap * PG_A * 4, true);
+    c->pg_meta_a.reserve(cap * 4, c->stream, keep, (size_t)old_cap * 4);
+    if (keep && cap > old_cap) CK(cudaMemsetAsync(c->pg_meta_a.as<uint32_t>() + old_cap, 0, (cap - old_cap) * 4, c->stream));
+    c->pgA_cap = (uint32_t)cap;
+    c->pgR_cap = (uint32_t)res;
+}
+
 // Level-1 pool for up to n_upper records on this GPU alone (one destination, no splitters). Clears the
 // page metas, cursors and block states. keep: the pool already holds live pages (ingest of a later batch).
 static Sc1Dst paged_begin_local(ps_ctx *c, uint64_t n_upper, bool keep, uint32_t slack_mult = 1) {
     const PagedTabs t = paged_tabs(c);
     const uint64_t slack = (uint64_t)c->sc1_grid * SC_BINS1 * (paged_groups(c) + 2) * slack_mult;   // open + spare pages
     const uint64_t cap = ceil_div<uint64_t>(n_upper, PG_A) + slack;
-    if (cap >= (1ull << 31)) PS_THROW(PS_ERR_NOMEM, "level-1 page pool of %llu pages: cut the job into k-mer ranges", (unsigned long long)cap);
-    const uint32_t old_cap = c->pgA_cap;
-    if (!keep || cap > old_cap) {
-        c->keys_a.reserve(cap * PG_A * 4, c->stream, keep, (size_t)old_cap * PG_A * 4);
-        c->pg_meta_a.reserve(cap * 4, c->stream, keep, (size_t)old_cap * 4);
-        if (keep) CK(cudaMemsetAsync(c->pg_meta_a.as<uint32_t>() + old_cap, 0, (cap - old_cap) * 4, c->stream));
-        c->pgA_cap = (uint32_t)cap;
-    }
+    if (!keep || cap > c->pgA_cap || paged_reserve_pages(c) != c->pgR_cap) paged_reserve_pool(c, cap, keep);
     c->pg_state.reserve((size_t)(c->sc1_grid + c->sc2_grid) * sizeof(ScState), c->stream, keep,
                         (size_t)(c->sc1_grid + c->sc2_grid) * sizeof(ScState));
     c->l1_live = false;
@@ -342,8 +355,19 @@ static void launch_scatter1(ps_ctx *c, const Sc1Src &src, const Sc1Dst &dst) {
 }
 
 // Thrown by paged_finish when records did not fit the page pools (PS_ERR_NOMEM): callers that can take larger pools
-// catch this type and build again.
+// catch this type and build again (a larger reserve if the level-2 reserve ran out: pgR_mult has doubled). k_scatter2
+// has then written over level-1 pages of the build's bins: the records must be extracted again.
 struct PagePoolExhausted : PsError {};
+
+// ps_scatter_range's pool: which level-1 bins a build has consumed
+static bool l1_consumed(const ps_ctx *c, uint32_t blo, uint32_t bhi) {
+    for (uint32_t b = blo; b < bhi; b++)
+        if ((c->l1_used[b >> 6] >> (b & 63)) & 1ull) return true;
+    return false;
+}
+static void l1_consume(ps_ctx *c, uint32_t blo, uint32_t bhi) {
+    for (uint32_t b = blo; b < bhi; b++) c->l1_used[b >> 6] |= 1ull << (b & 63);
+}
 
 // level-1 pages (this GPU's pool, pgA_cap pages, metas final) -> union + matrix
 // bin_lo / bin_hi: only the level-1 bins [bin_lo, bin_hi) take part (a sub-range of what the pool was scattered
@@ -367,19 +391,16 @@ static void paged_finish(ps_ctx *c, const Sc1Dst &dst_for_close, bool close_loca
     KLAUNCH(c, "pga_fill", (double)npa * 4,
             (k_pga_pages<true><<<ceil_div<uint32_t>(npa, PGL_THREADS * PGL_PER), PGL_THREADS, 0, c->stream>>>(
                 c->pg_meta_a.as<uint32_t>(), npa, bin_lo, bin_hi, t.scnt, t.tstart, t.sfill, c->pg_tiles.as<Sc2Tile>())));
-    // level-2 pool: every record once + the pages a block leaves half full when it moves to another stream
-    const uint64_t capb = ceil_div<uint64_t>(n_upper, PG_B) + ((uint64_t)paged_groups(c) * SC_BINS1 + 2 * c->sc2_grid) * 256;   // open + spare pages
-    if (capb >= (1ull << 31)) PS_THROW(PS_ERR_NOMEM, "level-2 page pool of %llu pages: cut the job into k-mer ranges", (unsigned long long)capb);
-    c->keys_b.reserve(capb * PG_B * 4, c->stream);
-    c->pg_meta_b.reserve(capb * 8, c->stream);
-    c->pgB_cap = (uint32_t)capb;
+    // level 2 writes its pages into the halves of the level-1 pages it has read, then into the reserve behind them
+    const uint64_t nslots = 2ull * npa + c->pgR_cap;
+    c->pg_meta_b.reserve(nslots * 8, c->stream);
     const uint32_t G = (uint32_t)paged_groups(c);
     Sc2Args a;
-    a.recs_a = c->keys_a.as<uint32_t>();
+    a.recs = c->keys_a.as<uint32_t>();
     a.tiles = c->pg_tiles.as<Sc2Tile>();
     a.ntiles = t.tstart + t.ns; a.bin_d2 = t.bin_d2;
-    a.recs_b = c->keys_b.as<uint32_t>(); a.meta_b = c->pg_meta_b.as<unsigned long long>();
-    a.cap_b = c->pgB_cap; a.cursor_b = t.cursor_b; a.overflow = t.overflow; a.trash = t.trash;
+    a.meta_b = c->pg_meta_b.as<unsigned long long>();
+    a.res0 = 2 * npa; a.nres = c->pgR_cap; a.cursor_b = t.cursor_b; a.overflow = t.overflow; a.trash = t.trash;
     a.bpcnt = t.bpcnt; a.brecs = t.brecs; a.G = G;
     KLAUNCH(c, "scatter2", (double)n_upper * 8, (k_scatter2<<<c->sc2_grid, SC_THREADS, SC2_SMEM, c->stream>>>(a, st2)));
     KLAUNCH(c, "pg_close", 0.0, (k_pg_close2<<<c->sc2_grid, 288, 0, c->stream>>>(st2, t.bin_d2, a.meta_b, t.bpcnt, t.brecs, G)));
@@ -388,9 +409,9 @@ static void paged_finish(ps_ctx *c, const Sc1Dst &dst_for_close, bool close_loca
     CK(cudaMemsetAsync(bt.fill, 0, 16, c->stream));
     const int lg = PS_SMS * 8;
     scan_counts_dev(c, "scan_bpages", t.bpcnt, (uint64_t)BK_N * G, bt.bstart);
-    c->pg_blist.reserve((size_t)capb * 8, c->stream);
-    KLAUNCH(c, "pgb_fill", (double)capb * 8, (k_pgb_fill<<<lg, 256, 0, c->stream>>>(a.meta_b, t.cursor_b, c->pgB_cap, G, bt.bstart, t.bpfill,
-                                                                                c->pg_blist.as<unsigned long long>())));
+    c->pg_blist.reserve((size_t)nslots * 8, c->stream);
+    KLAUNCH(c, "pgb_fill", (double)npa * 20, (k_pgb_fill<<<lg, 256, 0, c->stream>>>(a.meta_b, a.tiles, a.ntiles, t.cursor_b, a.res0, a.nres, G,
+                                                                                 bt.bstart, t.bpfill, c->pg_blist.as<unsigned long long>())));
     KLAUNCH(c, "bucket_order", (double)BK_N * 8, (k_bucket_order_pg<<<BK_N / 256, 256, 0, c->stream>>>(
                                      t.brecs, (uint32_t)std::min<uint64_t>(4 * (n_upper / BK_N) + 4096, 0xFFFFFFFFu), bt.fill, bt.order)));
     const int nwords = lbits >= 5 ? (1 << (lbits - 5)) : 1;
@@ -398,7 +419,7 @@ static void paged_finish(ps_ctx *c, const Sc1Dst &dst_for_close, bool close_loca
     uint32_t *gbm = c->tmp1.as<uint32_t>();
     KLAUNCH(c, "bucket_count", (double)n_upper * 4,
             (k_bucket_count_pg<<<BK_N, BK_THREADS, 0, c->stream>>>(
-                a.recs_b, c->pg_blist.as<unsigned long long>(), bt.bstart, G, bt.order, lbits, bt.counts, gbm)));
+                a.recs, c->pg_blist.as<unsigned long long>(), bt.bstart, G, bt.order, lbits, bt.counts, gbm)));
     scan_counts_dev(c, "scan_rows", bt.counts, BK_N, bt.first_row);
     const uint32_t stride = (uint32_t)std::min(c->row_words, 8) + 1;      // rows are assembled in 8-word column slices
     const uint32_t cap_small = (uint32_t)std::max(c->bk_row_words, round_up<int>((int)stride, 4));
@@ -415,7 +436,8 @@ static void paged_finish(ps_ctx *c, const Sc1Dst &dst_for_close, bool close_loca
     CK(cudaStreamSynchronize(c->stream));
     if (h32[1]) {
         char m[160];
-        snprintf(m, sizeof(m), "page pool exhausted (level-1 %u of %u pages, level-2 %u of %u)", h32[2], c->pgA_cap, h32[3], c->pgB_cap);
+        snprintf(m, sizeof(m), "page pool exhausted (level-1 %u of %u pages, level-2 reserve %u of %u)", h32[2], c->pgA_cap, h32[3], c->pgR_cap);
+        if (h32[3] > c->pgR_cap) c->pgR_mult *= 2;
         throw PagePoolExhausted{{PS_ERR_NOMEM, m}};
     }
     const uint64_t U = h[0];
@@ -431,12 +453,12 @@ static void paged_finish(ps_ctx *c, const Sc1Dst &dst_for_close, bool close_loca
     if (nbig)
         KLAUNCH(c, "bucket_build", alg * nbig / BK_N,
                 (k_bucket_build_pg<BK_MAX_THREADS><<<nbig, BK_MAX_THREADS, sm_big, c->stream>>>(
-                    a.recs_b, blist, bt.bstart, G, bt.order2, bt.first_row, gbm, lbits, c->row_words, cap_big,
+                    a.recs, blist, bt.bstart, G, bt.order2, bt.first_row, gbm, lbits, c->row_words, cap_big,
                     c->uni.as<uint64_t>(), c->matrix.as<uint32_t>())));
     if (nbig < BK_N)
         KLAUNCH(c, "bucket_build", alg * (BK_N - nbig) / BK_N,
                 (k_bucket_build_pg<BK_THREADS><<<BK_N - nbig, BK_THREADS, sm_small, c->stream>>>(
-                    a.recs_b, blist, bt.bstart, G, bt.order2 + nbig, bt.first_row, gbm, lbits, c->row_words, cap_small,
+                    a.recs, blist, bt.bstart, G, bt.order2 + nbig, bt.first_row, gbm, lbits, c->row_words, cap_small,
                     c->uni.as<uint64_t>(), c->matrix.as<uint32_t>())));
 }
 
@@ -536,12 +558,12 @@ static void add_samples_impl(ps_ctx *c, int first_idx, int count, const void *co
     if (pre && !ing) {
         uint64_t ub = pool0;
         for (int i = 0; i < count; i++) ub += round_up<uint64_t>(lens[i] + 1, POS_ALIGN);
-        // scattering during ingest only pays when the whole job fits at once (both page pools, 4 B per
-        // instance each, within a third of the free memory); larger jobs are built in k-mer ranges later
+        // scattering during ingest only pays when the whole job fits at once (the level-1 page pool, 4 B per
+        // instance, within a third of the free memory); larger jobs are built in k-mer ranges later
         size_t mem_free = 0, mem_total = 0;
         cudaMemGetInfo(&mem_free, &mem_total);
         const uint64_t have = (uint64_t)mem_free + c->keys_a.cap + c->keys_b.cap;
-        if (ub * 8 > have / 3) pre = false;
+        if (ub * 4 > have / 3) pre = false;
     }
     if (pre) {
         uint64_t ub = pool0;
@@ -798,21 +820,18 @@ static void build_union_impl(ps_ctx *c) {
             const uint64_t l1hi = c->l1_hi == 0 ? space : c->l1_hi;
             const bool lo_ok = lo == c->l1_lo || (lo > c->l1_lo && (lo & ((1ull << bshift) - 1)) == 0);
             const bool hi_ok = hi == l1hi || (hi < l1hi && (hi & ((1ull << bshift) - 1)) == 0);
-            if (lo_ok && hi_ok && lo < hi) {
-                const uint32_t blo = (uint32_t)(lo >> bshift), bhi = (uint32_t)((hi - 1) >> bshift) + 1;
-                n_upper = std::min<uint64_t>(n_upper, c->l1_instances);
-                for (int attempt = 0;; attempt++) {
-                    try {
-                        paged_finish(c, paged_local_dst(c), false, bin_d2, n_upper, blo, bhi, true);
-                        break;
-                    } catch (const PagePoolExhausted &) {
-                        if (attempt >= 3) throw;
-                        n_upper = std::min<uint64_t>(c->l1_instances, n_upper * 2);      // level 2 ran out: larger pool, same level 1
-                    }
+            const uint32_t blo = (uint32_t)(lo >> bshift), bhi = lo < hi ? (uint32_t)((hi - 1) >> bshift) + 1 : 0u;
+            if (lo_ok && hi_ok && lo < hi && !l1_consumed(c, blo, bhi)) {
+                // level 2 writes over the level-1 pages of these bins: a later build of them extracts again
+                l1_consume(c, blo, bhi);
+                try {
+                    paged_finish(c, paged_local_dst(c), false, bin_d2, std::min<uint64_t>(n_upper, c->l1_instances), blo, bhi, true);
+                    return;
+                } catch (const PagePoolExhausted &) {
+                    // the level-2 reserve ran out (pgR_mult has doubled): extract the range again below
                 }
-                return;
             }
-            c->l1_live = false;      // another range: extract again
+            c->l1_live = false;      // another range, or one already built: extract again
         }
         for (int attempt = 0;; attempt++) {
             Sc1Dst d;
@@ -1169,6 +1188,7 @@ int ps_scatter_range(ps_ctx *c, uint64_t lo, uint64_t hi, uint64_t n_instances) 
             if (!h32[0]) {
                 c->l1_instances = (uint64_t)std::min<uint32_t>(h32[1], c->pgA_cap) * PG_A;
                 c->l1_live = true;
+                memset(c->l1_used, 0, sizeof(c->l1_used));
                 c->l1_lo = lo;
                 c->l1_hi = hi_n;
                 return PS_OK;
@@ -1204,6 +1224,7 @@ int ps_scatter_range(ps_ctx *c, uint64_t lo, uint64_t hi, uint64_t n_instances) 
     }
     c->range_lo = keep_lo; c->range_hi = keep_hi; c->range_all = keep_all;
     c->l1_live = true;
+    memset(c->l1_used, 0, sizeof(c->l1_used));
     c->l1_lo = lo;
     c->l1_hi = (hi == 0 || hi >= space) ? 0 : hi;
     API_END(c)
@@ -1830,10 +1851,8 @@ int ps_route_setup(ps_ctx *c, int nparts, int my_rank, const uint64_t *splitters
     c->route_n = nparts; c->route_rank = my_rank; c->route_pages = (uint32_t)pages_per_sender;
     c->pre_valid = false; c->pgA_live = false; c->l1_live = false;
     paged_tabs(c);
-    c->keys_a.reserve(cap * PG_A * 4, c->stream);
-    c->pg_meta_a.reserve(cap * 4, c->stream);
+    paged_reserve_pool(c, cap, false);
     c->pg_state.reserve((size_t)(c->sc1_grid + c->sc2_grid) * sizeof(ScState), c->stream);
-    c->pgA_cap = (uint32_t)cap;
     // the peers' mappings stay valid as long as nothing changed shape or moved
     if (!same_shape || c->route_pool[my_rank] != c->keys_a.p || c->route_meta[my_rank] != c->pg_meta_a.p)
         for (int d = 0; d < PART_MAX; d++) { c->route_pool[d] = nullptr; c->route_meta[d] = nullptr; }

@@ -39,10 +39,13 @@ struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
     uint64_t *acct = nullptr;  // context-wide byte counter
-    void reserve(size_t bytes, cudaStream_t st, bool keep = false, size_t keep_bytes = 0) {
+    // exact: no room for growth (the page pool, sized from what the job needs). Without keep the old buffer is
+    // freed before the new one is taken, so that a large buffer can be replaced by a larger one.
+    void reserve(size_t bytes, cudaStream_t st, bool keep = false, size_t keep_bytes = 0, bool exact = false) {
         if (bytes <= cap) return;
-        size_t ncap = bytes + bytes / 8 + 256;
+        size_t ncap = exact ? bytes : bytes + bytes / 8 + 256;
         ncap = (ncap + 255) & ~size_t(255);
+        if (!keep) release(st);
         void *np = nullptr;
         cudaError_t e = cudaMalloc(&np, ncap);
         if (e != cudaSuccess)
@@ -59,7 +62,8 @@ struct DevBuf {
         p = np;
         cap = ncap;
     }
-    void release() {
+    void release(cudaStream_t st = nullptr) {
+        if (p && st) CK(cudaStreamSynchronize(st));
         if (p) cudaFree(p);
         if (acct) *acct -= cap;
         p = nullptr;
@@ -126,9 +130,11 @@ struct ps_ctx {
     bool sc1_lean = true;       // k_scatter1 recomputes its k-mers in the grouping phase (40 registers, 3 blocks per SM); PSKMER_SC1=regs: keeps them in registers (2 blocks per SM)
     bool chi2_sparse_force = false;   // PSKMER_CHI2=walk: the bit-walk kernel for every unweighted shape it can take (tests)
 
-    // paged partition (ps_paged.cuh): level-1 pool = keys_a, level-2 pool = keys_b
+    // paged partition (ps_paged.cuh): level-1 pool = keys_a: pgA_cap pages of 4 KB, then pgR_cap level-2 reserve
+    // pages of 2 KB (the other level-2 pages are the halves of level-1 pages k_scatter2 has read)
     int sc1_grid = 2 * PS_SMS, sc2_grid = 3 * PS_SMS;   // sc2_grid: k_scatter2 runs three blocks per SM (SC2_BLOCKS_PER_SM)
-    uint32_t pgA_cap = 0, pgB_cap = 0;   // pages
+    uint32_t pgA_cap = 0, pgR_cap = 0;   // pages
+    uint32_t pgR_mult = 1;      // reserve multiple: doubles when a build overran the reserve (kept for the context's life)
     double sc1_out_frac = 1.0;  // share of the positions whose record k_scatter1 writes (range-restricted runs): profile accounting only
     uint64_t cap_hint = 0;      // ps_set_capacity_hint: expected k-mer instances of the next build (0 = from input size)
     bool pgA_live = false;      // level-1 pool holds the records of pool positions [0, pre_n) (scattered during ingest)
@@ -142,6 +148,7 @@ struct ps_ctx {
     uint64_t pre_lo = 0, pre_hi = 0;
     bool l1_live = false;
     uint64_t l1_lo = 0, l1_hi = 0;
+    uint64_t l1_used[8] = {};   // level-1 bins whose pages a build has consumed (level-2 pages were written over them)
     uint64_t l1_instances = 0;  // records in the pool (pages x 1024, upper bound)
 
     // stage 2 results

@@ -28,7 +28,8 @@
 //   k_scatter2  level-2 partition of every stream (group, bin) by d1 into pages of 512 records
 //               tagged (bucket = d2 << 8 | d1, group). Input pages come in through the TMA unit
 //               (cp.async.bulk global -> shared, mbarrier completion); closing a page also counts
-//               it for its bucket's page list.
+//               it for its bucket's page list. The level-2 pages are the halves of the level-1 pages
+//               the block has read (plus a small reserve): no second pool.
 //   k_pgb_fill  pages -> per-bucket page lists (+ record counts for largest-first scheduling).
 //
 // The order of records inside a bucket is arbitrary (and varies from run to run); the bucket
@@ -592,15 +593,27 @@ k_pga_pages(const uint32_t *__restrict__ meta, uint32_t npages, uint32_t bin_lo,
 }
 
 // ---- level 2: pages of one stream -> pages of its 256 buckets ----------------------------------------
+// Level-2 pages (2 KB) live in the level-1 buffer: slots 2p and 2p + 1 are the two halves of level-1 page p, and the
+// `nres` slots from res0 = 2 x (level-1 pages) on are a reserve that the level-1 cursor never hands out. k_scatter2
+// reads every level-1 page of a range exactly once; when the copy of a tile has completed, the tile's pages are dead
+// and their slots join the SUPPLY of the block that read them. A block takes its pages from its own supply first, so
+// only the block that read a page ever writes it, and no separate level-2 pool is needed.
+//
+// Reserve bound. The records of a block's tiles up to tile t fill at most two slots per level-1 page of those tiles,
+// and that is what its supply has received by then. Beyond that the block holds at most 256 open pages, and every
+// change of stream closes at most 256 partial pages. A block changes stream at most once per stream of its tile
+// interval, so over all blocks demand beyond supply is at most (streams + 2 x blocks) x 256 pages, with streams <=
+// G x SC_BINS1 (a level-1 stream is a (group, bin) pair): one term for the stream a block shares with its neighbour,
+// one for the open pages at the end. The supply ring drops slots only while it holds SC2_FREE >= 256 + 16 of them;
+// whatever the block is short of afterwards is again covered by its stream changes. The overflow flag stays as a check.
 struct Sc2Args {
-    const uint32_t *recs_a;              // level-1 pool (this GPU's own)
+    uint32_t *recs;                      // level-1 pool (this GPU's own) and, in the same bytes, the level-2 slots
     const Sc2Tile *tiles;
     const uint32_t *ntiles;              // device scalar: tstart[ns]
     const uint8_t *bin_d2;               // [SC_BINS1] bin -> d2 for the bins this GPU owns
-    uint32_t *recs_b;                    // level-2 pool
-    unsigned long long *meta_b;
-    uint32_t cap_b;
-    uint32_t *cursor_b;
+    unsigned long long *meta_b;          // per level-2 slot
+    uint32_t res0, nres;                 // reserve slots [res0, res0 + nres)
+    uint32_t *cursor_b;                  // reserve slots taken
     uint32_t *overflow;
     uint32_t *trash;
     uint32_t *bpcnt, *brecs;             // [BK_N * G] pages per (bucket, group), [BK_N] records per bucket
@@ -621,6 +634,58 @@ __device__ __forceinline__ void pgb_close(unsigned long long *meta_b, uint32_t *
 // (Two landing zones of 4096 records at four blocks per SM, ranks kept in registers: 124 vs 81 ms on config 5.)
 #define SC2_BLOCKS_PER_SM 3
 #define SC2_SMEM (2 * SC_TILE * 4 + sizeof(ScShared<256>))
+#define SC2_FREE 512                     // supply ring of a block: >= 256 open pages + the 16 slots of one tile
+#define SC2_XPG 32                       // pages of the runs longer than one page in one tile: <= 8192 / 512 + 15
+
+// One level-2 page: the oldest free slot of the block's supply (ring[head, tail)), else a reserve slot.
+__device__ __forceinline__ uint32_t sc2_take(const Sc2Args &a, const uint32_t *ring, uint32_t *head, uint32_t tail) {
+    const uint32_t h = atomicAdd(head, 1u);
+    if (h < tail) return ring[h & (SC2_FREE - 1)];
+    const uint32_t r = atomicAdd(a.cursor_b, 1u);
+    return r < a.nres ? a.res0 + r : PG_NONE;
+}
+
+// Page bookkeeping of bin `b` for a tile that holds c > 0 records of it starting at tile-local index tb: like
+// sc_place_run, except that pages come one at a time and need not be adjacent. A remainder longer than one page is
+// described by its page addresses in xpg[x ..] (pb = x << 1 | 1; a page address is even).
+template <typename CloseFn>
+__device__ __forceinline__ void sc2_place_run(const Sc2Args &a, uint32_t c, uint32_t tb, uint32_t &pg, uint32_t &fill,
+                                              const uint32_t *ring, uint32_t *head, uint32_t tail, unsigned long long *xpg,
+                                              uint32_t *nx, uint32_t &split, unsigned long long &pa, unsigned long long &pb,
+                                              CloseFn close_page) {
+    auto addr = [&](uint32_t slot) -> unsigned long long {
+        return reinterpret_cast<unsigned long long>(slot == PG_NONE ? a.trash : a.recs + (size_t)slot * PG_B);
+    };
+    if (pg == PG_NONE) { pg = sc2_take(a, ring, head, tail); fill = 0; }
+    if (pg == PG_NONE) {
+        *a.overflow = 1u;
+        split = tb + c;
+        pa = pb = addr(PG_NONE) - 4ull * tb;
+        return;
+    }
+    const uint32_t lenA = min(c, (uint32_t)PG_B - fill);
+    pa = addr(pg) + 4ull * fill - 4ull * tb;
+    split = tb + lenA;
+    fill += lenA;
+    if (fill == PG_B) { close_page(pg, (uint32_t)PG_B); pg = PG_NONE; fill = 0; }
+    const uint32_t rest = c - lenA;
+    pb = pa;
+    if (!rest) return;
+    const uint32_t nnew = (rest + PG_B - 1) / PG_B;
+    const uint32_t x = nnew > 1 ? atomicAdd(nx, nnew) : 0u;
+    for (uint32_t q = 0; q < nnew; q++) {
+        const uint32_t s = sc2_take(a, ring, head, tail);
+        if (s == PG_NONE) *a.overflow = 1u;
+        if (nnew > 1) xpg[x + q] = addr(s);
+        else pb = addr(s) - 4ull * (tb + lenA);
+        const uint32_t n = min(rest - q * PG_B, (uint32_t)PG_B);
+        if (s != PG_NONE) {
+            if (n == PG_B) close_page(s, (uint32_t)PG_B);
+            else { pg = s; fill = n; }
+        }
+    }
+    if (nnew > 1) pb = (unsigned long long)x << 1 | 1ull;
+}
 
 __global__ void __launch_bounds__(SC_THREADS, SC2_BLOCKS_PER_SM)
 k_scatter2(Sc2Args a, ScState *__restrict__ state) {
@@ -631,17 +696,22 @@ k_scatter2(Sc2Args a, ScState *__restrict__ state) {
     ScShared<NB> &S = *reinterpret_cast<ScShared<NB> *>(sc2_dyn + 2 * SC_TILE * 4);
     __shared__ __align__(8) uint64_t bar;
     __shared__ uint32_t s_pcnt[SC_TILE_PAGES];
+    __shared__ uint32_t s_tpage[SC_TILE_PAGES];                     // level-1 pages of the tile in the landing zone
     __shared__ uint32_t s_key;
     __shared__ uint32_t s_cur_key;
     __shared__ Sc2Tile s_next;                                      // descriptor of the next tile to copy in
+    __shared__ uint32_t s_ring[SC2_FREE];                           // the block's supply: free slots [s_head, s_tail)
+    __shared__ uint32_t s_head, s_tail, s_nx;
+    __shared__ unsigned long long s_xpg[SC2_XPG];
     const unsigned tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     ScState &st = state[blockIdx.x];
     const uint32_t T = *a.ntiles;
     const uint32_t t_lo = (uint32_t)((uint64_t)T * blockIdx.x / gridDim.x), t_hi = (uint32_t)((uint64_t)T * (blockIdx.x + 1) / gridDim.x);
-    uint32_t my_pg = PG_NONE, my_fill = 0, my_spare = PG_NONE;      // thread b < 256 owns bin b
-    if (tid < NB) { my_pg = st.page[tid]; my_fill = st.fill[tid]; my_spare = st.spare[tid]; S.cnt[0][tid] = 0; S.cnt[1][tid] = 0; }
+    uint32_t my_pg = PG_NONE, my_fill = 0;                          // thread b < 256 owns bin b
+    if (tid < NB) { S.cnt[0][tid] = 0; S.cnt[1][tid] = 0; }
     if (tid == 0) {
-        s_cur_key = st.key;
+        s_cur_key = 0;
+        s_head = 0; s_tail = 0; s_nx = 0;
         mbar_init(&bar, 1);
         mbar_fence_init();
     }
@@ -660,10 +730,10 @@ k_scatter2(Sc2Args a, ScState *__restrict__ state) {
         const uint32_t c = lane < SC_TILE_PAGES && lane < s_next.np ? (uint32_t)s_next.cnt[lane] : 0u;
         const uint32_t bytes = (c * 4 + 15) & ~15u;
         const uint32_t total = __reduce_add_sync(0xffffffffu, bytes);
-        if (lane < SC_TILE_PAGES) s_pcnt[lane] = c;
+        if (lane < SC_TILE_PAGES) { s_pcnt[lane] = c; s_tpage[lane] = s_next.page[lane]; }
         if (lane == 0) { s_key = s_next.key; mbar_expect_tx(&bar, total); }
         __syncwarp();
-        if (bytes) bulk_g2s(sin + lane * PG_A, a.recs_a + (size_t)s_next.page[lane] * PG_A, bytes, &bar);
+        if (bytes) bulk_g2s(sin + lane * PG_A, a.recs + (size_t)s_next.page[lane] * PG_A, bytes, &bar);
         __syncwarp();                                               // s_next has been read: the next fetch may land
     };
     if (warp == 0 && t_lo < t_hi) {
@@ -676,7 +746,23 @@ k_scatter2(Sc2Args a, ScState *__restrict__ state) {
         uint32_t *cnt = S.cnt[buf], *cnt_next = S.cnt[buf ^ 1];
         mbar_wait(&bar, phase);
         phase ^= 1u;
-        if (warp == 0) fetch(t + 1);
+        if (warp == 0) {
+            // The tile's pages have been read: their slots join the supply. No proxy fence is needed before the generic
+            // stores that will reuse these bytes: the complete_tx that ended the wait comes after the bulk copy has read
+            // its source, and the completion of a bulk copy carries an implicit generic-async proxy fence (PTX ISA,
+            // cp.async.bulk). A slot's meta is cleared here, so that a slot that is never used lists nothing.
+            const bool v = lane < 2 * SC_TILE_PAGES && s_pcnt[lane >> 1] != 0;
+            const uint32_t nslot = __popc(__ballot_sync(0xffffffffu, v));
+            const uint32_t tail = s_tail, room = SC2_FREE - (tail - s_head);
+            if (v) {
+                const uint32_t slot = 2 * s_tpage[lane >> 1] + (lane & 1u);
+                a.meta_b[slot] = 0ull;
+                if (lane < room) s_ring[(tail + lane) & (SC2_FREE - 1)] = slot;
+            }
+            __syncwarp();
+            if (lane == 0) s_tail = tail + min(nslot, room);
+            fetch(t + 1);
+        }
         // ---- A: count the records of every bin (one shared-memory atomic per record) ----
 #pragma unroll
         for (int it = 0; it < SC_ITEMS; it++) {
@@ -700,10 +786,9 @@ k_scatter2(Sc2Args a, ScState *__restrict__ state) {
             if (c) {
                 const uint32_t bucket = ((uint32_t)a.bin_d2[key & 511u] << 8) | tid, grp = key >> 9;
                 unsigned long long *meta = a.meta_b;
-                uint32_t nfull = 0;                                // pages sc_place_run closes are full
-                sc_place_run<PG_B>(c, tb, my_pg, my_fill, my_spare, a.recs_b, 0u, a.cap_b, a.cursor_b, a.overflow, a.trash,
-                                   S.split[tid], S.pab[tid][0], S.pab[tid][1],
-                                   [meta, bucket, grp, &nfull](uint32_t page, uint32_t n) { meta[page] = PGB_META(bucket, grp, n); nfull++; });
+                uint32_t nfull = 0;                                // pages sc2_place_run closes are full
+                sc2_place_run(a, c, tb, my_pg, my_fill, s_ring, &s_head, s_tail, s_xpg, &s_nx, S.split[tid], S.pab[tid][0],
+                              S.pab[tid][1], [meta, bucket, grp, &nfull](uint32_t page, uint32_t n) { meta[page] = PGB_META(bucket, grp, n); nfull++; });
                 if (nfull) {
                     atomicAdd(&a.bpcnt[bucket * a.G + grp], nfull);
                     atomicAdd(&a.brecs[bucket], nfull * PG_B);
@@ -711,7 +796,11 @@ k_scatter2(Sc2Args a, ScState *__restrict__ state) {
             }
         }
         __syncthreads();
-        if (tid == 0) s_cur_key = key;
+        if (tid == 0) {
+            s_cur_key = key;
+            if (s_head > s_tail) s_head = s_tail;                  // takes past the end went to the reserve
+            s_nx = 0;
+        }
         // ---- C: group the records in shared memory ----
         // cnt[bin] holds the bin's base and moves up with every record placed (the order inside a bin is free). The
         // volatile reads make this a second read of shared memory, not phase A's values kept in (spilled) registers.
@@ -726,12 +815,19 @@ k_scatter2(Sc2Args a, ScState *__restrict__ state) {
         __syncthreads();
         // the landing zone has been read: the next tile comes in during the write-out
         if (warp == 0 && t + 1 < t_hi) issue();
-        // ---- D: runs -> pages ----
-        sc_write_flat<NB>(sk, cnt[NB], S.split, S.pab, [](uint32_t v, uint32_t) { return v >> 24; },
-                          [](uint32_t v) { return v & 0x00FFFFFFu; });
+        // ---- D: runs -> pages (a run's piece B either linear or, longer than a page, through s_xpg) ----
+        const uint32_t total = cnt[NB];
+#pragma unroll 4
+        for (uint32_t p = tid; p < total; p += SC_THREADS) {
+            const uint32_t v = sk[p], b = v >> 24, sp = S.split[b];
+            const unsigned long long d = S.pab[b][p >= sp ? 1 : 0];
+            uint32_t *dst = (d & 1ull) ? reinterpret_cast<uint32_t *>(s_xpg[(uint32_t)(d >> 1) + ((p - sp) >> 9)]) + ((p - sp) & (PG_B - 1))
+                                       : reinterpret_cast<uint32_t *>(d) + p;
+            *dst = v & 0x00FFFFFFu;
+        }
         __syncthreads();
     }
-    if (tid < NB) { st.page[tid] = my_pg; st.fill[tid] = my_fill; st.spare[tid] = my_spare; }
+    if (tid < NB) { st.page[tid] = my_pg; st.fill[tid] = my_fill; }
     if (tid == 0) st.key = s_cur_key;
 }
 
@@ -746,8 +842,6 @@ __global__ void k_pg_close2(ScState *__restrict__ state, const uint8_t *__restri
         const uint32_t pg = st.page[tid], fill = st.fill[tid];
         if (pg != PG_NONE && fill)
             pgb_close(meta_b, bpcnt, brecs, G, pg, ((uint32_t)bin_d2[key & 511u] << 8) | tid, key >> 9, fill);
-        const uint32_t sp = st.spare[tid];
-        if (sp != PG_NONE) meta_b[sp] = 0ull;                  // taken ahead of need, never used: no stale meta
     }
     if (tid < SC_BINS1) { st.page[tid] = PG_NONE; st.fill[tid] = 0; st.spare[tid] = PG_NONE; }
     if (tid == 0) st.key = 0;
@@ -756,16 +850,26 @@ __global__ void k_pg_close2(ScState *__restrict__ state, const uint8_t *__restri
 // ---- level-2 pages -> bucket page lists ---------------------------------------------------------------
 // Pages are listed per (bucket, sample group): key = bucket * G + group, so a bucket's pages are contiguous
 // and ordered by group. bpcnt[key] (pages) and brecs[bucket] (records) were counted as k_scatter2 closed the pages.
-// ---- level-2 pages -> bucket page lists ---------------------------------------------------------------
-__global__ void k_pgb_fill(const unsigned long long *__restrict__ meta, const uint32_t *__restrict__ npages_dev, uint32_t cap,
-                           uint32_t G, const unsigned long long *__restrict__ bpstart, uint32_t *__restrict__ bpfill,
-                           unsigned long long *__restrict__ blist) {
-    const uint32_t np = min(*npages_dev, cap);
-    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < np; p += gridDim.x * blockDim.x) {
-        const unsigned long long m = meta[p];
+// The slots a build can have written are those of the level-1 pages of its tiles (their metas were cleared as they
+// joined a supply) and the reserve slots it took; every other slot may hold the meta of an earlier build.
+__global__ void k_pgb_fill(const unsigned long long *__restrict__ meta, const Sc2Tile *__restrict__ tiles,
+                           const uint32_t *__restrict__ ntiles_dev, const uint32_t *__restrict__ cursor_b, uint32_t res0,
+                           uint32_t nres, uint32_t G, const unsigned long long *__restrict__ bpstart,
+                           uint32_t *__restrict__ bpfill, unsigned long long *__restrict__ blist) {
+    const uint64_t ntv = (uint64_t)*ntiles_dev * (2 * SC_TILE_PAGES);
+    const uint64_t nv = ntv + min(*cursor_b, nres);
+    for (uint64_t v = blockIdx.x * blockDim.x + threadIdx.x; v < nv; v += gridDim.x * blockDim.x) {
+        uint32_t slot;
+        if (v < ntv) {
+            const Sc2Tile &tl = tiles[v / (2 * SC_TILE_PAGES)];
+            const uint32_t j = (uint32_t)(v >> 1) % SC_TILE_PAGES;
+            if (j >= tl.np) continue;
+            slot = 2 * tl.page[j] + (uint32_t)(v & 1);
+        } else slot = res0 + (uint32_t)(v - ntv);
+        const unsigned long long m = meta[slot];
         if (!m) continue;
         const uint32_t bucket = (uint32_t)(m >> 40), grp = (uint32_t)(m >> 32) & 255u;
         const uint32_t key = bucket * G + grp;
-        blist[bpstart[key] + atomicAdd(&bpfill[key], 1u)] = BKP_ENTRY(p, grp, (uint32_t)m);
+        blist[bpstart[key] + atomicAdd(&bpfill[key], 1u)] = BKP_ENTRY(slot, grp, (uint32_t)m);
     }
 }

@@ -344,7 +344,7 @@ def exchange_streams(ka: KmerAssociation, n_samples, rank, world, device, dist=T
     return int((max_pos // 4 + max_pos // 8) * (world - 1))
 
 
-POOL_BUDGET_BYTES = 38e9      # one level-1 pool per GPU; the level-2 pool is as large again
+POOL_BUDGET_BYTES = 38e9      # one level-1 pool per GPU; level 2 writes into its read pages (and a small reserve)
 
 
 class PageRoute:

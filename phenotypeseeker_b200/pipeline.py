@@ -39,6 +39,22 @@ def read_sample_file(path):
         return f.read()
 
 
+PS_SMS = 148                # B200
+PAGE_TABLE_BYTES = 48       # per level-1 page: its meta, two level-2 metas and page-list entries, a share of a tile
+HEADROOM_BYTES = 4 << 30    # union, sort and test buffers of a range, the runtime's own
+
+
+def level1_pool_bytes(n_instances, n_samples):
+    """Device bytes of the level-1 page pool for n_instances records of n_samples samples, as ps_api.cu's
+    paged_begin_local reserves it: 4 KB pages for the records, the pages every k_scatter1 block (3 per SM) may hold
+    open per bin (264) and sample group (+2), then the level-2 reserve of 2 KB pages (256 per level-1 stream and two
+    per k_scatter2 block). The level-2 pages proper are written into the level-1 pages k_scatter2 has read."""
+    groups = (int(n_samples) + 255) // 256
+    pages = -(-int(n_instances) // 1024) + 3 * PS_SMS * 264 * (groups + 2)
+    reserve = (groups * 264 + 2 * 3 * PS_SMS) * 256
+    return pages * 4096 + reserve * 2048
+
+
 def unpack_rows(rowbits, n_samples):
     """S x W uint32 -> S x N uint8 presence (sample s = bit s%32 of word s//32)."""
     rb = np.ascontiguousarray(rowbits, dtype=np.uint32)
@@ -157,13 +173,13 @@ class KmerAssociation:
             i = j
 
     def fits_in_one_build(self, headroom=0.8):
-        """Whether union + matrix of the whole k-mer space fit in this GPU's memory at once: two page pools
-        (4 B per k-mer instance each, + 10 %) plus a matrix with one row per (pessimistically) every fourth
-        instance. When not, the job runs in k-mer ranges (test_in_ranges)."""
+        """Whether union + matrix of the whole k-mer space fit in this GPU's memory at once: the page pool
+        (4 B per k-mer instance, + 10 %, and its level-2 reserve) plus a matrix with one row per (pessimistically)
+        every fourth instance. When not, the job runs in k-mer ranges (test_in_ranges)."""
         import torch
         n = self.ctx.instances_upper()
         row_bytes = self.ctx.row_words() * 4
-        need = n * 8 * 1.1 + (n / 4) * (8 + row_bytes) + (1 << 30)
+        need = level1_pool_bytes(n * 1.1, self.n_samples) + (n / 4) * (8 + row_bytes) + (1 << 30)
         free, _total = torch.cuda.mem_get_info(self.ctx.device)
         return need <= (free + self.ctx.device_bytes()) * headroom
 
@@ -172,8 +188,8 @@ class KmerAssociation:
         n = self.ctx.instances_upper()
         row_bytes = self.ctx.row_words() * 4
         free, _total = torch.cuda.mem_get_info(self.ctx.device)
-        have = (free + self.ctx.device_bytes()) * headroom - (1 << 30)
-        need = n * 8 * 1.3 + (n / 4) * (8 + row_bytes)
+        have = (free + self.ctx.device_bytes()) * headroom - (1 << 30) - level1_pool_bytes(0, self.n_samples)
+        need = n * 4 * 1.3 + (n / 4) * (8 + row_bytes)
         return max(1, int(np.ceil(need / max(have, 1))))
 
     def instances_upper(self):
@@ -299,21 +315,39 @@ class KmerAssociation:
         self.build()
         return self.test(pheno, binary, weights, **kw)
 
+    def _one_super_range(self, n_ranges, spl, n_instances):
+        """Whether the level-1 pool of the whole job fits beside everything else the context holds: the pool and its
+        reserve (level1_pool_bytes, as ps_scatter_range will size it), its page tables, the 2-bit streams, the
+        matrix of the largest range and some headroom, against the device's free memory plus what the context holds
+        now. The range sizes come from the previous test_in_ranges of the same job; without them, or with a context
+        that cannot report its memory, the answer is no."""
+        sizes = getattr(self, "_range_sizes", {}).get((self.k, self.n_samples, tuple(spl)))
+        mem_info = getattr(self.ctx, "mem_info", None)
+        if not n_instances or not sizes or mem_info is None:
+            return False
+        free, held = mem_info()
+        n = int(n_instances) + (1 << 20)
+        row_bytes = ((((self.n_samples + 31) // 32) + 3) // 4 * 4) * 4
+        need = (level1_pool_bytes(n, self.n_samples) + -(-n // 1024) * PAGE_TABLE_BYTES + n * 3 // 8 * 9 // 8
+                + max(sizes) * (8 + row_bytes) * 9 // 8 + HEADROOM_BYTES)
+        return need <= free + held
+
     def plan_ranges(self, n_ranges, splitters, n_instances=None, n_super=None):
         """Range boundaries, super-range grouping and pool capacities of a run in k-mer ranges (test_in_ranges).
+        n_super None: one super-range when its pool fits (_one_super_range), else half as many as ranges.
         -> dict(splitters, grouped, slack, first_of {first range of a super-range: one past its last},
         ingest (lo, hi, n_instances, share) of the FIRST super-range for count(ingest_range=...) or None)."""
         spl = [int(x) for x in splitters]
         assert len(spl) == n_ranges - 1
-        if n_super is None:
-            n_super = (n_ranges + 1) // 2
-        grouped = bool(n_ranges > 1 and n_super and 9 <= self.k <= 16)
+        grouped = bool(n_ranges > 1 and (n_super is None or n_super) and 9 <= self.k <= 16)
         if grouped:
             unit = 1 << (2 * self.k - 8)
             spl = [max(unit, (x + unit // 2) // unit * unit) for x in spl]
             for i in range(1, len(spl)):                       # keep them strictly ascending
                 spl[i] = max(spl[i], spl[i - 1] + unit)
             grouped = spl[-1] < (1 << (2 * self.k))
+        if n_super is None:
+            n_super = 1 if grouped and self._one_super_range(n_ranges, spl, n_instances) else (n_ranges + 1) // 2
         slack = 1.15 if grouped else 1.3
         first_of, ingest = {}, None
         if grouped:
@@ -323,8 +357,17 @@ class KmerAssociation:
                 first_of[a] = b
             if n_instances:
                 b = first_of[0]
-                ingest = (0, 0 if b == n_ranges else spl[b - 1], int(n_instances * slack * b / n_ranges) + (1 << 20), b / n_ranges)
+                ingest = (0, 0 if b == n_ranges else spl[b - 1], self._super_capacity(n_instances, slack, 0, b, n_ranges),
+                          b / n_ranges)
         return {"splitters": spl, "grouped": grouped, "slack": slack, "first_of": first_of, "ingest": ingest}
+
+    @staticmethod
+    def _super_capacity(n_instances, slack, a, b, n_ranges):
+        """Level-1 pool capacity (records) of the super-range of ranges [a, b): its share of the job's instances with
+        slack; the whole space takes n_instances itself, the text bytes, which already bound the positions."""
+        if b - a == n_ranges:
+            return int(n_instances) + (1 << 20)
+        return int(n_instances * slack * (b - a) / n_ranges) + (1 << 20)
 
     def test_in_ranges(self, pheno, binary, n_ranges, weights=None, pvalue_cutoff=0.05, omit_b=False,
                        splitters=None, n_instances=None, top_k=None, n_super=None, restrict=None, **kw):
@@ -334,7 +377,8 @@ class KmerAssociation:
         own, and the survivors are concatenated — ranges are ascending, so k-mer order and global
         ranks are those of a single build.
 
-        n_super (k = 9..16; default: half as many as ranges, 0 = off): the ranges are grouped into n_super
+        n_super (k = 9..16; default: one when the whole job's level-1 pool fits, else half as many as ranges;
+        0 = off): the ranges are grouped into n_super
         super-ranges whose k-mer instances are extracted ONCE into the level-1 page pool
         (ps_scatter_range); the ranges of a super-range then start from that pool. Their boundaries are
         moved to the nearest multiple of 4^(k-4) (a top-k-mer-byte boundary) for that.
@@ -359,14 +403,14 @@ class KmerAssociation:
         plan = self.plan_ranges(n_ranges, spl, n_instances, n_super)
         spl, grouped, slack, first_of = plan["splitters"], plan["grouped"], plan["slack"], plan["first_of"]
         self.range_splitters = spl
-        parts, U = [], 0
+        parts, U, sizes = [], 0, []
         for r in range(n_ranges):
             lo = 0 if r == 0 else spl[r - 1]
             hi = 0 if r == n_ranges - 1 else spl[r]
             if r in first_of:
                 b = first_of[r]
                 self.ctx.scatter_range(lo, 0 if b == n_ranges else spl[b - 1],
-                                       int(n_instances * slack * (b - r) / n_ranges) + (1 << 20) if n_instances else 0)
+                                       self._super_capacity(n_instances, slack, r, b, n_ranges) if n_instances else 0)
             if n_ranges > 1:
                 self.ctx.set_range(lo, hi)
                 if n_instances:
@@ -378,8 +422,10 @@ class KmerAssociation:
                             n_union_total=(U + u_r) if not (binary and omit_b) else None, **kw) if u_r else None
             parts.append((U, res))
             U += u_r
+            sizes.append(u_r)
         if n_ranges > 1:
             self.ctx.set_range(0, 0)      # back to the whole k-mer space
+            self._range_sizes = {(self.k, self.n_samples, tuple(spl)): sizes}   # the next call's super-range choice
         self.U = U
         exact = float(pvalue_cutoff) if (binary and omit_b) else (float(pvalue_cutoff) / U if U else 0.0)
         out = []
