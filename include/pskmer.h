@@ -164,6 +164,21 @@ int ps_test_welch(ps_ctx *ctx, int n_pheno, const double *pheno, const double *w
                   uint64_t *n_survivors);
 
 /*
+ * Permutation min-p: minp[c] = smallest p over the k-mers of this range's union that pass the sample filter,
+ * for each of the n_cols phenotype columns given (1 if none). Leaves union, matrix and the survivors of the
+ * last ps_test_* call untouched.
+ *
+ * Same table layout and conventions as ps_test_chi2 / ps_test_welch (column c at pheno[c*N + s]); the
+ * columns are typically permutations of an observed column. The statistic and p of a (k-mer, column) pair
+ * are those ps_test_* computes; a NaN p is never a minimum. Runs the columns in batches, one pass over the
+ * matrix per batch. For Westfall & Young's single-step min-p threshold (DESIGN.md "Permutation threshold").
+ */
+int ps_minp_chi2(ps_ctx *ctx, int n_cols, const int8_t *pheno, const double *weights,
+                 int min_samples, int max_samples, double *minp);
+int ps_minp_welch(ps_ctx *ctx, int n_cols, const double *pheno, const double *weights,
+                  int min_samples, int max_samples, double *minp);
+
+/*
  * Top-k cut on device: of the survivors of the last ps_test_* call keep, for every phenotype column, the
  * n_top with the smallest p-values (numeric order; every survivor tied with the n_top-th is kept too, so
  * slightly more than n_top may remain). ps_fetch_survivors then returns only those. *n_selected = how

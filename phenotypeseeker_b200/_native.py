@@ -36,6 +36,10 @@ SIGNATURES = {
                                     ctypes.c_int, ctypes.c_int, ctypes.c_double, c_u64_p]),
     "ps_test_welch": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
                                      ctypes.c_int, ctypes.c_int, ctypes.c_double, c_u64_p]),
+    "ps_minp_chi2": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
+                                    ctypes.c_int, ctypes.c_int, ctypes.c_void_p]),
+    "ps_minp_welch": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
+                                     ctypes.c_int, ctypes.c_int, ctypes.c_void_p]),
     "ps_select_top": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_uint64, c_u64_p]),
     "ps_fetch_survivors": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_size_t] + [ctypes.c_void_p] * 9),
     "ps_lookup": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_size_t,
@@ -250,6 +254,31 @@ class Context:
         self._ck(self.L.ps_test_welch(self.h, ph.shape[0], _ptr(ph), _ptr(w), int(min_samples),
                                       int(max_samples), float(p_threshold), ctypes.byref(ns)))
         return ns.value
+
+    def minp_chi2(self, pheno, weights, min_samples, max_samples):
+        """Smallest p per column over the union k-mers that pass the sample filter (1.0 if none).
+        pheno: C x N int8 (1/0/-1=NA), typically permuted columns; weights: N float64 or None. -> C float64."""
+        ph = np.ascontiguousarray(pheno, dtype=np.int8)
+        if ph.ndim == 1:
+            ph = ph[None, :]
+        assert ph.shape[1] == self.n_samples
+        w = None if weights is None else np.ascontiguousarray(weights, dtype=np.float64)
+        out = np.empty(ph.shape[0], dtype=np.float64)
+        self._ck(self.L.ps_minp_chi2(self.h, ph.shape[0], _ptr(ph), _ptr(w), int(min_samples), int(max_samples),
+                                     _ptr(out)))
+        return out
+
+    def minp_welch(self, pheno, weights, min_samples, max_samples):
+        """As minp_chi2 for the Welch test. pheno: C x N float64, NaN = NA."""
+        ph = np.ascontiguousarray(pheno, dtype=np.float64)
+        if ph.ndim == 1:
+            ph = ph[None, :]
+        assert ph.shape[1] == self.n_samples
+        w = None if weights is None else np.ascontiguousarray(weights, dtype=np.float64)
+        out = np.empty(ph.shape[0], dtype=np.float64)
+        self._ck(self.L.ps_minp_welch(self.h, ph.shape[0], _ptr(ph), _ptr(w), int(min_samples), int(max_samples),
+                                      _ptr(out)))
+        return out
 
     def select_top(self, n_pheno, n_top):
         n = ctypes.c_uint64()

@@ -976,18 +976,19 @@ static void row_mapping(const ps_ctx *c, int &wq, int &lpr_log2, int &qpl) {
     qpl = ceil_div(wq, 1 << lpr_log2);
 }
 
-template <bool WEIGHTED>
+template <bool WEIGHTED, class Out>
 static void launch_chi2(ps_ctx *c, int qpl, int grid, const uint4 *m, int wq, int lpr_log2, int P,
                         const uint32_t *masks, const double *totw, const int *totn, const double *w,
-                        const double *wtot, int mn, int mx, double thr, SurvOut o) {
+                        const double *wtot, int mn, int mx, double thr, Out o) {
     const double bytes = (double)c->U * c->row_words * 4;
-    const char *nm = WEIGHTED ? "test_chi2_w" : "test_chi2";
+    const bool minp = std::is_same<Out, MinpOut>::value;
+    const char *nm = WEIGHTED ? (minp ? "minp_chi2_w" : "test_chi2_w") : (minp ? "minp_chi2" : "test_chi2");
     // the column masks go to shared memory when they fit the default 48 KB
     const size_t mask_bytes = (size_t)P * 2 * c->row_words * 4;
     const int sm = mask_bytes <= 40 * 1024 ? 1 : 0;
     const size_t dyn = sm ? mask_bytes : 0;
     const int N = c->n_samples;
-#define PS_CHI2(Q) KLAUNCH(c, nm, bytes, (k_test_chi2<WEIGHTED, Q><<<grid, 256, dyn, c->stream>>>(m, c->U, wq, lpr_log2, P, N, masks, totw, totn, w, wtot, mn, mx, thr, sm, o)))
+#define PS_CHI2(Q) KLAUNCH(c, nm, bytes, (k_test_chi2<WEIGHTED, Q, Out><<<grid, 256, dyn, c->stream>>>(m, c->U, wq, lpr_log2, P, N, masks, totw, totn, w, wtot, mn, mx, thr, sm, o)))
     if (qpl <= 1) PS_CHI2(1);
     else if (qpl <= 2) PS_CHI2(2);
     else if (qpl <= 4) PS_CHI2(4);
@@ -995,13 +996,15 @@ static void launch_chi2(ps_ctx *c, int qpl, int grid, const uint4 *m, int wq, in
 #undef PS_CHI2
 }
 
+template <class Out>
 static void launch_chi2_sp(ps_ctx *c, int grid, const uint4 *m, int wq, int lpr_log2, int P, bool no_na,
                            const ulonglong2 *e1, const ulonglong2 *e0, int npad, const int *tot1, const int *tot0,
-                           const int2 *reach, int np_lo, int np_hi, double thr, SurvOut o) {
+                           const int2 *reach, int np_lo, int np_hi, double thr, Out o) {
     const double bytes = (double)c->U * c->row_words * 4;
     const int N = c->n_samples;
+    const char *nm = std::is_same<Out, MinpOut>::value ? "minp_chi2" : "test_chi2";
     if (lpr_log2 < 5) {
-#define PS_CHI2SP(NN) KLAUNCH(c, "test_chi2", bytes, (k_test_chi2_sp<NN><<<grid, 256, 0, c->stream>>>(m, c->U, wq, lpr_log2, P, N, e1, e0, npad, tot1, tot0, reach, np_lo, np_hi, thr, o)))
+#define PS_CHI2SP(NN) KLAUNCH(c, nm, bytes, (k_test_chi2_sp<NN, Out><<<grid, 256, 0, c->stream>>>(m, c->U, wq, lpr_log2, P, N, e1, e0, npad, tot1, tot0, reach, np_lo, np_hi, thr, o)))
         if (no_na) PS_CHI2SP(true); else PS_CHI2SP(false);
 #undef PS_CHI2SP
         return;
@@ -1009,7 +1012,7 @@ static void launch_chi2_sp(ps_ctx *c, int grid, const uint4 *m, int wq, int lpr_
     // rows that fill the warp: one instance per number of 32-bit words a lane owns (3..8 for 2,048 < N <= 8,190)
     const uint32_t *mw = reinterpret_cast<const uint32_t *>(m);
     const int kw = ceil_div(ceil_div(N, 32), 32), wp = c->row_words;
-#define PS_CHI2SPW(K, NN) KLAUNCH(c, "test_chi2", bytes, (k_test_chi2_sp_warp<K, NN><<<grid, 256, 0, c->stream>>>(mw, c->U, wp, P, N, e1, e0, npad, tot1, tot0, reach, np_lo, np_hi, thr, o)))
+#define PS_CHI2SPW(K, NN) KLAUNCH(c, nm, bytes, (k_test_chi2_sp_warp<K, NN, Out><<<grid, 256, 0, c->stream>>>(mw, c->U, wp, P, N, e1, e0, npad, tot1, tot0, reach, np_lo, np_hi, thr, o)))
 #define PS_CHI2SPW_K(K) case K: if (no_na) PS_CHI2SPW(K, true); else PS_CHI2SPW(K, false); break
     switch (kw) {
         PS_CHI2SPW_K(3); PS_CHI2SPW_K(4); PS_CHI2SPW_K(5); PS_CHI2SPW_K(6); PS_CHI2SPW_K(7); PS_CHI2SPW_K(8);
@@ -1019,9 +1022,10 @@ static void launch_chi2_sp(ps_ctx *c, int grid, const uint4 *m, int wq, int lpr_
 #undef PS_CHI2SPW
 }
 
+template <class Out>
 static void launch_welch(ps_ctx *c, int qpl, int grid, const uint4 *m, int wq, int lpr_log2, int P, int N,
                          const uint32_t *nonna, const double *vals, const double *w, const double *tot,
-                         const int *totn, int mn, int mx, double thr, SurvOut o) {
+                         const int *totn, int mn, int mx, double thr, Out o) {
     // normal quantile of the threshold: erfc(t_min / sqrt 2) = thr (bisection; thr >= 1: no screen)
     double t_min = 0.0;
     if (thr < 1.0) {
@@ -1034,14 +1038,15 @@ static void launch_welch(ps_ctx *c, int qpl, int grid, const uint4 *m, int wq, i
         t_min = lo * (1.0 - 1e-9);          // stay on the safe side of rounding
     }
     const double bytes = (double)c->U * c->row_words * 4;
+    const char *nm = std::is_same<Out, MinpOut>::value ? "minp_welch" : "test_welch";
     if (qpl <= 1)
-        KLAUNCH(c, "test_welch", bytes, (k_test_welch<1><<<grid, 256, 0, c->stream>>>(m, c->U, wq, lpr_log2, P, N, nonna, vals, w, tot, totn, mn, mx, thr, t_min, o)));
+        KLAUNCH(c, nm, bytes, (k_test_welch<1, Out><<<grid, 256, 0, c->stream>>>(m, c->U, wq, lpr_log2, P, N, nonna, vals, w, tot, totn, mn, mx, thr, t_min, o)));
     else if (qpl <= 2)
-        KLAUNCH(c, "test_welch", bytes, (k_test_welch<2><<<grid, 256, 0, c->stream>>>(m, c->U, wq, lpr_log2, P, N, nonna, vals, w, tot, totn, mn, mx, thr, t_min, o)));
+        KLAUNCH(c, nm, bytes, (k_test_welch<2, Out><<<grid, 256, 0, c->stream>>>(m, c->U, wq, lpr_log2, P, N, nonna, vals, w, tot, totn, mn, mx, thr, t_min, o)));
     else if (qpl <= 4)
-        KLAUNCH(c, "test_welch", bytes, (k_test_welch<4><<<grid, 256, 0, c->stream>>>(m, c->U, wq, lpr_log2, P, N, nonna, vals, w, tot, totn, mn, mx, thr, t_min, o)));
+        KLAUNCH(c, nm, bytes, (k_test_welch<4, Out><<<grid, 256, 0, c->stream>>>(m, c->U, wq, lpr_log2, P, N, nonna, vals, w, tot, totn, mn, mx, thr, t_min, o)));
     else
-        KLAUNCH(c, "test_welch", bytes, (k_test_welch<16><<<grid, 256, 0, c->stream>>>(m, c->U, wq, lpr_log2, P, N, nonna, vals, w, tot, totn, mn, mx, thr, t_min, o)));
+        KLAUNCH(c, nm, bytes, (k_test_welch<16, Out><<<grid, 256, 0, c->stream>>>(m, c->U, wq, lpr_log2, P, N, nonna, vals, w, tot, totn, mn, mx, thr, t_min, o)));
 }
 
 extern "C" {
@@ -1393,11 +1398,13 @@ int ps_restrict_union(ps_ctx *c, const uint64_t *db_kmers, size_t n_db, uint64_t
     API_END(c)
 }
 
-int ps_test_chi2(ps_ctx *c, int P, const int8_t *pheno, const double *weights, int min_samples, int max_samples,
-                 double thr, uint64_t *n_survivors) {
-    API_BEGIN(c)
-    if (!c->have_union) PS_THROW(PS_ERR_STATE, "ps_build_union first");
-    if (P < 1 || !pheno) PS_THROW(PS_ERR_ARG, "bad phenotype table");
+}  // extern "C"
+
+// One pass of the chi2 kernels over the matrix for P columns. minp == nullptr: the survivors (p < thr) are
+// compacted, they replace those of the previous test. Otherwise the min-p epilogue lowers minp[0..P) (device,
+// bit patterns of p) and the survivors of the previous test stay as they are.
+static void chi2_pass(ps_ctx *c, int P, const int8_t *pheno, const double *weights, int min_samples, int max_samples,
+                      double thr, unsigned long long *minp, uint64_t *n_survivors) {
     const int N = c->n_samples, wp = c->row_words;
     std::vector<uint32_t> masks((size_t)P * 2 * wp, 0);
     std::vector<double> totw((size_t)P * 2, 0.0), wtot((size_t)P * 2 * wp, 0.0);
@@ -1477,11 +1484,21 @@ int ps_test_chi2(ps_ctx *c, int P, const int8_t *pheno, const double *weights, i
         d_reach = dr;
     }
     CK(cudaStreamSynchronize(c->stream));  // host vectors above go out of scope
-    c->surv_welch = false;
-    c->n_surv = 0;
-    if (c->U == 0) { if (n_survivors) *n_survivors = 0; return PS_OK; }
     int wq, lpr_log2, qpl;
     row_mapping(c, wq, lpr_log2, qpl);
+    if (minp) {
+        if (qpl > 16) PS_THROW(PS_ERR_ARG, "too many samples for the test kernel (max 65535)");
+        if (c->U == 0) return;
+        const MinpOut o{minp};
+        const int grid = PS_SMS * 8;
+        if (weights) launch_chi2<true>(c, qpl, grid, c->matrix.as<uint4>(), wq, lpr_log2, P, c->ph_masks.as<uint32_t>(), d_totw, d_totn, d_w, c->ph_vals.as<double>(), min_samples, max_samples, thr, o);
+        else if (sparse_walk) launch_chi2_sp(c, grid, c->matrix.as<uint4>(), wq, lpr_log2, P, no_na, d_e1, d_e0, wp * 32, d_tot1, d_tot0, d_reach, np_lo, np_hi, thr, o);
+        else launch_chi2<false>(c, qpl, grid, c->matrix.as<uint4>(), wq, lpr_log2, P, c->ph_masks.as<uint32_t>(), d_totw, d_totn, d_w, c->ph_vals.as<double>(), min_samples, max_samples, thr, o);
+        return;
+    }
+    c->surv_welch = false;
+    c->n_surv = 0;
+    if (c->U == 0) { if (n_survivors) *n_survivors = 0; return; }
     if (qpl > 16) PS_THROW(PS_ERR_ARG, "too many samples for the test kernel (max 65535)");
     uint64_t cap = std::max<uint64_t>(c->sv_ph.cap / 4, 1u << 16);
     const int grid = PS_SMS * 8;
@@ -1498,14 +1515,11 @@ int ps_test_chi2(ps_ctx *c, int P, const int8_t *pheno, const double *weights, i
         cap = ns;
     }
     if (n_survivors) *n_survivors = c->n_surv;
-    API_END(c)
 }
 
-int ps_test_welch(ps_ctx *c, int P, const double *pheno, const double *weights, int min_samples, int max_samples,
-                  double thr, uint64_t *n_survivors) {
-    API_BEGIN(c)
-    if (!c->have_union) PS_THROW(PS_ERR_STATE, "ps_build_union first");
-    if (P < 1 || !pheno) PS_THROW(PS_ERR_ARG, "bad phenotype table");
+// ps_test_welch / ps_minp_welch: one pass of k_test_welch over the matrix, as chi2_pass.
+static void welch_pass(ps_ctx *c, int P, const double *pheno, const double *weights, int min_samples, int max_samples,
+                       double thr, unsigned long long *minp, uint64_t *n_survivors) {
     const int N = c->n_samples, wp = c->row_words;
     const int Npad = wp * 32;
     std::vector<uint32_t> nonna((size_t)P * wp, 0);
@@ -1550,11 +1564,18 @@ int ps_test_welch(ps_ctx *c, int P, const double *pheno, const double *weights, 
         d_w = c->weights.as<double>();
     }
     CK(cudaStreamSynchronize(c->stream));
-    c->surv_welch = true;
-    c->n_surv = 0;
-    if (c->U == 0) { if (n_survivors) *n_survivors = 0; return PS_OK; }
     int wq, lpr_log2, qpl;
     row_mapping(c, wq, lpr_log2, qpl);
+    if (minp) {
+        if (qpl > 16) PS_THROW(PS_ERR_ARG, "too many samples for the test kernel (max 65535)");
+        if (c->U == 0) return;
+        launch_welch(c, qpl, PS_SMS * 8, c->matrix.as<uint4>(), wq, lpr_log2, P, Npad, c->ph_masks.as<uint32_t>(),
+                     c->ph_vals.as<double>(), d_w, d_tot, d_totn, min_samples, max_samples, thr, MinpOut{minp});
+        return;
+    }
+    c->surv_welch = true;
+    c->n_surv = 0;
+    if (c->U == 0) { if (n_survivors) *n_survivors = 0; return; }
     if (qpl > 16) PS_THROW(PS_ERR_ARG, "too many samples for the test kernel (max 65535)");
     uint64_t cap = std::max<uint64_t>(c->sv_ph.cap / 4, 1u << 16);
     const int grid = PS_SMS * 8;
@@ -1570,6 +1591,69 @@ int ps_test_welch(ps_ctx *c, int P, const double *pheno, const double *weights, 
         cap = ns;
     }
     if (n_survivors) *n_survivors = c->n_surv;
+}
+
+// ps_minp_*: the columns in batches whose masks fit the shared-memory staging of k_test_chi2 (40 KB; whole
+// groups of CHI2_SP_COLS for the bit walk), one pass over the matrix per batch, thr = 1 (no screen prunes a row).
+template <class T, class Pass>
+static void minp_batches(ps_ctx *c, int n_cols, const T *pheno, double *minp, Pass pass) {
+    const int N = c->n_samples;
+    int bs = std::max(1, (int)((40 * 1024) / ((size_t)2 * c->row_words * 4)));
+    if (bs >= CHI2_SP_COLS) bs -= bs % CHI2_SP_COLS;
+    c->ph_minp.reserve((size_t)n_cols * 8, c->stream);
+    unsigned long long *d = c->ph_minp.as<unsigned long long>();
+    std::vector<unsigned long long> one((size_t)n_cols);
+    const double v1 = 1.0;
+    unsigned long long b1;
+    memcpy(&b1, &v1, 8);
+    std::fill(one.begin(), one.end(), b1);
+    CK(cudaMemcpyAsync(d, one.data(), one.size() * 8, cudaMemcpyHostToDevice, c->stream));
+    for (int c0 = 0; c0 < n_cols; c0 += bs)
+        pass(std::min(bs, n_cols - c0), pheno + (size_t)c0 * N, d + c0);
+    CK(cudaMemcpyAsync(one.data(), d, one.size() * 8, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    memcpy(minp, one.data(), one.size() * 8);
+}
+
+extern "C" {
+
+int ps_test_chi2(ps_ctx *c, int P, const int8_t *pheno, const double *weights, int min_samples, int max_samples,
+                 double thr, uint64_t *n_survivors) {
+    API_BEGIN(c)
+    if (!c->have_union) PS_THROW(PS_ERR_STATE, "ps_build_union first");
+    if (P < 1 || !pheno) PS_THROW(PS_ERR_ARG, "bad phenotype table");
+    chi2_pass(c, P, pheno, weights, min_samples, max_samples, thr, nullptr, n_survivors);
+    API_END(c)
+}
+
+int ps_test_welch(ps_ctx *c, int P, const double *pheno, const double *weights, int min_samples, int max_samples,
+                  double thr, uint64_t *n_survivors) {
+    API_BEGIN(c)
+    if (!c->have_union) PS_THROW(PS_ERR_STATE, "ps_build_union first");
+    if (P < 1 || !pheno) PS_THROW(PS_ERR_ARG, "bad phenotype table");
+    welch_pass(c, P, pheno, weights, min_samples, max_samples, thr, nullptr, n_survivors);
+    API_END(c)
+}
+
+int ps_minp_chi2(ps_ctx *c, int n_cols, const int8_t *pheno, const double *weights, int min_samples, int max_samples,
+                 double *minp) {
+    API_BEGIN(c)
+    if (!c->have_union) PS_THROW(PS_ERR_STATE, "ps_build_union first");
+    if (n_cols < 1 || !pheno || !minp) PS_THROW(PS_ERR_ARG, "bad phenotype table");
+    minp_batches(c, n_cols, pheno, minp, [&](int P, const int8_t *ph, unsigned long long *d) {
+        chi2_pass(c, P, ph, weights, min_samples, max_samples, 1.0, d, nullptr);
+    });
+    API_END(c)
+}
+
+int ps_minp_welch(ps_ctx *c, int n_cols, const double *pheno, const double *weights, int min_samples, int max_samples,
+                  double *minp) {
+    API_BEGIN(c)
+    if (!c->have_union) PS_THROW(PS_ERR_STATE, "ps_build_union first");
+    if (n_cols < 1 || !pheno || !minp) PS_THROW(PS_ERR_ARG, "bad phenotype table");
+    minp_batches(c, n_cols, pheno, minp, [&](int P, const double *ph, unsigned long long *d) {
+        welch_pass(c, P, ph, weights, min_samples, max_samples, 1.0, d, nullptr);
+    });
     API_END(c)
 }
 

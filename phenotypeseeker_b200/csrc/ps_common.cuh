@@ -168,6 +168,7 @@ struct ps_ctx {
     DevBuf keys_a, keys_b, tags_a, tags_b, hist, lookback;  // sort
     DevBuf uni, matrix;                                     // union + matrix
     DevBuf ph_masks, ph_vals, ph_tot, weights;              // phenotypes
+    DevBuf ph_minp;                                         // ps_minp_*: per-column minima (bit patterns)
     DevBuf sv_ph, sv_row, sv_stat, sv_p, sv_mx, sv_my, sv_n, sv_perm, sv_bits, sv_kmer;
     DevBuf sel_ph, sel_row, sel_stat, sel_p, sel_mx, sel_my, sel_n;   // ps_select_top
     DevBuf tmp1, tmp2, tmp3;
@@ -188,7 +189,7 @@ struct ps_ctx {
         return {&staging, &tile_tab, &tile_sum, &file_tab, &pool_seq, &pool_bad, &list_keys,
                 &list_counts, &samp_tab, &blk_counts, &blk_offs, &scalars, &scan_sums, &keys_a, &keys_b,
                 &tags_a, &tags_b, &hist, &lookback, &uni, &matrix, &ph_masks, &ph_vals, &ph_tot,
-                &weights, &sv_ph, &sv_row, &sv_stat, &sv_p, &sv_mx, &sv_my, &sv_n, &sv_perm,
+                &ph_minp, &weights, &sv_ph, &sv_row, &sv_stat, &sv_p, &sv_mx, &sv_my, &sv_n, &sv_perm,
                 &sv_bits, &sv_kmer, &tmp1, &tmp2, &tmp3, &pg_meta_a, &pg_meta_b, &pg_tiles,
                 &pg_tabs, &pg_state, &pg_blist, &sel_ph, &sel_row, &sel_stat, &sel_p, &sel_mx, &sel_my, &sel_n,
                 &mash_tab, &mash_parts, &mash_parts_n, &mash_h, &mash_n, &mash_sd, &nj_d, &nj_d2, &nj_act, &nj_nd,

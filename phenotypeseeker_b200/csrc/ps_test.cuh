@@ -22,6 +22,7 @@
 // p = 2*t.sf(|t|, dof) = I_{dof/(dof+t^2)}(dof/2, 1/2) (regularised incomplete beta, FP64
 // continued fraction).
 #pragma once
+#include <type_traits>
 #include "ps_common.cuh"
 
 struct SurvOut {
@@ -42,6 +43,27 @@ __device__ __forceinline__ void surv_push(const SurvOut &o, int ph, unsigned lon
     }
 }
 
+// The min-p epilogue (ps_minp_*, permutation thresholds): the test kernels are instantiated with this in place of
+// SurvOut. Nothing is compacted; every (row, column) pair that passes the sample filter and has a p (not NaN)
+// offers it to minp[column], the bit pattern of the smallest p so far (1.0 before the pass). p >= 0, so the
+// IEEE pattern orders like the value and one integer atomicMin keeps the minimum.
+struct MinpOut {
+    unsigned long long *minp;
+};
+
+template <class Out>
+__device__ __forceinline__ constexpr bool is_minp() { return std::is_same<Out, MinpOut>::value; }
+
+// The lanes lane ^ step, lane ^ 2 step, ... ^ 16 hold the same column; their smallest candidate goes to memory with
+// one atomicMin from the owner lane, and only when it is below the value read there (a stale read is higher, never
+// lower, so no minimum is lost). Called by all 32 lanes; cand = 1.0 offers nothing.
+__device__ __forceinline__ void minp_offer(const MinpOut &o, int ph, bool owner, double cand, int step) {
+    if (!__any_sync(0xffffffffu, cand < 1.0)) return;
+    unsigned long long b = (unsigned long long)__double_as_longlong(cand);
+    for (int s = step; s < 32; s <<= 1) b = min(b, __shfl_xor_sync(0xffffffffu, b, s));
+    if (owner && b < __ldcg(o.minp + ph)) atomicMin(o.minp + ph, b);
+}
+
 __device__ __forceinline__ uint32_t u4_get(const uint4 &v, int j) {
     return j == 0 ? v.x : j == 1 ? v.y : j == 2 ? v.z : v.w;
 }
@@ -57,12 +79,13 @@ __device__ __forceinline__ uint32_t u4_get(const uint4 &v, int j) {
 // row occupies a whole warp and ten columns are finished by ten lanes in parallel instead of one after
 // the other on lane 0. Column masks are staged in shared memory (smem_masks != 0); a column without NA
 // samples needs one popcount per word instead of two (absent-with-phenotype = popcount(row) - present).
-template <bool WEIGHTED, int QPL>
+// Out = SurvOut compacts the survivors (p < thr); Out = MinpOut keeps each column's smallest p (ps_minp_chi2).
+template <bool WEIGHTED, int QPL, class Out = SurvOut>
 __global__ void __launch_bounds__(256)
 k_test_chi2(const uint4 *__restrict__ matrix, unsigned long long U, int wq, int lpr_log2, int P, int n_samples,
             const uint32_t *__restrict__ masks, const double *__restrict__ totw,
             const int *__restrict__ totn, const double *__restrict__ weights,
-            const double *__restrict__ wtot, int min_s, int max_s, double thr, int smem_masks, SurvOut out) {
+            const double *__restrict__ wtot, int min_s, int max_s, double thr, int smem_masks, Out out) {
     extern __shared__ uint32_t s_masks[];
     const int lpr = 1 << lpr_log2;
     const unsigned lane = threadIdx.x & 31;
@@ -169,8 +192,11 @@ k_test_chi2(const uint4 *__restrict__ matrix, unsigned long long U, int wq, int 
                 }
                 if ((int)sub == j) { my_ai = ai; my_ci = ci; my_a = a; my_c = c; }
             }
-            // every lane finishes its own column
+            // every lane finishes its own column; a `continue` inside the do-while(0) leaves the finish only, so
+            // that the min-p epilogue after it is reached by the whole warp
             const int ph = p0 + (int)sub;
+            double cand = 1.0;
+            do {
             if (ph >= P || !rvalid) continue;
             const uint32_t n_with = my_ai + my_ci;
             const int n_without = totn[ph] - (int)n_with;
@@ -194,7 +220,11 @@ k_test_chi2(const uint4 *__restrict__ matrix, unsigned long long U, int wq, int 
             const double tc = (c - ec) * (c - ec) / ec, td = (d - ed) * (d - ed) / ed;
             const double chi2 = ((ta + tb) + tc) + td;
             const double p = exp(-0.5 * chi2);
-            if (p < thr) surv_push(out, ph, r, chi2, p, 0.0, 0.0, n_with);  // NaN compares false
+            if constexpr (is_minp<Out>()) { if (p < cand) cand = p; }
+            else if (p < thr) surv_push(out, ph, r, chi2, p, 0.0, 0.0, n_with);  // NaN compares false
+            } while (0);
+            // lanes sub, sub + lpr, ... hold column ph; lane sub of the first row group offers their minimum
+            if constexpr (is_minp<Out>()) minp_offer(out, ph, (int)lane < lpr && ph < P, cand, lpr);
         }
     }
 }
@@ -229,12 +259,12 @@ __device__ __forceinline__ uint32_t pick_reg(const uint32_t (&v)[K], int i) {   
 // Lane j of the row group finishes column ph from its summed fields: fa = number of walked samples with phenotype
 // 1 in that column, fb = with phenotype 0 (the walked samples are the cleared ones of a dense row). A count
 // outside reach[ph] fails the sample filter or the screen below; from the counts on, the arithmetic is that of
-// k_test_chi2 (unweighted), operation for operation.
-template <bool NO_NA>
+// k_test_chi2 (unweighted), operation for operation. With MinpOut the p lowers cand instead of being pushed.
+template <bool NO_NA, class Out>
 __device__ __forceinline__ void chi2_sp_finish(int ph, unsigned long long r, uint32_t fa, uint32_t fb, uint32_t np,
                                                bool dense, const int *__restrict__ tot1, const int *__restrict__ tot0,
                                                const int2 *__restrict__ reach, double chi2_min, double thr,
-                                               const SurvOut &out) {
+                                               const Out &out, double &cand) {
     const uint32_t ai = dense ? (uint32_t)tot1[ph] - fa : fa;
     const uint32_t ci = NO_NA ? np - ai : dense ? (uint32_t)tot0[ph] - fb : fb;
     const uint32_t n_with = ai + ci;
@@ -255,17 +285,18 @@ __device__ __forceinline__ void chi2_sp_finish(int ph, unsigned long long r, uin
     const double tc = (c - ec) * (c - ec) / ec, td = (d - ed) * (d - ed) / ed;
     const double chi2 = ((ta + tb) + tc) + td;
     const double p = exp(-0.5 * chi2);
-    if (p < thr) surv_push(out, ph, r, chi2, p, 0.0, 0.0, n_with);  // NaN compares false
+    if constexpr (is_minp<Out>()) { if (p < cand) cand = p; }
+    else if (p < thr) surv_push(out, ph, r, chi2, p, 0.0, 0.0, n_with);  // NaN compares false
 }
 
 // Rows of at most 16 uint4 (N <= 2,048): LPR = pow2 >= wq lanes per row, one uint4 per lane, fields summed with
 // xor-shuffles inside the group.
-template <bool NO_NA>
+template <bool NO_NA, class Out = SurvOut>
 __global__ void __launch_bounds__(256, 3)
 k_test_chi2_sp(const uint4 *__restrict__ matrix, unsigned long long U, int wq, int lpr_log2, int P, int n_samples,
                const ulonglong2 *__restrict__ e1, const ulonglong2 *__restrict__ e0, int npad,
                const int *__restrict__ tot1, const int *__restrict__ tot0, const int2 *__restrict__ reach,
-               int np_lo, int np_hi, double thr, SurvOut out) {
+               int np_lo, int np_hi, double thr, Out out) {
     const int lpr = 1 << lpr_log2;
     const unsigned lane = threadIdx.x & 31;
     const unsigned sub = lane & (lpr - 1);
@@ -316,13 +347,30 @@ k_test_chi2_sp(const uint4 *__restrict__ matrix, unsigned long long U, int wq, i
                 a1 += __shfl_xor_sync(0xffffffffu, a1, o);
                 if (!NO_NA) { b0 += __shfl_xor_sync(0xffffffffu, b0, o); b1 += __shfl_xor_sync(0xffffffffu, b1, o); }
             }
+            // lane j of the group finishes columns c0 + j, c0 + j + lpr, ... (min-p: in steps the whole warp takes,
+            // each followed by the offer of the lanes that hold the same column)
+            if constexpr (is_minp<Out>()) {
+                for (int j0 = 0; j0 < CHI2_SP_COLS; j0 += lpr) {
+                    const int j = j0 + (int)sub;
+                    const bool mine = j < CHI2_SP_COLS && c0 + j < P;
+                    double cand = 1.0;
+                    if (live && mine) {
+                        const int sh = 12 * (j % 5);
+                        const uint32_t fa = (uint32_t)(((j < 5 ? a0 : a1) >> sh) & 4095ull);
+                        const uint32_t fb = NO_NA ? 0u : (uint32_t)(((j < 5 ? b0 : b1) >> sh) & 4095ull);
+                        chi2_sp_finish<NO_NA>(c0 + j, r, fa, fb, np, dense, tot1, tot0, reach, chi2_min, thr, out, cand);
+                    }
+                    minp_offer(out, c0 + j, (int)lane < lpr && mine, cand, lpr);
+                }
+                continue;
+            }
             if (!live) continue;
-            // lane j of the group finishes columns c0 + j, c0 + j + lpr, ...
+            double unused = 1.0;
             for (int j = (int)sub; j < CHI2_SP_COLS && c0 + j < P; j += lpr) {
                 const int sh = 12 * (j % 5);
                 const uint32_t fa = (uint32_t)(((j < 5 ? a0 : a1) >> sh) & 4095ull);
                 const uint32_t fb = NO_NA ? 0u : (uint32_t)(((j < 5 ? b0 : b1) >> sh) & 4095ull);
-                chi2_sp_finish<NO_NA>(c0 + j, r, fa, fb, np, dense, tot1, tot0, reach, chi2_min, thr, out);
+                chi2_sp_finish<NO_NA>(c0 + j, r, fa, fb, np, dense, tot1, tot0, reach, chi2_min, thr, out, unused);
             }
         }
     }
@@ -347,12 +395,12 @@ __device__ __forceinline__ void fields16(unsigned long long x0, unsigned long lo
 // word is empty it takes the next non-empty one — so the warp runs max over lanes of the lane's bit count, not
 // the sum over words of the per-word maxima. The fields are summed over the warp by REDUX (five u32 of two 16-bit
 // fields) instead of twenty shuffles and adds; every lane gets every sum and lane j finishes column c0 + j.
-template <int KW, bool NO_NA>
+template <int KW, bool NO_NA, class Out = SurvOut>
 __global__ void __launch_bounds__(256, 3)
 k_test_chi2_sp_warp(const uint32_t *__restrict__ matrix, unsigned long long U, int wp, int P, int n_samples,
                     const ulonglong2 *__restrict__ e1, const ulonglong2 *__restrict__ e0, int npad,
                     const int *__restrict__ tot1, const int *__restrict__ tot0, const int2 *__restrict__ reach,
-                    int np_lo, int np_hi, double thr, SurvOut out) {
+                    int np_lo, int np_hi, double thr, Out out) {
     __shared__ uint32_t s_valid[KW * 32];    // s_valid[wi]: the bits of row word wi that are samples
     const int lane = (int)(threadIdx.x & 31);
     const int wv = (n_samples + 31) >> 5;
@@ -414,12 +462,16 @@ k_test_chi2_sp_warp(const uint32_t *__restrict__ matrix, unsigned long long U, i
             uint32_t fa[5], fb[5];
             fields16(a0, a1, fa);
             if (!NO_NA) fields16(b0, b1, fb);
-            if (lane < CHI2_SP_COLS && c0 + lane < P) {
+            const bool mine = lane < CHI2_SP_COLS && c0 + lane < P;
+            double cand = 1.0;
+            if (mine) {
                 const int sh = 16 * (lane & 1);
                 const uint32_t ca = (pick_reg(fa, lane >> 1) >> sh) & 0xFFFFu;
                 const uint32_t cb = NO_NA ? 0u : (pick_reg(fb, lane >> 1) >> sh) & 0xFFFFu;
-                chi2_sp_finish<NO_NA>(c0 + lane, r, ca, cb, np, dense, tot1, tot0, reach, chi2_min, thr, out);
+                chi2_sp_finish<NO_NA>(c0 + lane, r, ca, cb, np, dense, tot1, tot0, reach, chi2_min, thr, out, cand);
             }
+            // one row per warp: lane j alone holds column c0 + j
+            if constexpr (is_minp<Out>()) minp_offer(out, c0 + lane, mine, cand, 32);
         }
     }
 }
@@ -497,12 +549,12 @@ __device__ __forceinline__ void welch_direct_group(const uint32_t *__restrict__ 
     var = q / a;
 }
 
-template <int QPL>
+template <int QPL, class Out = SurvOut>
 __global__ void __launch_bounds__(256)
 k_test_welch(const uint4 *__restrict__ matrix, unsigned long long U, int wq, int lpr_log2, int P, int N,
              const uint32_t *__restrict__ nonna, const double *__restrict__ vals,
              const double *__restrict__ weights, const double *__restrict__ tot, const int *__restrict__ totn,
-             int min_s, int max_s, double thr, double t_min, SurvOut out) {
+             int min_s, int max_s, double thr, double t_min, Out out) {
     const int lpr = 1 << lpr_log2;
     const unsigned lane = threadIdx.x & 31;
     const unsigned sub = lane & (lpr - 1);
@@ -595,6 +647,10 @@ k_test_welch(const uint4 *__restrict__ matrix, unsigned long long U, int wq, int
             }
             for (int o = lpr >> 1; o > 0; o >>= 1) qs += __shfl_xor_sync(0xffffffffu, qs, o);
             if (!exact2) qs = qs1;
+            // lane 0 of each row group finishes the row; a `continue` inside the do-while(0) leaves the finish
+            // only, so that the min-p epilogue after it is reached by the whole warp
+            double cand = 1.0;
+            do {
             if (sub != 0 || !tested) continue;
             const double Tw = tot[ph * 4], Twv = tot[ph * 4 + 1], Twvv = tot[ph * 4 + 2], mu = tot[ph * 4 + 3];
             const double var_s = qs / sw;
@@ -619,7 +675,11 @@ k_test_welch(const uint4 *__restrict__ matrix, unsigned long long U, int wq, int
             if (fabs(t) < t_min) continue;
             const double dof = 1.0 / (r1 * r1 / (n1 - 1.0) + r2 * r2 / (n2 - 1.0));
             const double p = ps_t_two_sided(t, dof);
-            if (p < thr) surv_push(out, ph, r, t, p, mu + m1c, mu + m2c, nx);
+            if constexpr (is_minp<Out>()) { if (p < cand) cand = p; }
+            else if (p < thr) surv_push(out, ph, r, t, p, mu + m1c, mu + m2c, nx);
+            } while (0);
+            // lanes 0, lpr, 2 lpr, ... hold column ph for their rows; lane 0 offers the minimum
+            if constexpr (is_minp<Out>()) minp_offer(out, ph, lane == 0, cand, lpr);
         }
     }
 }

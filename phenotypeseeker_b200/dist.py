@@ -250,7 +250,8 @@ def gather_results(parts, rank, world, device, dist, top_k=None, p_exact=None):
     header = passes x (U_local, payload bytes, survivors per column). Every rank sees every header, so
     all ranks agree when the capacity has to grow (then, and only then, a second round). Ranges ascend
     pass-major, then by rank: that is the order of the merge and of the global row numbers.
-    p_exact: final threshold (passes test against a laxer one while U is still growing).
+    p_exact: final threshold, one for all columns or one per column (passes test against a laxer one while U is
+    still growing).
     -> merged list on rank 0, None elsewhere."""
     import torch
     from .pipeline import trim_top
@@ -294,9 +295,9 @@ def gather_results(parts, rank, world, device, dist, top_k=None, p_exact=None):
             bases.append(base)
             base += int(metas[r, j, 0])
     out = []
-    for r in merge_results(gathered, bases):
+    for j, r in enumerate(merge_results(gathered, bases)):
         if p_exact is not None:
-            r = r.take(r.p < p_exact)
+            r = r.take(r.p < (p_exact[j] if np.ndim(p_exact) else p_exact))
         out.append(trim_top(r, top_k))
     return out
 
@@ -460,6 +461,8 @@ def build_and_test(ka: KmerAssociation, n_samples, k, pheno, binary, weights, ra
     (--kmerDB): each range keeps only those (ps_restrict_union) and U counts what is left. passes: number of
     super-ranges of the "pages" route (None: as many as the pool budget needs). A page-pool overflow raises
     PoolOverflow after every rank has doubled its pools: running this step again (without a new ingest) retries.
+    n_perm > 0 (test_kw, with perm_seed): permutation thresholds (KmerAssociation.test); every pass min-reduces the
+    ranks' min-p of the permuted columns over their own k-mers, so thresholds and survivors are those of one build.
     Returns (U_total, results on rank 0 / None elsewhere, info)."""
     ctx = ka.ctx
     dist = TORCH_GROUP if group is None else group
@@ -471,6 +474,30 @@ def build_and_test(ka: KmerAssociation, n_samples, k, pheno, binary, weights, ra
         res = ka.test(pheno, binary, weights, **test_kw)
         return U, res, {"U_local": U, "nvlink_bytes": 0, "splitters": []}
     import torch
+    from .pipeline import permutation_thresholds
+
+    n_perm, perm_seed = int(test_kw.pop("n_perm", 0)), test_kw.pop("perm_seed", 0)
+    perm = n_perm > 0 and not (binary and test_kw.get("omit_b"))
+    P = np.asarray(pheno).reshape(n_samples, -1).shape[1]
+    minp = np.ones((P, n_perm)) if perm else None
+    alpha = float(test_kw.get("pvalue_cutoff", 0.05))
+    if perm:
+        permutation_thresholds(minp, alpha)          # too few permutations: raise before any build
+
+    def combine_minp(m_local):
+        """Element-wise minimum of every rank's min-p (an all-gather: the collectives have no min-reduce)."""
+        t = torch.from_numpy(np.ascontiguousarray(m_local, dtype=np.float64).reshape(-1)).to(device)
+        allt = torch.empty(world * t.numel(), dtype=torch.float64, device=device)
+        dist.all_gather_into_tensor(allt, t)
+        return np.minimum(minp, allt.cpu().numpy().reshape(world, P, n_perm).min(axis=0))
+
+    def test_pass(n_union_total):
+        nonlocal minp
+        if not perm:
+            return ka.test(pheno, binary, weights, n_union_total=n_union_total, **test_kw)
+        minp = combine_minp(ka.permutation_minp(pheno, binary, n_perm, weights, test_kw.get("min_samples", 2),
+                                                test_kw.get("max_samples"), perm_seed))
+        return ka.test(pheno, binary, weights, minp=minp, **test_kw)
 
     if route == "auto":
         route = "pages" if 9 <= int(k) <= 16 else "streams"
@@ -512,7 +539,7 @@ def build_and_test(ka: KmerAssociation, n_samples, k, pheno, binary, weights, ra
                                        "the next step will use pools twice as large")
                 # Bonferroni needs the total U: a pass tests against the union seen so far (a laxer threshold),
                 # the exact filter follows when every pass is done
-                parts.append((U_local, ka.test(pheno, binary, weights, n_union_total=U_seen if exact else None, **test_kw)))
+                parts.append((U_local, test_pass(U_seen if exact else None)))
                 mark(f"pass{j}")
             if pr.passes > 1:
                 ctx.set_range(0, 0)
@@ -533,11 +560,18 @@ def build_and_test(ka: KmerAssociation, n_samples, k, pheno, binary, weights, ra
             u = torch.tensor([U_local], dtype=torch.int64, device=device)
             dist.all_reduce(u)
             U_total = int(u[0].item())
-            parts.append((U_local, ka.test(pheno, binary, weights, n_union_total=U_total, **test_kw)))
+            parts.append((U_local, test_pass(U_total)))
             mark("test")
-        merged = gather_results(parts, rank, world, device, dist, top_k=test_kw.get("top_k"),
-                                p_exact=(float(test_kw.get("pvalue_cutoff", 0.05)) / U_total if U_total else 0.0)
-                                if not (binary and test_kw.get("omit_b")) else None)
+        if perm:
+            p_exact = permutation_thresholds(minp, alpha)
+        elif binary and test_kw.get("omit_b"):
+            p_exact = None
+        else:
+            p_exact = alpha / U_total if U_total else 0.0
+        merged = gather_results(parts, rank, world, device, dist, top_k=test_kw.get("top_k"), p_exact=p_exact)
+        if perm and merged is not None:
+            for j, r in enumerate(merged):
+                r.threshold, r.minp = float(p_exact[j]), minp[j]
         mark("gather")
     mark.report()
     return U_total, merged, {"U_local": sum(p[0] for p in parts), "nvlink_bytes": nvl_bytes, "splitters": spl, "route": route,

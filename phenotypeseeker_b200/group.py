@@ -91,17 +91,19 @@ class GpuGroup:
 
     # stages 2-3
     def test(self, pheno, binary, weights=None, min_samples=2, max_samples=None, pvalue_cutoff=0.05, omit_b=False,
-             pheno_names=None, top_k=None, restrict=None, passes=None):
+             pheno_names=None, top_k=None, restrict=None, passes=None, n_perm=0, perm_seed=0):
         """Build and test on every rank (dist.build_and_test) -> (U, [PhenoResult per phenotype column]), merged
         on rank 0: global rows and ascending k-mer order as in a single build. restrict: ascending database k-mers
         (--kmerDB), any number of passes. passes: super-ranges of the k-mer space (None: as the pool budget needs).
+        n_perm, perm_seed: permutation thresholds as KmerAssociation.test; each rank computes the min-p over its own
+        k-mers and the ranks' minima are min-reduced, so thresholds and survivors equal one GPU's.
         A page-pool overflow is retried once with the doubled pools; the samples are not ingested again."""
         import torch
         ph = np.asarray(pheno, dtype=np.float64)
         if ph.ndim == 1:
             ph = ph[:, None]
         kw = dict(min_samples=min_samples, max_samples=max_samples, pvalue_cutoff=pvalue_cutoff, omit_b=omit_b,
-                  pheno_names=pheno_names, top_k=top_k)
+                  pheno_names=pheno_names, top_k=top_k, n_perm=n_perm, perm_seed=perm_seed)
 
         def one(r):
             try:

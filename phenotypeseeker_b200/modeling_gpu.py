@@ -152,14 +152,32 @@ def pheno_matrix(samples, pheno_names):
     return out
 
 
+def permutation_options():
+    """PS_PERMUTATIONS=B (> 0): the permutation threshold of B phenotype permutations replaces the Bonferroni cut
+    (pvalue / U) of the tests; PS_PERMUTATION_SEED (default 0) seeds them. Unset or 0: the reference's rule, and
+    no keyword at all. -> keyword arguments of KmerAssociation.test / test_in_ranges / GpuGroup.test."""
+    n_perm = int(os.environ.get("PS_PERMUTATIONS", "0") or 0)
+    if n_perm <= 0:
+        return {}
+    return dict(n_perm=n_perm, perm_seed=int(os.environ.get("PS_PERMUTATION_SEED", "0") or 0))
+
+
+def threshold_log_line(res):
+    """The log.txt line of a column tested against a permutation threshold, None for the reference's rule."""
+    if getattr(res, "threshold", None) is None:
+        return None
+    return f"Permutation threshold for {res.name}: p < {res.threshold:.6E} ({len(res.minp)} permutations)\n"
+
+
 def run_hot_path(files, sample_names, k, cutoff, pheno, pheno_names, binary, weights, min_samples, max_samples,
                  pvalue_cutoff, omit_b, n_stripes, real_counts=False, device=None):
     """Stages 1-3 on the GPU -> (U, {pheno_name: ML_df}). Plain-data entry used by tests/standalone.
-    device: as PS_DEVICE (parse_devices); several entries run on a GpuGroup."""
+    device: as PS_DEVICE (parse_devices); several entries run on a GpuGroup. PS_PERMUTATIONS: see
+    permutation_options."""
     ka = _ka(device)
     ka.count(files, k, cutoff)
     kw = dict(min_samples=min_samples, max_samples=max_samples, pvalue_cutoff=pvalue_cutoff, omit_b=omit_b,
-              pheno_names=list(pheno_names))
+              pheno_names=list(pheno_names), **permutation_options())
     if ka.fits_in_one_build():
         U = ka.build()
         res = ka.test(pheno, binary, weights, **kw)
@@ -233,7 +251,7 @@ def install(m, device=None, native_weights=None):
         ph = pheno_matrix(samples, cols)
         w = np.array([float(s.weight) for s in samples])
         kw = dict(min_samples=Samples.min_samples, max_samples=Samples.max_samples, pvalue_cutoff=phenotypes.pvalue_cutoff,
-                  omit_b=bool(phenotypes.omit_B), pheno_names=cols)
+                  omit_b=bool(phenotypes.omit_B), pheno_names=cols, **permutation_options())
         if _STATE["ranges"] > 1:
             _, res = ka.test_in_ranges(ph, binary, _STATE["ranges"], w, n_instances=ka.instances_upper(),
                                        restrict=_STATE["db"], **kw)
@@ -269,6 +287,8 @@ def install(m, device=None, native_weights=None):
             write_legacy_outputs(self.ML_df, self.name, binary)
         with open("log.txt", "a") as log:       # the reference's `timer` line (modeling.py:54-61)
             log.write(f"Func {test_kmers_association_with_phenotype} took {time.time() - start} secs\n")
+            if threshold_log_line(res):
+                log.write(threshold_log_line(res))
 
     def get_mash_sketches(self):       # runs in Pool workers: sketching happens in get_weights
         return None

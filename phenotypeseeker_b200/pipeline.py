@@ -5,7 +5,9 @@ Mirrors the stage order and the keep rules of `modeling.modeling()` lines 1644-1
 Everything numeric happens on the GPU; this module only shapes inputs and outputs.
 """
 import gzip
+import math
 import os
+from fractions import Fraction
 
 import numpy as np
 
@@ -91,6 +93,8 @@ class PhenoResult:
                 rowbits.view(np.uint8).reshape(rowbits.shape[0], -1)[:, :pk.shape[1]] = pk
         self.rowbits = np.ascontiguousarray(rowbits, dtype=np.uint32)
         self.n_samples = int(n_samples)
+        self.threshold = None     # permutation threshold of the column (test(n_perm=...)), else None
+        self.minp = None          # its B permutation minima
 
     @property
     def presence(self):
@@ -113,6 +117,54 @@ def trim_top(res, top_k):
     order = np.lexsort((res.row, res.p))[:top_k]
     order.sort()
     return res.take(order)
+
+
+def permute_columns(pheno, n_perm, seed=0, first=0):
+    """Permutations first .. first + n_perm - 1 of every column of an N x P phenotype table (NaN = NA) -> P x n_perm x N.
+    A permutation shuffles the column's non-NA values among its non-NA samples: NA positions stay, and so do the
+    samples' weights, so the sample filter (n_with / n_without) of every k-mer is that of the observed column.
+    Permutation b of column j is drawn from numpy.random.default_rng((seed, j, b)) alone: it does not depend on which
+    other permutations or columns are drawn with it (any batching gives the same columns)."""
+    ph = np.asarray(pheno, dtype=np.float64)
+    if ph.ndim == 1:
+        ph = ph[:, None]
+    N, P = ph.shape
+    out = np.empty((P, int(n_perm), N))
+    for j in range(P):
+        col = ph[:, j]
+        idx = np.flatnonzero(~np.isnan(col))
+        vals = col[idx]
+        out[j] = col
+        for b in range(int(n_perm)):
+            out[j, b, idx] = vals[np.random.default_rng((int(seed), j, int(first) + b)).permutation(len(idx))]
+    return out
+
+
+def permutation_thresholds(minp, alpha):
+    """Westfall & Young's single-step min-p threshold per column: minp is P x B (the smallest p of each permuted column
+    over all testable k-mers), alpha the family-wise error rate (the p-value cut-off). With q_1 <= ... <= q_B the sorted
+    minima of a column, t = q_{floor(alpha B) + 1}; at most floor(alpha B) permutations have a k-mer below it. Returns
+    min(t, alpha) per column: a k-mer survives iff p < that. B < 1/alpha permutations cannot give a threshold."""
+    m = np.atleast_2d(np.asarray(minp, dtype=np.float64))
+    B = m.shape[1]
+    k = math.floor(Fraction(repr(float(alpha))) * B)     # exact: 0.05 * 20 is 1, not 0.999...
+    if k < 1:
+        raise ValueError(f"{B} permutations cannot give a threshold at alpha = {alpha}: at least "
+                         f"{math.ceil(1 / Fraction(repr(float(alpha))))} are needed")
+    if k >= B:
+        return np.full(m.shape[0], float(alpha))
+    return np.minimum(np.sort(m, axis=1)[:, k], float(alpha))
+
+
+def _unit_weights_as_none(weights):
+    """The reference's default weight is the int 1: all-ones weights run the exact integer tables."""
+    if weights is None:
+        return None
+    w = np.asarray(weights, dtype=np.float64)
+    return None if np.all(w == 1.0) else w
+
+
+PERM_BATCH_BYTES = 256 << 20        # host bytes of permuted columns handed to ps_minp_* at once
 
 
 class KmerAssociation:
@@ -263,7 +315,7 @@ class KmerAssociation:
 
     # stage 3 (modeling.py:1679-1683)
     def test(self, pheno, binary, weights=None, min_samples=2, max_samples=None, pvalue_cutoff=0.05,
-             omit_b=False, n_union_total=None, pheno_names=None, top_k=None):
+             omit_b=False, n_union_total=None, pheno_names=None, top_k=None, n_perm=0, perm_seed=0, minp=None):
         """pheno: N x P float array, NaN = NA (binary columns hold 0/1).
 
         Keep rule (modeling.py:738, 795): chi2 keeps p < cutoff (omit_B) or p < cutoff/U;
@@ -271,6 +323,10 @@ class KmerAssociation:
         pass n_union_total when this context holds only a shard of the k-mer space.
         top_k: keep only the top_k survivors per column by p-value, selected on the GPU before anything
         is copied to the host (`--n_kmers`, modeling.py:1128-1131); self.n_survivors is the count before the cut.
+        n_perm > 0: the permutation threshold replaces cutoff/U (not the uncorrected omit_B rule): column j keeps
+        p < permutation_thresholds(minp, cutoff)[j], minp from permutation_minp(..., n_perm, seed=perm_seed), or
+        the P x B `minp` given (minima already combined over k-mer ranges or shards). The results then carry
+        `threshold` and `minp` of their column.
         """
         ph = np.asarray(pheno, dtype=np.float64)
         if ph.ndim == 1:
@@ -281,12 +337,15 @@ class KmerAssociation:
             max_samples = N - 2
         U = self.U if n_union_total is None else n_union_total
         names = pheno_names or [f"pheno{j + 1}" for j in range(P)]
-        w = None
-        if weights is not None:
-            w = np.asarray(weights, dtype=np.float64)
-            if np.all(w == 1.0):
-                w = None   # the reference's default weight is the int 1: exact integer tables
-        if U == 0:
+        w = _unit_weights_as_none(weights)
+        perm = (n_perm > 0 or minp is not None) and not (binary and omit_b)
+        if perm:
+            if minp is None:
+                permutation_thresholds(np.ones((1, int(n_perm))), pvalue_cutoff)     # too few permutations: raise now
+                minp = self.permutation_minp(ph, binary, n_perm, w, min_samples, max_samples, perm_seed)
+            cut = permutation_thresholds(minp, pvalue_cutoff)
+            thr = float(cut.max())
+        elif U == 0:
             thr = 0.0
         elif binary and omit_b:
             thr = float(pvalue_cutoff)
@@ -304,10 +363,39 @@ class KmerAssociation:
         out = []
         for j in range(P):
             sel = sv["pheno"] == j
+            if perm:
+                sel &= sv["p"] < cut[j]     # one pass at the largest threshold, each column cut to its own
             out.append(trim_top(PhenoResult(
                 name=names[j], kmer=sv["kmer"][sel], row=sv["row"][sel], stat=sv["stat"][sel],
                 p=sv["p"][sel], mean_x=sv["mean_x"][sel], mean_y=sv["mean_y"][sel],
                 n_with=sv["n_with"][sel], rowbits=sv["rowbits"][sel], n_samples=N), top_k))
+            if perm:
+                out[-1].threshold, out[-1].minp = float(cut[j]), np.asarray(minp[j], dtype=np.float64)
+        return out
+
+    def permutation_minp(self, pheno, binary, n_perm, weights=None, min_samples=2, max_samples=None, seed=0):
+        """Min-p of n_perm permutations of every phenotype column (permute_columns) over this build's union: P x n_perm,
+        entry [j, b] = the smallest p (chi2 or Welch, as test() computes it) over the k-mers that pass the sample
+        filter in permutation b of column j, 1.0 if none. Union, matrix and the survivors of the last test stay."""
+        ph = np.asarray(pheno, dtype=np.float64)
+        if ph.ndim == 1:
+            ph = ph[:, None]
+        N, P = ph.shape
+        assert N == self.n_samples
+        n_perm = int(n_perm)
+        if max_samples is None:
+            max_samples = N - 2
+        w = _unit_weights_as_none(weights)
+        out = np.empty((P, n_perm))
+        step = max(1, PERM_BATCH_BYTES // max(1, 8 * P * N))
+        for b0 in range(0, n_perm, step):
+            nb = min(step, n_perm - b0)
+            cols = permute_columns(ph, nb, seed, first=b0).reshape(P * nb, N)
+            if binary:
+                m = self.ctx.minp_chi2(np.where(np.isnan(cols), -1, cols).astype(np.int8), w, min_samples, max_samples)
+            else:
+                m = self.ctx.minp_welch(cols, w, min_samples, max_samples)
+            out[:, b0:b0 + nb] = m.reshape(P, nb)
         return out
 
     def run(self, buffers, k, pheno, binary, weights=None, cutoff=1, **kw):
@@ -370,7 +458,8 @@ class KmerAssociation:
         return int(n_instances * slack * (b - a) / n_ranges) + (1 << 20)
 
     def test_in_ranges(self, pheno, binary, n_ranges, weights=None, pvalue_cutoff=0.05, omit_b=False,
-                       splitters=None, n_instances=None, top_k=None, n_super=None, restrict=None, **kw):
+                       splitters=None, n_instances=None, top_k=None, n_super=None, restrict=None, n_perm=0,
+                       perm_seed=0, **kw):
         """Stages 2-3 when records or matrix do not fit in HBM at once (SURVEY.md §7 "memory at
         config 5"): the k-mer space is cut into n_ranges contiguous ranges (quantiles of sample 0,
         or `splitters` from an earlier call on the same job), each range is built and tested on its
@@ -389,6 +478,9 @@ class KmerAssociation:
         n_instances: k-mer instances of the whole job (positions); sizes the page pools of a range
         (ps_set_capacity_hint) instead of reserving for every position of the input.
         restrict (--kmerDB database k-mers): only with n_ranges == 1, which restricts the one build.
+        n_perm > 0 (test()): each range's pass also gives that range's min-p of the permuted columns; the minima
+        are combined over the ranges (element-wise minimum) and the range is tested against the thresholds of the
+        minima seen so far, which can only fall as ranges follow: again a laxer cut, the exact one at the end.
         Call after count(). Returns (U, [PhenoResult per phenotype column])."""
         if restrict is not None and n_ranges > 1:
             raise RuntimeError("--kmerDB needs union and matrix in GPU memory at once; this input needs "
@@ -403,6 +495,10 @@ class KmerAssociation:
         plan = self.plan_ranges(n_ranges, spl, n_instances, n_super)
         spl, grouped, slack, first_of = plan["splitters"], plan["grouped"], plan["slack"], plan["first_of"]
         self.range_splitters = spl
+        perm = n_perm > 0 and not (binary and omit_b)
+        minp = np.ones((ph.shape[1], int(n_perm))) if perm else None
+        if perm:
+            permutation_thresholds(minp, pvalue_cutoff)      # too few permutations: raise before any build
         parts, U, sizes = [], 0, []
         for r in range(n_ranges):
             lo = 0 if r == 0 else spl[r - 1]
@@ -418,8 +514,12 @@ class KmerAssociation:
             u_r = self.build()
             if restrict is not None:
                 u_r = self.restrict_to(restrict)
+            if perm and u_r:
+                minp = np.minimum(minp, self.permutation_minp(ph, binary, n_perm, weights, kw.get("min_samples", 2),
+                                                              kw.get("max_samples"), perm_seed))
             res = self.test(ph, binary, weights, pvalue_cutoff=pvalue_cutoff, omit_b=omit_b, top_k=top_k,
-                            n_union_total=(U + u_r) if not (binary and omit_b) else None, **kw) if u_r else None
+                            n_union_total=(U + u_r) if not (binary and omit_b) else None, minp=minp,
+                            **kw) if u_r else None
             parts.append((U, res))
             U += u_r
             sizes.append(u_r)
@@ -428,6 +528,7 @@ class KmerAssociation:
             self._range_sizes = {(self.k, self.n_samples, tuple(spl)): sizes}   # the next call's super-range choice
         self.U = U
         exact = float(pvalue_cutoff) if (binary and omit_b) else (float(pvalue_cutoff) / U if U else 0.0)
+        cut = permutation_thresholds(minp, pvalue_cutoff) if perm else np.full(ph.shape[1], exact)
         out = []
         W = self.ctx.row_words()
         for j in range(ph.shape[1]):
@@ -438,7 +539,7 @@ class KmerAssociation:
                     continue
                 r = res[j]
                 name = r.name
-                keep = r.p < exact
+                keep = r.p < cut[j]
                 cols["kmer"].append(r.kmer[keep]); cols["row"].append(r.row[keep] + np.uint64(base))
                 for f in ("stat", "p", "mean_x", "mean_y", "n_with", "rowbits"):
                     cols[f].append(getattr(r, f)[keep])
@@ -449,4 +550,6 @@ class KmerAssociation:
                 mean_x=cat("mean_x", np.float64), mean_y=cat("mean_y", np.float64), n_with=cat("n_with", np.uint32),
                 rowbits=(np.concatenate(cols["rowbits"]) if cols["rowbits"] else np.zeros((0, W), np.uint32)),
                 n_samples=self.n_samples), top_k))
+            if perm:
+                out[-1].threshold, out[-1].minp = float(cut[j]), minp[j]
         return U, out
